@@ -21,6 +21,10 @@ Default workload = BASELINE.json configs[1]: 100 plates x 4 conditions x 10 load
   c3 / c1     : BASELINE configs 3 (~1 M-DOF single solves) and 1 (one plate-condition through the
                 drop-in FEAnalysis.calculate())
 
+`--steps K` is the number of timed steps of value, e2e and dataset_e2e.  `--dump-outputs DIR` writes what the last
+timed device-resident step computed (dump_outputs); the workload is seeded, so two builds run with the same
+arguments can be compared output for output.
+
 `--impl reference` times the reference's CPU algorithm (oracle port; sfepy itself is not
 installable here) with all host cores on bounded samples of the same workload.
 Under torchrun (N > 1) every rank processes its own plates (weak scaling, no collective on the
@@ -61,7 +65,12 @@ def parse():
                     help="--impl reference: re-factorise at every load step like sfepy's ScipyDirect (reference) or "
                          "factor once and scale (best)")
     ap.add_argument("--skip", default="", help="comma list of optional blocks to skip: dataset,as_sampled,c3,c1,cpu_best")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed device-resident step computed as DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 # --------------------------------------------------------------------------
@@ -210,6 +219,29 @@ def workload_name(a):
             % (a.plates, a.conditions, a.steps_per_condition - 1, a.image_size))
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, res, packed):
+    """The BatchResult of one step as path/<name>.npy, so that two builds can be compared output for output on the
+    same seeded workload: u (final-step displacement of the kept samples' vertices, concatenated), ranges, iters,
+    relres, status and images, in float64 (images in float32), plus sample_index, the plate-conditions kept.  All of
+    them are kept while the files stay within DUMP_LIMIT bytes; past that a fixed, seeded sample of them."""
+    u = packed.split_vertices(res.u)
+    per = np.array([x.nbytes for x in u]) + 4 * res.images[0].size + 8 * 8
+    budget = DUMP_LIMIT - 7 * 128    # the .npy headers
+    keep = np.arange(packed.n)
+    if per.sum() > budget:
+        order = np.random.default_rng(0).permutation(packed.n)
+        keep = np.sort(order[:np.searchsorted(np.cumsum(per[order]), budget, side="right")])
+    arrays = {"sample_index": keep.astype(np.float64), "u": np.concatenate([u[i] for i in keep]),
+              "ranges": res.ranges[keep], "iters": res.iters[keep].astype(np.float64), "relres": res.relres[keep],
+              "status": res.status[keep].astype(np.float64), "images": res.images[keep].astype(np.float32)}
+    os.makedirs(path, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), x)
+
+
 # --------------------------------------------------------------------------
 def run_reference(a):
     rank, world, local = dist_env()
@@ -341,9 +373,9 @@ def run_b200(a):
         # cluster kernels by ~8 %, so it is only created when asked for)
         dist.init_process_group("cpu:gloo,cuda:nccl")
     use_nccl = os.environ.get("FEA_BENCH_NCCL", "0") == "1"
-    import __graft_entry__ as ge
-    ge.build()
-    from fea_diffusion_b200 import Context, pack
+    # the library __graft_entry__.build() left in the tree; the bench compiles nothing and writes nothing there
+    from fea_diffusion_b200 import Context, load_library, pack
+    load_library()
     from fea_diffusion_b200.solver import BatchResult
     from fea_diffusion_b200.workload import build_workload
 
@@ -448,6 +480,8 @@ def run_b200(a):
     cl_size = stats[0]["cluster_size"]
     res0 = batches[0].download()
     rounds0 = batches[0].refine_rounds()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, batches[-1].download(images=True), packed)
     for b in batches:
         b.destroy()
 
@@ -585,7 +619,7 @@ def run_b200(a):
         barrier()
         ctx.event_record(4)
         t0 = time.perf_counter()
-        n_ds = max(a.steps, 12)      # the pipeline's fill (packing step 0) and drain (last read-back) are inside the timed region
+        n_ds = a.steps               # the pipeline's fill (packing step 0) and drain (last read-back) are inside the timed region
         last = run_dataset(n_ds)
         ctx.event_record(5)
         barrier()

@@ -13,9 +13,13 @@ _F = None
 
 
 def fixtures():
+    """The golden arrays by name: tests/golden/fixtures.npz and the reference's displacements (reference_u.npz)."""
     global _F
     if _F is None:
-        _F = np.load(os.path.join(ROOT, "tests", "golden", "fixtures.npz"))
+        _F = {}
+        for name in ("fixtures.npz", "reference_u.npz"):
+            with np.load(os.path.join(ROOT, "tests", "golden", name)) as f:
+                _F.update(f)
     return _F
 
 

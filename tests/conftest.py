@@ -1,7 +1,6 @@
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
@@ -17,7 +16,8 @@ def pytest_configure(config):
 def golden():
     """Committed fixtures converted from the reference's data artefacts
     (tests/golden/make_golden.py)."""
-    return np.load(os.path.join(ROOT, "tests", "golden", "fixtures.npz"))
+    import cases
+    return cases.fixtures()
 
 
 @pytest.fixture(scope="session")

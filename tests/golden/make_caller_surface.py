@@ -5,7 +5,7 @@ with their positional counts and keywords, attributes read.  The result is commi
 tests/golden/caller_surface.json so that the GPU box (which has no reference checkout) can check
 the drop-in against it; tests/test_caller_surface.py re-derives it when the checkout is present.
 
-    python tests/golden/make_caller_surface.py /root/reference > tests/golden/caller_surface.json
+    python tests/golden/make_caller_surface.py <reference checkout> > tests/golden/caller_surface.json
 """
 import ast
 import json
@@ -63,6 +63,6 @@ def surface(source: str) -> dict:
 
 
 if __name__ == "__main__":
-    root = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+    root = sys.argv[1]
     with open(root + "/datagen/generate.py") as f:
         print(json.dumps(surface(f.read()), indent=1, sort_keys=True))

@@ -1,12 +1,11 @@
 #!/usr/bin/env python
-"""Generate the golden fixtures under tests/golden/ from /root/reference.
-
-Run once in the build container (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+"""Generate the golden fixtures under tests/golden/ from a checkout of the reference project
+(namanxkumar/fea-diffusion):
+    python tests/golden/make_golden.py <reference checkout>
 
 Only DATA artefacts are converted (meshes, sfepy's committed fp64 ``u`` outputs,
 committed PNG renders, text-format samples, log pins) -- no reference source.
-Sources (relative to /root/reference, SURVEY.md App. B):
+Sources (relative to the checkout, SURVEY.md App. B):
   applications/cantilever/cantilever.{mesh,vtk}, displacement_[xy].png, outline.png
   applications/shearblade/shearblade.{mesh,vtk}, displacement_[xy].png, outline.png
   applications/gusset/gusset.mesh
@@ -24,7 +23,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.abspath(os.path.join(HERE, "..", "..")))
 from oracle.mesh_io import read_medit, read_vtk_legacy  # noqa: E402
 
-REF = "/root/reference"
+REF = sys.argv[1] if len(sys.argv) > 1 else os.environ.get("FEA_REFERENCE_DIR", "")
 
 
 def sha16(path):
@@ -72,6 +71,8 @@ def main():
                        src="applications/composite/datagenapplication.ipynb:331,384,387,420"),
         cantilever=dict(n=4844, nnz=65896, fixed=42, src="SURVEY.md App. B (oracle-derived size)"),
     )
+    # sfepy's displacements in a file of their own, which keeps each file under 1 MB
+    np.savez_compressed(os.path.join(HERE, "reference_u.npz"), **{k: out.pop(k) for k in ("cantilever_u", "shearblade_u")})
     np.savez_compressed(os.path.join(HERE, "fixtures.npz"), **out)
     with open(os.path.join(HERE, "fixtures.json"), "w") as f:
         json.dump(meta, f, indent=1)

@@ -1,9 +1,10 @@
 """The reference's own caller against the drop-in surface (north_star: "datagen/generate.py and
 generate_data.py drive it unchanged").  Every call, keyword and attribute that
-/root/reference/datagen/generate.py:56-164 uses on FEAnalysis / MeshGenerator / the two utils
+the reference's datagen/generate.py:56-164 uses on FEAnalysis / MeshGenerator / the two utils
 functions -- extracted from its source by tests/golden/make_caller_surface.py and committed as
-tests/golden/caller_surface.json -- must bind against this package's classes; with the checkout
-present the fixture is re-derived and the reference's file itself is loaded over the drop-in."""
+tests/golden/caller_surface.json -- must bind against this package's classes; with a checkout of the
+reference named by FEA_REFERENCE_DIR the fixture is re-derived and the reference's file itself is loaded
+over the drop-in."""
 import importlib.util
 import inspect
 import json
@@ -16,7 +17,7 @@ from fea_diffusion_b200.datagen.generate import generate_data, load_reference_ge
 from fea_diffusion_b200.datagen.mesh_generator import MeshGenerator
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("FEA_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("FEA_REFERENCE_DIR", "")
 
 
 def committed():
@@ -69,7 +70,7 @@ def test_constructor_signature_is_the_reference_one():
         (11, False, None, 210000, 0.3)
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "datagen", "generate.py")), reason="no reference checkout here")
+@pytest.mark.skipif(not (REF and os.path.isfile(os.path.join(REF, "datagen", "generate.py"))), reason="needs a reference checkout (FEA_REFERENCE_DIR)")
 def test_fixture_is_current_and_the_reference_file_loads_over_the_dropin():
     spec = importlib.util.spec_from_file_location("make_caller_surface", os.path.join(HERE, "golden", "make_caller_surface.py"))
     mod = importlib.util.module_from_spec(spec)
