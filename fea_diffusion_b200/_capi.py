@@ -27,6 +27,7 @@ EXPORTS = [
     "fea_batch_get_timed_launches",
     "fea_batch_sample_sizes", "fea_batch_get_conn", "fea_batch_get_element_stiffness",
     "fea_batch_get_csr", "fea_batch_spmv", "fea_rasterize_fields", "fea_solve_batch",
+    "fea_batch_set_refinement", "fea_batch_get_mg_levels", "fea_batch_get_level_csr", "fea_batch_mg_apply",
 ]
 
 STATUS_NAMES = {0: "OK", 1: "BAD_ARG", 2: "CUDA_ERROR", 3: "OUT_OF_MEMORY", 4: "BAD_STATE", 5: "MESH_ERROR"}
@@ -84,6 +85,17 @@ class SolveStats(C.Structure):
         ("cluster_ms", C.c_float), ("cluster_size", C.c_int32),
         ("refined_systems", C.c_int32), ("pad_", C.c_int32),
         ("cluster_block_reads_tmem", C.c_int64), ("cluster_block_reads_smem", C.c_int64), ("cluster_block_reads_l2", C.c_int64),
+    ]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class MgLevel(C.Structure):
+    """fea_mg_level (include/fea_b200.h)."""
+    _fields_ = [
+        ("n_vertices", C.c_int64), ("n_cells", C.c_int64), ("n_active_dofs", C.c_int64), ("nnz", C.c_int64),
+        ("lambda_max", C.c_double), ("vcycle_ms", C.c_double),
     ]
 
     def as_dict(self):
@@ -149,6 +161,10 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "fea_batch_cell_strain_stress": (C.c_int, [P, I32, P, P]),
         "fea_batch_rasterize_flags": (C.c_int, [P, P, P, P]),
         "fea_rasterize_fields": (C.c_int, [P, P, C.c_int64, P, C.c_int64, I32, P, I32, I32, P, P, I32, P]),
+        "fea_batch_set_refinement": (C.c_int, [P, I32]),
+        "fea_batch_get_mg_levels": (C.c_int, [P, I32, C.POINTER(MgLevel), P]),
+        "fea_batch_get_level_csr": (C.c_int, [P, I32, P, P, P]),
+        "fea_batch_mg_apply": (C.c_int, [P, P, P]),
         "fea_solve_batch": (C.c_int, [P, C.POINTER(BatchDesc), F64, I32, I32, P, F64, P, P, P, P, P, P,
                                       C.POINTER(SolveStats)]),
     }

@@ -56,6 +56,7 @@ void api_free_batch(fea_batch* hb) {
   if (!hb) return;
   Batch& b = hb->b;
   cudaSetDevice(b.ctx->device);
+  mg_release(b);
   for (void* p : b.allocs) cudaFreeAsync(p, b.ctx->stream);
   b.allocs.clear();
   if (b.ev_staged) cudaEventDestroy(b.ev_staged);
@@ -144,6 +145,75 @@ cudaError_t api_batch_finish(Batch& b, const int8_t* creg_local, const int32_t* 
 #undef A
   b.ctx->launches += 7;
   return e;
+}
+
+int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke) {
+  cudaStream_t st = ctx->c.stream;
+  const int N = 2 * b.npc;
+  CK(ctx, dalloc(b, &b.inc_ptr, b.NV + 1));
+  CK(ctx, dalloc(b, &b.inc, b.NC * b.npc));
+  CK(ctx, dalloc(b, &b.adj_ptr, b.NV + 1));
+  CK(ctx, dalloc(b, &b.ke, b.NC * N * N));
+  b.n_slices = (int32_t)(b.NBR / kSlice);
+  CK(ctx, dalloc(b, &b.slice_len, b.n_slices));
+  CK(ctx, dalloc(b, &b.slice_ptr, (int64_t)b.n_slices + 1));
+  CK(ctx, fill_ke(b));
+  CK(ctx, launch_topology_counts(b));
+  CK(ctx, launch_sell_lengths(b));
+  // one host round trip: totals and error flags
+  int32_t h_adj = 0, h_err[3] = {0, 0, 0};
+  int64_t h_blocks = 0;
+  CK(ctx, cudaMemcpyAsync(&h_adj, b.adj_ptr + b.NV, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(&h_blocks, b.slice_ptr + b.n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(h_err, b.err_flag, 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  if (h_err[0] & 2) return api_fail(ctx, FEA_MESH_ERROR, "connectivity or cell_region index out of range");
+  if (h_err[0] & 1) return api_fail(ctx, FEA_MESH_ERROR, "vertex valence exceeds the supported maximum (63)");
+  if (h_err[2] & 4) return api_fail(ctx, FEA_MESH_ERROR, "more than 16 distinct overlap combinations of material regions in one sample");
+  b.n_adj = h_adj;
+  b.n_blocks = b.n_slices ? h_blocks : 0;
+  b.max_row_blocks = h_err[1];
+  CK(ctx, dalloc(b, &b.adj, b.n_adj));
+  CK(ctx, launch_topology_fill(b));
+  CK(ctx, dalloc(b, &b.val, b.n_blocks * 4));
+  CK(ctx, dalloc(b, &b.col, b.n_blocks));
+  CK(ctx, dalloc(b, &b.dscale, b.NBR * 2));
+  CK(ctx, dalloc(b, &b.scoup, b.NBR));
+  CK(ctx, dalloc(b, &b.x, b.NBR * 2));
+  CK(ctx, dalloc(b, &b.rp, b.NBR * 4));
+  CK(ctx, dalloc(b, &b.q, b.NBR * 2));
+  CK(ctx, dalloc(b, &b.xlo, b.NBR * 2));
+  CK(ctx, dalloc(b, &b.sb, b.NBR * 2));
+  const int64_t ncta = b.NBR / kCtaRows;
+  CK(ctx, dalloc(b, &b.active_cta, 4 * ncta));  // int4 entries
+  CK(ctx, dalloc(b, &b.partA, ncta));
+  CK(ctx, dalloc(b, &b.partB, ncta));
+  CK(ctx, dalloc(b, &b.sc.rz[0], b.ns));
+  CK(ctx, dalloc(b, &b.sc.rz[1], b.ns));
+  CK(ctx, dalloc(b, &b.sc.pq, b.ns));
+  CK(ctx, dalloc(b, &b.sc.rz0, b.ns));
+  CK(ctx, dalloc(b, &b.sc.tol2, b.ns));
+  CK(ctx, dalloc(b, &b.sc.done, b.ns));
+  CK(ctx, dalloc(b, &b.sc.iters, b.ns));
+  CK(ctx, dalloc(b, &b.sc.cap, b.ns));
+  CK(ctx, dalloc(b, &b.sc.rz_mon, b.ns));
+  CK(ctx, dalloc(b, &b.sc.rounds, b.ns));
+  CK(ctx, dalloc(b, &b.sc.arrive, 2 * (int64_t)b.ns));
+  CK(ctx, dalloc(b, &b.sc.status, b.ns));
+  CK(ctx, dalloc(b, &b.sc.psumA, b.ns));
+  CK(ctx, dalloc(b, &b.sc.psumB, b.ns));
+  CK(ctx, dalloc(b, &b.sc.n_done, 1));
+  CK(ctx, dalloc(b, &b.rz_last, b.ns));
+  CK(ctx, dalloc(b, &b.relres, b.ns));
+  CK(ctx, dalloc(b, &b.u, b.NV * 2));
+  CK(ctx, dalloc(b, &b.ranges, (int64_t)b.ns * 4));
+  CK(ctx, cudaMemsetAsync(b.sc.status, 0xFF, sizeof(int32_t) * b.ns, st));
+  CK(ctx, cudaMemsetAsync(b.sc.iters, 0, sizeof(int32_t) * b.ns, st));
+  CK(ctx, cudaMemsetAsync(b.relres, 0, sizeof(double) * b.ns, st));
+  CK(ctx, launch_sell_fill(b));
+  ctx->c.launches += 1 + 10 + 4 + 1 + 2;
+  b.assembled = true;
+  return FEA_OK;
 }
 
 }  // namespace fea
@@ -354,7 +424,12 @@ int fea_batch_create(fea_ctx* ctx, const fea_batch_desc* d, fea_batch** out) {
   A(cudaMemcpyAsync(b.fixed, d->fixed, b.NV, cudaMemcpyHostToDevice, st));
   A(cudaMemcpyAsync(b.rhs, d->rhs, sizeof(double) * b.NV * 2, cudaMemcpyHostToDevice, st));
   A(api_batch_finish(b, creg_local, conn_local));
-  if (conn_local) cudaFreeAsync(conn_local, st);
+  if (e == cudaSuccess && b.ns == 1 && b.npc == 3) {   // a possible uniform refinement (fea_batch_set_refinement)
+    b.conn_given = conn_local;
+    b.allocs.push_back(conn_local);
+  } else if (conn_local) {
+    cudaFreeAsync(conn_local, st);
+  }
   if (creg_local) cudaFreeAsync(creg_local, st);
 #undef A
   if (e != cudaSuccess) {
@@ -377,73 +452,23 @@ int fea_batch_assemble(fea_batch* hb) {
   fea_ctx* ctx = hb->owner;
   Batch& b = hb->b;
   if (b.assembled) return FEA_OK;
+  if (b.mg && b.mg->failed) return api_fail(ctx, FEA_BAD_STATE, "building the multigrid hierarchy of this batch failed");
   CK(ctx, cudaSetDevice(ctx->c.device));
-  cudaStream_t st = ctx->c.stream;
-  const int N = 2 * b.npc;
-  CK(ctx, dalloc(b, &b.inc_ptr, b.NV + 1));
-  CK(ctx, dalloc(b, &b.inc, b.NC * b.npc));
-  CK(ctx, dalloc(b, &b.adj_ptr, b.NV + 1));
-  CK(ctx, dalloc(b, &b.ke, b.NC * N * N));
-  b.n_slices = (int32_t)(b.NBR / kSlice);
-  CK(ctx, dalloc(b, &b.slice_len, b.n_slices));
-  CK(ctx, dalloc(b, &b.slice_ptr, (int64_t)b.n_slices + 1));
-  CK(ctx, launch_element_stiffness(b));
-  CK(ctx, launch_topology_counts(b));
-  CK(ctx, launch_sell_lengths(b));
-  // one host round trip: totals and error flags
-  int32_t h_adj = 0, h_err[3] = {0, 0, 0};
-  int64_t h_blocks = 0;
-  CK(ctx, cudaMemcpyAsync(&h_adj, b.adj_ptr + b.NV, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  CK(ctx, cudaMemcpyAsync(&h_blocks, b.slice_ptr + b.n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  CK(ctx, cudaMemcpyAsync(h_err, b.err_flag, 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  CK(ctx, cudaStreamSynchronize(st));
-  if (h_err[0] & 2) return api_fail(ctx, FEA_MESH_ERROR, "connectivity or cell_region index out of range");
-  if (h_err[0] & 1) return api_fail(ctx, FEA_MESH_ERROR, "vertex valence exceeds the supported maximum (63)");
-  if (h_err[2] & 4) return api_fail(ctx, FEA_MESH_ERROR, "more than 16 distinct overlap combinations of material regions in one sample");
-  b.n_adj = h_adj;
-  b.n_blocks = b.n_slices ? h_blocks : 0;
-  b.max_row_blocks = h_err[1];
-  CK(ctx, dalloc(b, &b.adj, b.n_adj));
-  CK(ctx, launch_topology_fill(b));
-  CK(ctx, dalloc(b, &b.val, b.n_blocks * 4));
-  CK(ctx, dalloc(b, &b.col, b.n_blocks));
-  CK(ctx, dalloc(b, &b.dscale, b.NBR * 2));
-  CK(ctx, dalloc(b, &b.scoup, b.NBR));
-  CK(ctx, dalloc(b, &b.x, b.NBR * 2));
-  CK(ctx, dalloc(b, &b.rp, b.NBR * 4));
-  CK(ctx, dalloc(b, &b.q, b.NBR * 2));
-  CK(ctx, dalloc(b, &b.xlo, b.NBR * 2));
-  CK(ctx, dalloc(b, &b.sb, b.NBR * 2));
-  const int64_t ncta = b.NBR / kCtaRows;
-  CK(ctx, dalloc(b, &b.active_cta, 4 * ncta));  // int4 entries
-  CK(ctx, dalloc(b, &b.partA, ncta));
-  CK(ctx, dalloc(b, &b.partB, ncta));
-  CK(ctx, dalloc(b, &b.sc.rz[0], b.ns));
-  CK(ctx, dalloc(b, &b.sc.rz[1], b.ns));
-  CK(ctx, dalloc(b, &b.sc.pq, b.ns));
-  CK(ctx, dalloc(b, &b.sc.rz0, b.ns));
-  CK(ctx, dalloc(b, &b.sc.tol2, b.ns));
-  CK(ctx, dalloc(b, &b.sc.done, b.ns));
-  CK(ctx, dalloc(b, &b.sc.iters, b.ns));
-  CK(ctx, dalloc(b, &b.sc.cap, b.ns));
-  CK(ctx, dalloc(b, &b.sc.rz_mon, b.ns));
-  CK(ctx, dalloc(b, &b.sc.rounds, b.ns));
-  CK(ctx, dalloc(b, &b.sc.arrive, 2 * (int64_t)b.ns));
-  CK(ctx, dalloc(b, &b.sc.status, b.ns));
-  CK(ctx, dalloc(b, &b.sc.psumA, b.ns));
-  CK(ctx, dalloc(b, &b.sc.psumB, b.ns));
-  CK(ctx, dalloc(b, &b.sc.n_done, 1));
-  CK(ctx, dalloc(b, &b.rz_last, b.ns));
-  CK(ctx, dalloc(b, &b.relres, b.ns));
-  CK(ctx, dalloc(b, &b.u, b.NV * 2));
-  CK(ctx, dalloc(b, &b.ranges, (int64_t)b.ns * 4));
-  CK(ctx, cudaMemsetAsync(b.sc.status, 0xFF, sizeof(int32_t) * b.ns, st));
-  CK(ctx, cudaMemsetAsync(b.sc.iters, 0, sizeof(int32_t) * b.ns, st));
-  CK(ctx, cudaMemsetAsync(b.relres, 0, sizeof(double) * b.ns, st));
-  CK(ctx, launch_sell_fill(b));
-  ctx->c.launches += 1 + 10 + 4 + 1 + 2;
-  b.assembled = true;
-  return FEA_OK;
+  int rc = api_batch_assemble(ctx, b, launch_element_stiffness);
+  if (rc == FEA_OK && b.mg) {
+    rc = mg_assemble(ctx, b);
+    if (rc != FEA_OK) {   // terminal: no solve on a half-built hierarchy, no second build over it
+      b.assembled = false;
+      b.mg->failed = true;
+    }
+  }
+  if (b.conn_given) {   // only fea_batch_set_refinement, which must precede assemble, reads it
+    cudaFreeAsync(b.conn_given, ctx->c.stream);
+    b.allocs.erase(std::find(b.allocs.begin(), b.allocs.end(), (void*)b.conn_given));
+    b.conn_given = nullptr;
+    if (b.mg) b.mg->lev[b.mg->levels].conn = nullptr;
+  }
+  return rc;
 }
 
 int fea_batch_solve(fea_batch* hb, double rtol, int32_t max_iter) {
@@ -453,7 +478,12 @@ int fea_batch_solve(fea_batch* hb, double rtol, int32_t max_iter) {
   if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_solve before fea_batch_assemble");
   if (!(rtol >= 0.0) || max_iter < 1) return api_fail(ctx, FEA_BAD_ARG, "rtol must be >= 0 and max_iter >= 1");
   CK(ctx, cudaSetDevice(ctx->c.device));
-  CK(ctx, run_pcg(b, rtol, max_iter));
+  if (b.mg) {
+    const int rc = mg_solve(ctx, b, rtol, max_iter);
+    if (rc != FEA_OK) return rc;
+  } else {
+    CK(ctx, run_pcg(b, rtol, max_iter));
+  }
   b.solved = true;
   return FEA_OK;
 }
@@ -815,6 +845,78 @@ int fea_solve_batch(fea_ctx* ctx, const fea_batch_desc* desc, double rtol, int32
   if (rc == FEA_OK && stats) *stats = hb->b.stats;
   fea_batch_destroy(hb);
   return rc;
+}
+
+int fea_batch_set_refinement(fea_batch* hb, int32_t levels) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_set_refinement after fea_batch_assemble");
+  if (b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch already declared its refinement");
+  if (b.ns != 1 || b.npc != 3) return api_fail(ctx, FEA_BAD_ARG, "a refinement hierarchy needs one sample of triangles");
+  if (levels < 1 || levels > 8) return api_fail(ctx, FEA_BAD_ARG, "levels must be 1..8");
+  if (!b.conn_given) return api_fail(ctx, FEA_BAD_ARG, "a refinement hierarchy is declared on a batch made by fea_batch_create, before fea_batch_assemble");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  return mg_set_refinement(ctx, b, levels);
+}
+
+int fea_batch_get_mg_levels(fea_batch* hb, int32_t cap, fea_mg_level* out, int32_t* n_out) {
+  if (!hb || !n_out || cap < 0 || (cap > 0 && !out)) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch declared no refinement");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_mg_levels before fea_batch_assemble");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  const int n = b.mg->levels + 1;
+  *n_out = n;
+  for (int l = 0; l < n && l < cap; ++l) {
+    const MgLevel& L = b.mg->lev[l];
+    int32_t na = 0;
+    CK(ctx, cudaMemcpyAsync(&na, L.b->n_active, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->c.stream));
+    CK(ctx, cudaStreamSynchronize(ctx->c.stream));
+    out[l].n_vertices = L.nv;
+    out[l].n_cells = L.nc;
+    out[l].n_active_dofs = 2 * (int64_t)na;
+    out[l].nnz = 4 * L.b->n_adj;
+    out[l].lambda_max = L.lmax;
+    out[l].vcycle_ms = L.ms;
+  }
+  return FEA_OK;
+}
+
+int fea_batch_get_level_csr(fea_batch* hb, int32_t level, int32_t* indptr, int32_t* indices, double* data) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch declared no refinement");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_level_csr before fea_batch_assemble");
+  if (level < 0 || level > b.mg->levels) return api_fail(ctx, FEA_BAD_ARG, "level out of range");
+  fea_batch* lb = b.mg->lev[level].hb ? b.mg->lev[level].hb : hb;
+  return fea_batch_get_csr(lb, 0, indptr, indices, data);
+}
+
+int fea_batch_mg_apply(fea_batch* hb, const double* r, double* z) {
+  if (!hb || !r || !z) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch declared no refinement");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_mg_apply before fea_batch_assemble");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
+  int32_t na = 0;
+  CK(ctx, cudaMemcpyAsync(&na, b.n_active, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  const int64_t n = 2 * (int64_t)na;
+  double* d = nullptr;
+  CK(ctx, cudaMallocAsync((void**)&d, sizeof(double) * 2 * std::max<int64_t>(1, n), st));
+  cudaError_t e = cudaMemcpyAsync(d, r, sizeof(double) * n, cudaMemcpyHostToDevice, st);
+  int rc = e == cudaSuccess ? mg_apply(ctx, b, d, d + std::max<int64_t>(1, n)) : FEA_CUDA_ERROR;
+  if (rc == FEA_OK) e = cudaMemcpyAsync(z, d + std::max<int64_t>(1, n), sizeof(double) * n, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  cudaFreeAsync(d, st);
+  if (rc != FEA_OK) return rc;
+  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_mg_apply", e);
+  return FEA_OK;
 }
 
 }  // extern "C"

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <functional>
 #include <map>
 #include <string>
 #include <vector>
@@ -69,6 +70,8 @@ struct SysScalars {
   double* psumB;
   int32_t* n_done;   // single counter: finished systems
 };
+
+struct Mg;
 
 struct Batch {
   Ctx* ctx = nullptr;
@@ -164,6 +167,38 @@ struct Batch {
   uint8_t* stage_regions = nullptr;       // [stage_field_off[ns]][size][size]
   int32_t* stage_class = nullptr;         // [2*ns] floating parts, empty vertices
   cudaEvent_t ev_staged = nullptr;        // recorded behind the last kernel that writes an output
+  // ---- multigrid hierarchy (fea_batch_set_refinement, k_mg.cu) ----
+  int32_t* conn_given = nullptr;  // [NC*3] connectivity as given (single-sample triangle batches, until assemble)
+  Mg* mg = nullptr;
+};
+
+// One level of the multigrid hierarchy of a uniformly refined single-sample batch (DESIGN.md section 3.9).
+// Level 0 is the coarsest mesh, level `levels` the batch itself.  Vectors are in the level's scaled
+// row space (Khat = S^T K S, rows in the level batch's solver order).
+struct MgLevel {
+  fea_batch* hb = nullptr;       // internal batch of a coarse level (nullptr for the finest: the batch itself)
+  Batch* b = nullptr;            // the level's batch
+  int64_t nv = 0, nc = 0;
+  int32_t* conn = nullptr;       // [nc*3] as-given numbering (derived from the children for coarse levels)
+  int32_t* creg = nullptr;       // [nc] cell region (the finest level: its cell_dreg)
+  int8_t* creg8 = nullptr;       // [nc] the same as the int8 input of a coarse level batch
+  int2* par = nullptr;           // [nv] levels >= 1: (v, -1) for a vertex of level l-1, else the edge's two ends
+  int32_t* child_ptr = nullptr;  // [nv(l-1)+1] levels >= 1: vertex of level l-1 -> the midpoints of level l
+  int32_t* child = nullptr;      //   that have it as an end, ascending
+  double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};   // levels >= 1
+  double lmax = 0.0;             // power-iteration estimate of the largest eigenvalue of Khat
+  double inv_theta = 0.0, c1[2] = {0.0, 0.0}, c2[2] = {0.0, 0.0};   // Chebyshev coefficients
+  double ms = 0.0;               // V-cycle time spent on the level in the last solve
+};
+struct Mg {
+  int levels = 0;
+  bool failed = false;           // building the hierarchy failed in fea_batch_assemble: the batch cannot be solved
+  std::vector<MgLevel> lev;      // [levels + 1]
+  double2 *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, finest row space (x = Batch::x)
+  double *partA = nullptr, *partB = nullptr;          // per-CTA partial sums
+  double* sc = nullptr;          // device scalars (kSc* slots, k_mg.cu)
+  double* h_sc = nullptr;        // pinned copy
+  std::vector<cudaEvent_t> ev;   // 4 per level + 2 around the solve
 };
 
 }  // namespace fea
@@ -192,6 +227,16 @@ int api_batch_begin(fea_ctx* ctx, int32_t ns, int32_t npc, const int64_t* vtx_of
 // device-side ordering of the cluster queues; b.xy, b.D, b.fixed, b.rhs must be allocated and
 // (stream-ordered) filled, conn_local / creg_local are consumed.
 cudaError_t api_batch_finish(Batch& b, const int8_t* d_creg_local, const int32_t* d_conn_local);
+// element stiffness (fill_ke: launch_element_stiffness, or the Galerkin product of a multigrid level),
+// topology, block-SELL matrix and solver vectors of a created batch
+int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke);
+
+// multigrid path (k_mg.cu): return FEA_OK or a status with the message set on ctx
+int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels);   // derive and validate the hierarchy
+int mg_assemble(fea_ctx* ctx, Batch& b);                     // coarse level batches, Galerkin operators, smoothers
+int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter);   // flexible CG preconditioned by V-cycles
+int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z);   // one V-cycle, active-DOF vectors
+void mg_release(Batch& b);
 
 template <class T>
 inline cudaError_t dalloc(Batch& b, T** p, int64_t n) {

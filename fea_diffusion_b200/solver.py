@@ -14,7 +14,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from . import _capi
-from ._capi import BatchDesc, BatchInfo, ConditionsDesc, FeaError, SolveStats, ptr
+from ._capi import BatchDesc, BatchInfo, ConditionsDesc, FeaError, MgLevel, SolveStats, ptr
 
 
 @dataclass
@@ -665,3 +665,34 @@ class Batch:
         y = np.empty_like(x)
         self.ctx._check(self.ctx.lib.fea_batch_spmv(self.h, int(sample), ptr(x), ptr(y)))
         return y
+
+    # ---- multigrid hierarchy of a uniformly refined single-sample batch ------------------------
+    def set_refinement(self, levels: int):
+        """Declare the only sample a ``levels``-times uniform red refinement (``workload.refine_uniform``
+        numbering); assemble then builds the coarse levels and solve runs multigrid-preconditioned CG."""
+        self.ctx._check(self.ctx.lib.fea_batch_set_refinement(self.h, int(levels)))
+        return self
+
+    def mg_levels(self) -> List[dict]:
+        """Per level, coarsest first: sizes, lambda_max of the scaled operator, V-cycle ms of the last solve."""
+        n = C.c_int32()
+        self.ctx._check(self.ctx.lib.fea_batch_get_mg_levels(self.h, 0, None, C.byref(n)))
+        arr = (MgLevel * n.value)()
+        self.ctx._check(self.ctx.lib.fea_batch_get_mg_levels(self.h, n.value, arr, C.byref(n)))
+        return [a.as_dict() for a in arr]
+
+    def level_csr(self, level: int):
+        """scipy CSR of level ``level``'s Galerkin operator, in the layout of ``csr``."""
+        import scipy.sparse as sp
+        lv = self.mg_levels()[level]
+        n, nnz = int(lv["n_active_dofs"]), int(lv["nnz"])
+        indptr, indices, data = np.empty(n + 1, np.int32), np.empty(nnz, np.int32), np.empty(nnz)
+        self.ctx._check(self.ctx.lib.fea_batch_get_level_csr(self.h, int(level), ptr(indptr), ptr(indices), ptr(data)))
+        return sp.csr_matrix((data, indices, indptr), shape=(n, n))
+
+    def mg_apply(self, r: np.ndarray) -> np.ndarray:
+        """z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as ``spmv``)."""
+        r = np.ascontiguousarray(r, dtype=np.float64)
+        z = np.empty_like(r)
+        self.ctx._check(self.ctx.lib.fea_batch_mg_apply(self.h, ptr(r), ptr(z)))
+        return z

@@ -348,6 +348,36 @@ int  fea_batch_get_csr(fea_batch* b, int32_t sample, int32_t* indptr, int32_t* i
 /* y = K x for one sample through the product SpMV kernel (x, y over active DOFs, unscaled) */
 int  fea_batch_spmv(fea_batch* b, int32_t sample, const double* x, double* y);
 
+/* ---- multigrid-preconditioned solve of a uniformly refined mesh ---------------------------
+ * A batch whose only sample is a uniform red refinement of a coarser mesh may declare its hierarchy
+ * (before fea_batch_assemble).  fea_batch_assemble then also builds the coarse levels -- Galerkin
+ * operators P^T K P assembled cell by cell, block-Jacobi Chebyshev smoothers -- and fea_batch_solve
+ * runs flexible CG preconditioned by one V-cycle per iteration, whose coarsest level is solved by the
+ * block-Jacobi CG of fea_batch_solve to rtol 1e-4.  Outputs keep their meaning: iterations are outer
+ * iterations, relres is the TRUE residual in the block-Jacobi-scaled norm. */
+typedef struct {
+  int64_t n_vertices, n_cells, n_active_dofs, nnz;   /* nnz of the reduced scalar CSR */
+  double lambda_max;   /* estimate of the largest eigenvalue of the block-Jacobi-scaled operator */
+  double vcycle_ms;    /* V-cycle time spent on the level in the last solve (level 0: the coarse solves) */
+} fea_mg_level;
+/* The batch's only sample is its own mesh refined `levels` (1..8) times, in the vertex and cell numbering
+ * of uniform red refinement: vertices of level l-1 keep their indices, the midpoint of each level-(l-1)
+ * edge follows them, children of cell p are p, p+nc, p+2nc, p+3nc = (a,ab,ca), (ab,b,bc), (ca,bc,c),
+ * (ab,bc,ca).  Checked on the device against the connectivity AS GIVEN (before the orientation fix) and
+ * the coordinates (midpoint == 0.5*(a+b) bit for bit, children share the parent's cell_region):
+ * FEA_MESH_ERROR if the mesh is not such a refinement; FEA_BAD_ARG for n_samples != 1,
+ * nodes_per_cell != 3 or levels out of range; FEA_BAD_STATE after fea_batch_assemble.  A vertex that no cell
+ * references is not a midpoint, so such a mesh is a MESH_ERROR too.  If fea_batch_assemble then fails to build
+ * the coarse levels, the batch stays unassembled: a second fea_batch_assemble returns FEA_BAD_STATE. */
+int  fea_batch_set_refinement(fea_batch* b, int32_t levels);
+/* per level l = 0 (coarsest) .. levels: vertices, cells, active DOFs, nnz, lambda_max estimate,
+ * V-cycle ms spent on the level in the last solve; *n_out = levels + 1 */
+int  fea_batch_get_mg_levels(fea_batch* b, int32_t cap, fea_mg_level* out, int32_t* n_out);
+/* reduced scalar CSR of level l's Galerkin operator, same layout and numbering rule as fea_batch_get_csr */
+int  fea_batch_get_level_csr(fea_batch* b, int32_t level, int32_t* indptr, int32_t* indices, double* data);
+/* z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as fea_batch_spmv) */
+int  fea_batch_mg_apply(fea_batch* b, const double* r, double* z);
+
 /* ---- scalar-field images of one mesh ----------------------------------------
  * The point-scalar renders of FEAnalysis.save_input_image / save_region_images (reference
  * fea_analysis.py:472-524: the constant field "1" and the 0/1 region flags of regions.vtk) and the
