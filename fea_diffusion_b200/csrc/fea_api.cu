@@ -246,16 +246,11 @@ int fea_ctx_create_prio(int device, int priority, fea_ctx** out) {
   // urgent priorities, the smaller the cluster the more urgent.
   if ((e = cudaStreamCreateWithPriority(&ctx->c.stream, cudaStreamNonBlocking, priority)) != cudaSuccess) { delete ctx; return FEA_CUDA_ERROR; }
   cudaDeviceGetAttribute(&ctx->c.sm_count, cudaDevAttrMultiProcessorCount, device);
-  if (const char* v = getenv("FEA_SPMV_VARIANT")) ctx->c.spmv_variant = atoi(v);
   cudaMemPool_t pool;
   if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
     uint64_t thr = UINT64_MAX;
     cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
   }
-  if (const char* v = getenv("FEA_NO_GRAPHS")) ctx->c.use_graphs = atoi(v) ? 0 : 1;
-  if (const char* v = getenv("FEA_ROW_ORDER")) ctx->c.row_order = atoi(v);
-  if (const char* v = getenv("FEA_CLUSTER_MIN")) ctx->c.cluster_min = std::max(1, std::min(8, atoi(v)));
-  if (const char* v = getenv("FEA_PCG_PATH")) ctx->c.pcg_path = (strcmp(v, "stream") == 0 || atoi(v) == 1) ? 1 : 0;
   if (cudaHostAlloc((void**)&ctx->c.h_flag, 8 * sizeof(int32_t), cudaHostAllocDefault) != cudaSuccess ||
       cudaMalloc(&ctx->c.d_pcg_params, kPcgParamBytes) != cudaSuccess) {
     if (ctx->c.h_flag) cudaFreeHost(ctx->c.h_flag);
@@ -273,8 +268,6 @@ int fea_ctx_create_prio(int device, int priority, fea_ctx** out) {
     cudaStreamCreateWithPriority(&ctx->c.aux[i], cudaStreamNonBlocking, std::max(hi, priority - 1 - i));
     cudaEventCreateWithFlags(&ctx->c.ev_join[i], cudaEventDisableTiming);
   }
-  ctx->c.prio_lo = priority;
-  ctx->c.prio_hi = hi;
   cudaEventCreate(&ctx->c.ev_c0);
   cudaEventCreate(&ctx->c.ev_c1);
   for (auto& ev : ctx->ev_user) cudaEventCreate(&ev);
@@ -300,8 +293,6 @@ int fea_ctx_destroy(fea_ctx* ctx) {
     cudaEventDestroy(ctx->c.ev_join[i]);
     if (ctx->c.aux[i]) cudaStreamDestroy(ctx->c.aux[i]);
   }
-  for (auto& st : ctx->c.prio_streams)
-    if (st) cudaStreamDestroy(st);
   cudaEventDestroy(ctx->c.ev_c0);
   cudaEventDestroy(ctx->c.ev_c1);
   for (auto& ev : ctx->ev_user) cudaEventDestroy(ev);
@@ -382,11 +373,8 @@ int fea_ctx_set_int(fea_ctx* ctx, const char* key, int64_t value) {
   if (strcmp(key, "pcg_path") == 0) ctx->c.pcg_path = value == 1 ? 1 : 0;
   else if (strcmp(key, "row_order") == 0) ctx->c.row_order = (value >= 1 && value <= 3) ? (int)value : 0;
   else if (strcmp(key, "cluster_halo_cap") == 0) ctx->c.cluster_halo_cap = value < 0 ? 0 : value > (1 << 30) ? (1 << 30) : (int)value;
-  else if (strcmp(key, "cluster_prio") == 0) ctx->c.cluster_prio = (int)value;
   else if (strcmp(key, "cluster_min") == 0) ctx->c.cluster_min = value < 1 ? 1 : value > 8 ? 8 : (int)value;
   else if (strcmp(key, "refine_rounds") == 0) ctx->c.refine_rounds = value < 0 ? 0 : value > 8 ? 8 : (int)value;
-  else if (strcmp(key, "spmv_variant") == 0) ctx->c.spmv_variant = (int)value;
-  else if (strcmp(key, "use_graphs") == 0) ctx->c.use_graphs = value ? 1 : 0;
   else return api_fail(ctx, FEA_BAD_ARG, "unknown option key");
   return FEA_OK;
 }

@@ -30,12 +30,11 @@ struct Ctx {
   // PCG driver state, owned by the context so that CUDA graphs survive across solves
   int32_t* h_flag = nullptr;           // pinned [8]: polled counters
   void* d_pcg_params = nullptr;        // device copy of the current solve's PcgPtrs
-  std::map<int64_t, cudaGraphExec_t> pcg_graphs;  // key: grid size class * 2 + two_level
+  std::map<int64_t, cudaGraphExec_t> pcg_graphs;  // key: grid size class * 2 + L2 hints of the SpMV
   std::vector<cudaEvent_t> events;     // 3 per timed launch
   cudaEvent_t ev_poll[2] = {nullptr, nullptr};
   cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;
   cudaEvent_t ev_c0 = nullptr, ev_c1 = nullptr;  // around the cluster-path kernel
-  int use_graphs = 1;                  // env FEA_NO_GRAPHS=1 disables
   int refine_rounds = 1;               // restarts from the true residual per solve (0 = check only)
   int pcg_path = 0;                    // 0 = auto (on-chip cluster kernel where systems fit), 1 = streaming only
   int cluster_capacity[9] = {-1, -1, -1, -1, -1, -1, -1, -1, -1};  // co-resident clusters of c CTAs (-1 = not queried)
@@ -45,11 +44,6 @@ struct Ctx {
   static constexpr int kAux = 8;       // one stream per cluster class (1..8) beside the main stream
   cudaStream_t aux[kAux] = {};         // cluster kernels of different classes run concurrently
   cudaEvent_t ev_fork = nullptr, ev_join[kAux] = {};
-  int prio_lo = 0, prio_hi = 0;        // least / most urgent stream priority this context may use
-  cudaStream_t prio_streams[9] = {};   // (cluster_prio knob) stream of class k at its chosen urgency, made on demand
-  int prio_streams_key = 0;
-  int cluster_prio = 0;                // tuning knob: decimal digit k (from the right) = urgency 1 (the device's least urgent level) .. 6 of class k, 0 = default rule
-  int spmv_variant = 0;  // tuning knob (env FEA_SPMV_VARIANT), 0 = default
   int64_t launches = 0;  // kernels launched (bookkeeping for bench.py's gpu_launches)
 };
 
@@ -264,8 +258,8 @@ cudaError_t launch_csr_export(Batch& b, int32_t s, int32_t* d_indptr, int32_t* d
 cudaError_t run_pcg(Batch& b, double rtol, int max_iter);
 void pcg_release(Ctx& c);                                     // destroys the cached graphs
 int pcg_cluster_class(int64_t n_vertices_of_sample, int min_cl);  // CTAs per cluster (1..8), 0: streaming
-int pcg_cluster_capacity(Ctx& c, int cl);
-int pcg_cluster_rows_per_cta();                               // block rows a CTA of the on-chip path holds                     // co-resident clusters (0 = unavailable)
+int pcg_cluster_capacity(Ctx& c, int cl);                     // co-resident clusters of cl CTAs (0 = unavailable)
+int pcg_cluster_rows_per_cta();                               // block rows a CTA of the on-chip path holds
 struct PcgPtrs;
 cudaError_t launch_pcg_cluster(Ctx& c, const PcgPtrs* dP, int n_systems, int cl, cudaStream_t st);
 cudaError_t launch_finalize(Batch& b);                        // u, ranges, max-iter status

@@ -92,13 +92,13 @@ __device__ __forceinline__ double sum_partials(const double* __restrict__ part, 
 }
 
 
-// U = entries whose loads are issued together before any of them is consumed (memory-level
-// parallelism per thread); MINB = minimum resident CTAs per SM asked of the register allocator.
 // Grid = any size >= P.n_active (the host picks a size class from a slightly stale count).
+// 16 resident CTAs per SM (a 32-register budget): the SpMV of a single ~1 M-DOF system is latency-bound
+// and needs full occupancy.
 // HINT: L2 eviction policies on the loads (matrix evict_first, gathered records evict_last) for systems
 // whose matrix does not fit the L2.
-template <int U, int MINB, bool HINT = false>
-__global__ void __launch_bounds__(kT, MINB) k_pcg_spmv(const PcgPtrs* __restrict__ Pp, int parity) {
+template <bool HINT>
+__global__ void __launch_bounds__(kT, 16) k_pcg_spmv(const PcgPtrs* __restrict__ Pp, int parity) {
   __shared__ double sm[kT / 32];
   const PcgPtrs& P = *Pp;
   if ((int)blockIdx.x >= P.n_active) return;
@@ -138,50 +138,21 @@ __global__ void __launch_bounds__(kT, MINB) k_pcg_spmv(const PcgPtrs* __restrict
   const double2 pn = make_double2(fma(beta, own.z, own.x), fma(beta, own.w, own.y));
   double a0 = pn.x, a1 = pn.y;   // the diagonal block of Khat is the identity
 #pragma unroll 1
-  for (int j0 = 0; j0 < L; j0 += U) {
-    int c[U];
-    d4 k[U], g[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u)
-      c[u] = (j0 + u < L) ? (HINT ? ld_stream_i32_hint(cp + (j0 + u) * 32, pol_m) : ld_stream_i32(cp + (j0 + u) * 32)) : (int)row;
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      k[u].x = k[u].y = k[u].z = k[u].w = 0.0;
-      if (j0 + u < L) k[u] = HINT ? ld_stream_d4_hint(vt + (j0 + u) * 32, pol_m) : ld_stream_d4(vt + (j0 + u) * 32);
-    }
-#pragma unroll
-    for (int u = 0; u < U; ++u) g[u] = HINT ? ld_nc_d4_hint(rp + c[u], pol_v) : ld_nc_d4(rp + c[u]);
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const double px = fma(beta, g[u].z, g[u].x);
-      const double py = fma(beta, g[u].w, g[u].y);
-      a0 = fma(k[u].x, px, a0);
-      a0 = fma(k[u].y, py, a0);
-      a1 = fma(k[u].z, px, a1);
-      a1 = fma(k[u].w, py, a1);
-    }
+  for (int j = 0; j < L; ++j) {
+    const int c = HINT ? ld_stream_i32_hint(cp + j * 32, pol_m) : ld_stream_i32(cp + j * 32);
+    const d4 k = HINT ? ld_stream_d4_hint(vt + j * 32, pol_m) : ld_stream_d4(vt + j * 32);
+    const d4 g = HINT ? ld_nc_d4_hint(rp + c, pol_v) : ld_nc_d4(rp + c);
+    const double px = fma(beta, g.z, g.x);
+    const double py = fma(beta, g.w, g.y);
+    a0 = fma(k.x, px, a0);
+    a0 = fma(k.y, py, a0);
+    a1 = fma(k.z, px, a1);
+    a1 = fma(k.w, py, a1);
   }
   P.q[row] = make_double2(a0, a1);
   const double part = cta_sum(fma(pn.x, a0, pn.y * a1), sm);
   if (threadIdx.x == 0) P.partA[cta] = part;
   if (P.two_level) presum_if_last(P.partA, first, w.w, P.sc.arrive + 2 * s, P.sc.psumA + s, sm);
-}
-
-typedef void (*spmv_fn)(const PcgPtrs*, int);
-static spmv_fn pick_spmv(int variant) {
-  switch (variant) {  // "spmv_variant" option = 100 * U + MINB (tuning knob; measured on B200: 116 best)
-    case 112: return k_pcg_spmv<1, 12>;
-    case 216: return k_pcg_spmv<2, 16>;
-    case 212: return k_pcg_spmv<2, 12>;
-    case 210: return k_pcg_spmv<2, 10>;
-    case 408: return k_pcg_spmv<4, 8>;
-    case 406: return k_pcg_spmv<4, 6>;
-    case 308: return k_pcg_spmv<3, 8>;
-    case 1116: return k_pcg_spmv<1, 16, true>;
-    case 1212: return k_pcg_spmv<2, 12, true>;
-    case 1408: return k_pcg_spmv<4, 8, true>;
-    default: return k_pcg_spmv<1, 16>;
-  }
 }
 
 __global__ void __launch_bounds__(kT) k_pcg_update(const PcgPtrs* __restrict__ Pp, int parity) {
@@ -465,8 +436,8 @@ static PcgPtrs make_ptrs(Batch& b, int max_iter) {
 }
 
 // one iteration = two kernels on a grid of g CTAs
-static void launch_iteration(Ctx& c, const PcgPtrs* dP, int g, int parity, cudaStream_t st, int variant) {
-  pick_spmv(variant)<<<g, kT, 0, st>>>(dP, parity);
+static void launch_iteration(const PcgPtrs* dP, int g, int parity, cudaStream_t st, bool hint) {
+  (hint ? k_pcg_spmv<true> : k_pcg_spmv<false>)<<<g, kT, 0, st>>>(dP, parity);
   k_pcg_update<<<g, kT, 0, st>>>(dP, parity);
 }
 
@@ -478,14 +449,14 @@ static int grid_class(int n_active, int ncta) {
   return gi < ncta ? gi : ncta;
 }
 
-static cudaError_t get_chunk_graph(Ctx& c, const PcgPtrs* dP, int g, int variant, cudaGraphExec_t* out) {
-  const int64_t key = ((int64_t)g << 32) | (int64_t)(uint32_t)variant;   // the SpMV variant is baked into the kernel nodes
+static cudaError_t get_chunk_graph(Ctx& c, const PcgPtrs* dP, int g, bool hint, cudaGraphExec_t* out) {
+  const int64_t key = 2 * (int64_t)g + (hint ? 1 : 0);   // the SpMV instantiation is baked into the kernel nodes
   auto it = c.pcg_graphs.find(key);
   if (it != c.pcg_graphs.end()) { *out = it->second; return cudaSuccess; }
   cudaGraph_t graph = nullptr;
   cudaError_t e = cudaStreamBeginCapture(c.stream, cudaStreamCaptureModeThreadLocal);
   if (e != cudaSuccess) return e;
-  for (int i = 2; i < kChunk; ++i) launch_iteration(c, dP, g, i & 1, c.stream, variant);
+  for (int i = 2; i < kChunk; ++i) launch_iteration(dP, g, i & 1, c.stream, hint);
   k_compact_active<<<1, 1024, 0, c.stream>>>((PcgPtrs*)dP);
   e = cudaStreamEndCapture(c.stream, &graph);
   if (e != cudaSuccess) return e;
@@ -523,8 +494,7 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
   }
   const int per_iter = 2;
   // L2 eviction hints (matrix evict_first, gathered records evict_last) when the matrix does not fit the L2
-  int variant = c.spmv_variant;
-  if (variant == 0 && (int64_t)b.n_blocks * 36 > (int64_t)96 << 20) variant = 1116;
+  const bool hint = (int64_t)b.n_blocks * 36 > (int64_t)96 << 20;
   int64_t launches = 0;
   cudaError_t e;
   b.stats = fea_solve_stats{};
@@ -540,39 +510,20 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
   if (n_cluster > 0) {  // systems that fit on chip: one per cluster, pulled from a queue
     cudaMemsetAsync(b.cl_counter, 0, 24 * sizeof(int32_t), st);
     cudaEventRecord(c.ev_c0, st);
-    // one persistent kernel per cluster class, largest clusters first; classes are spread over the
-    // main stream and three auxiliary streams so that their clusters are co-scheduled and small
-    // clusters fill the SMs that larger ones cannot use (GPC granularity)
+    // one persistent kernel per cluster class, largest clusters first; the largest class runs on the
+    // main stream, every other one on an auxiliary stream of its own (more urgent the smaller its
+    // clusters, fea_ctx_create), so that their clusters are co-scheduled and small clusters fill the
+    // SMs that larger ones cannot use (GPC granularity)
     cudaEventRecord(c.ev_fork, st);
     bool used[Ctx::kAux] = {};
-    cudaStream_t aux_of[Ctx::kAux];
-    for (int a = 0; a < Ctx::kAux; ++a) aux_of[a] = c.aux[a];
-    if (c.cluster_prio != c.prio_streams_key) {   // tuning knob changed: streams at the requested urgencies
-      for (auto& s2 : c.prio_streams) { if (s2) cudaStreamDestroy(s2); s2 = nullptr; }
-      c.prio_streams_key = c.cluster_prio;
-    }
     int slot = 0;
     for (int k = 8; k >= 1; --k) {
       if (!P.cl_cnt[k]) continue;
       cudaStream_t ks = st;
-      int a = -1;
-      if (c.cluster_prio) {
-        int digit = c.cluster_prio;
-        for (int i = 1; i < k; ++i) digit /= 10;
-        digit %= 10;
-        if (digit > 0) {
-          if (!c.prio_streams[k]) {
-            const int pr = -(digit - 1) < c.prio_hi ? c.prio_hi : -(digit - 1);   // absolute: 1 = the device's least urgent level
-            cudaStreamCreateWithPriority(&c.prio_streams[k], cudaStreamNonBlocking, pr);
-          }
-          a = k - 1;                                 // join-event slot of this class
-          aux_of[a] = c.prio_streams[k];
-        }
-      }
-      if (a < 0 && slot > 0 && c.aux[slot - 1]) a = slot - 1;
-      if (a >= 0) {
-        ks = aux_of[a];
-        if (!used[a]) cudaStreamWaitEvent(ks, c.ev_fork, 0);
+      const int a = slot - 1;   // auxiliary stream of this class
+      if (a >= 0 && c.aux[a]) {
+        ks = c.aux[a];
+        cudaStreamWaitEvent(ks, c.ev_fork, 0);
         used[a] = true;
       }
       if ((e = launch_pcg_cluster(c, dP, P.cl_cnt[k], k, ks)) != cudaSuccess) return e;
@@ -581,7 +532,7 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
     }
     for (int a = 0; a < Ctx::kAux; ++a) {
       if (!used[a]) continue;
-      cudaEventRecord(c.ev_join[a], aux_of[a]);
+      cudaEventRecord(c.ev_join[a], c.aux[a]);
       cudaStreamWaitEvent(st, c.ev_join[a], 0);
     }
     cudaEventRecord(c.ev_c1, st);
@@ -623,20 +574,15 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
     for (; k < k_end; ++k) {
       const int g = grid_class(n_active, ncta);
       cudaGraphExec_t exec = nullptr;
-      if (c.use_graphs && (e = get_chunk_graph(c, dP, g, variant, &exec)) != cudaSuccess) return e;
+      if ((e = get_chunk_graph(c, dP, g, hint, &exec)) != cudaSuccess) return e;
       const bool t = timed < kMaxTimed;
       if (t) cudaEventRecord(c.events[3 * timed], st);
-      pick_spmv(variant)<<<g, kT, 0, st>>>(dP, 0);
+      (hint ? k_pcg_spmv<true> : k_pcg_spmv<false>)<<<g, kT, 0, st>>>(dP, 0);
       if (t) cudaEventRecord(c.events[3 * timed + 1], st);
       k_pcg_update<<<g, kT, 0, st>>>(dP, 0);
       if (t) { cudaEventRecord(c.events[3 * timed + 2], st); ++timed; }
-      launch_iteration(c, dP, g, 1, st, variant);
-      if (exec) {
-        if ((e = cudaGraphLaunch(exec, st)) != cudaSuccess) return e;
-      } else {
-        for (int i = 2; i < kChunk; ++i) launch_iteration(c, dP, g, i & 1, st, variant);
-        k_compact_active<<<1, 1024, 0, st>>>(dP);
-      }
+      launch_iteration(dP, g, 1, st, hint);
+      if ((e = cudaGraphLaunch(exec, st)) != cudaSuccess) return e;
       launches += (int64_t)per_iter * kChunk + 1;
       if ((k - k_first + 1) % mon_chunks == 0) {   // periodic true-residual monitor (see k_pcg_true_residual)
         k_pcg_true_residual<<<ncta, kT, 0, st>>>(dP, b.vertex_of_row, b.rhs, b.dscale, b.scoup, 1);
@@ -883,7 +829,7 @@ cudaError_t launch_plain_spmv(Batch& b, int32_t s, const double* d_x, double* d_
   k_compact_active<<<1, 1024, 0, st>>>(dP);
   k_spmv_load<<<g, T, 0, st>>>(b.NBR, b.vertex_of_row, b.vrank, v0, v1, b.dscale, b.scoup, d_x, (d4*)b.rp);
   cudaMemsetAsync(b.sc.arrive, 0, sizeof(int32_t) * 2 * b.ns, st);
-  pick_spmv(b.ctx->spmv_variant)<<<ncta, kT, 0, st>>>(dP, 0);
+  k_pcg_spmv<false><<<ncta, kT, 0, st>>>(dP, 0);
   k_spmv_store<<<g, T, 0, st>>>(b.NBR, b.vertex_of_row, b.vrank, v0, v1, b.dscale, b.scoup, (const double2*)b.q, d_y);
   return cudaGetLastError();
 }

@@ -68,47 +68,15 @@ __device__ __forceinline__ unsigned long long gtime() {
 #endif
 
 constexpr int kClMax = 8;                   // largest cluster (portable maximum)
-#ifndef FEA_CL_THREADS
-#define FEA_CL_THREADS 512
-#endif
-constexpr int kClT = FEA_CL_THREADS;        // threads per CTA
+constexpr int kClT = 512;                   // threads per CTA (one CTA per SM)
 constexpr int kClW = kClT / 32;             // warps per CTA
-#ifndef FEA_CL_CTAS_PER_SM
-#define FEA_CL_CTAS_PER_SM 1
-#endif
-#ifndef FEA_CL_RPT
-#define FEA_CL_RPT 4
-#endif
-constexpr int kClRpt = FEA_CL_RPT;          // block rows per thread
-#ifndef FEA_CL_UNROLL
-#define FEA_CL_UNROLL 4
-#endif
-constexpr int kClU = FEA_CL_UNROLL;         // gathers in flight per thread (resident slices)
-#ifndef FEA_CL_UNROLL_STREAM
-#define FEA_CL_UNROLL_STREAM 4
-#endif
-constexpr int kClUs = FEA_CL_UNROLL_STREAM; // blocks in flight per thread (slices streamed from L2)
+constexpr int kClRpt = 4;                   // block rows per thread
+constexpr int kClU = 4;                     // gathers in flight per thread (resident slices)
+constexpr int kClUs = 4;                    // blocks in flight per thread (slices streamed from L2)
 static_assert(kClU % 4 == 0 && kClUs % 4 == 0, "gather codes are fetched four at a time");
-#ifndef FEA_CL_MONITOR
-#define FEA_CL_MONITOR 1024
-#endif
-
-#ifndef FEA_CL_TMEM
-#define FEA_CL_TMEM 1
-#endif
-// The scaled diagonal block is the identity, so a row's product starts from q = p.  FEA_CL_DCS = 1 (A/B build)
-// keeps the per-row coupling array of the point-Jacobi layout (all zeros) and its two FMAs in the SpMV: with
-// ptxas' own unrolling of the block loops that build was the faster one (27.5 against 28.0 ms: different
-// register allocation), with the loops kept rolled both take 26.4 ms.  Same bits either way.
-#ifndef FEA_CL_DCS
-#define FEA_CL_DCS 0
-#endif
-#ifndef FEA_CL_ONE_DIV
-#define FEA_CL_ONE_DIV 1
-#endif
-constexpr int kMonitor = FEA_CL_MONITOR;    // iterations between true-residual monitor passes
+constexpr int kMonitor = 1024;              // iterations between true-residual monitor passes
 constexpr int kClSlices = kClT / 32 * kClRpt;  // local slices per CTA (64 with 512 threads)
-constexpr int kClSmemBytes = (FEA_CL_CTAS_PER_SM == 1 ? 227 : 113) * 1024;  // dynamic shared memory per CTA
+constexpr int kClSmemBytes = 227 * 1024;    // dynamic shared memory per CTA: all an SM has
 constexpr int kClWords = (kClMax * kClSlices + kClT - 1) / kClT * kClT;   // 32-row slices of the largest system = words of the halo bitmap (padded to whole threads)
 static_assert(kClWords % kClT == 0 && kClSlices <= kClT && kClSlices * 32 <= 4096, "the halo scan handles kClWords / kClT bitmap words per thread");
 constexpr int kClWpt = kClWords / kClT;     // bitmap words per thread (consecutive)
@@ -119,9 +87,9 @@ constexpr int kClTmpBytes = 2 * kClWords * 4 + 128;   // halo bitmap + its prefi
 // 456 B/clk/SM into registers, and beside saturating ld.shared traffic both run at 120 B/clk/SM -- TMEM reads
 // do not use the L1TEX data pipe that bounds this kernel, while blocks streamed from L2 do (at 61 B/clk/SM).
 // A warp may only touch the 32 lanes of its quadrant (warp % 4); the warps of a quadrant split the columns.
-constexpr int kTmCols = FEA_CL_TMEM ? 512 / FEA_CL_CTAS_PER_SM : 0;        // columns allocated per CTA (power of two)
-constexpr int kTmWarpCols = FEA_CL_TMEM ? kTmCols / (kClW / 4) / 8 * 8 : 0;  // columns of one warp's strip
-constexpr int kTmWarpBlocks = kTmWarpCols / 8;                               // 2x2 blocks per lane in that strip
+constexpr int kTmCols = 512;                             // columns allocated per CTA: all of the SM's TMEM (a power of two)
+constexpr int kTmWarpCols = kTmCols / (kClW / 4) / 8 * 8;  // columns of one warp's strip
+constexpr int kTmWarpBlocks = kTmWarpCols / 8;             // 2x2 blocks per lane in that strip
 static_assert(kClW % 4 == 0, "TMEM strips are per quadrant of four warps");
 
 struct ClHeader {                 // start of the dynamic shared memory of every CTA
@@ -130,7 +98,7 @@ struct ClHeader {                 // start of the dynamic shared memory of every
   // table a slower warp is still summing, nor complete bytes on a phase that has not opened yet
   alignas(32) double partA[2][kClMax * kClW * 4];
   double partB[kClMax * kClW];    // r.r partials of the true-residual passes (check / monitor / refinement)
-  double rz_zero;                 // (A/B build FEA_CL_DCS == 2) 0.0
+  double pad1_;                   // unused; without it ptxas allocates one more register in some k_pcg_cluster<CL>
   double rz_monitor;              // smallest true r.r any monitor pass has seen
   double tol2;                    // rtol^2 * r0.r0 of the current system (tightened by an extended-precision round)
   int32_t mon_strikes;            // consecutive monitor passes without a 4x gain on rz_monitor
@@ -405,7 +373,7 @@ constexpr double kRefineTighten = 1e-4;  // a refined system is solved to rtol /
                                          // amplifies the residual into the displacement (measured: 200x)
 
 template <int CL>
-__global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const PcgPtrs* __restrict__ Pp) {
+__global__ void __launch_bounds__(kClT, 1) k_pcg_cluster(const PcgPtrs* __restrict__ Pp) {
   constexpr int kCl = CL;
   constexpr int kClass = CL;
   extern __shared__ __align__(128) unsigned char smem[];
@@ -429,17 +397,15 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   // (the first cluster.sync() of the queue loop orders the initialisation before any push)
-  uint32_t tm_strip = 0;   // this warp's TMEM strip: lanes of its quadrant, its share of the columns
-  if (kTmCols) {
-    if (warp == 0) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&h->tmem_base)), "n"(kTmCols > 0 ? kTmCols : 32) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    tm_strip = h->tmem_base + ((uint32_t)(warp & 3) * 32u << 16) + (uint32_t)(warp >> 2) * (uint32_t)kTmWarpCols;
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&h->tmem_base)), "n"(kTmCols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  // this warp's TMEM strip: lanes of its quadrant, its share of the columns
+  const uint32_t tm_strip = h->tmem_base + ((uint32_t)(warp & 3) * 32u << 16) + (uint32_t)(warp >> 2) * (uint32_t)kTmWarpCols;
 
   for (;;) {
     // ---- next system of the queue (rank 0 pulls, everyone reads it through DSMEM) --------------
@@ -541,7 +507,7 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
       int ent = 0;
       for (int i = 0; i < kClSlices; ++i) { h->s_aoff[i] = ent; ent += (h->s_len[i] + 3) / 4 * 128; }
       const int off_pbuf = kHdr + (4 * S + 127) / 128 * 128;
-      const int mat0 = (off_pbuf + 16 * (Rc + H) + (FEA_CL_DCS == 1 ? 8 * Rc : 0) + 127) / 128 * 128;
+      const int mat0 = (off_pbuf + 16 * (Rc + H) + 127) / 128 * 128;
       int off = (ent * 2 + 127) / 128 * 128;
       const int fit = (mat0 + off <= kClSmemBytes - kClTmpBytes && Rc + H <= 0xffff && H <= P.cl_halo_cap) ? 1 : 0;
       h->off_pbuf = off_pbuf;
@@ -578,9 +544,6 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
     }
     const int off_pbuf = h->off_pbuf, mat0 = h->mat0;
     double2* pbuf = reinterpret_cast<double2*>(smem + off_pbuf);   // [Rc] published p + [H] halo
-#if FEA_CL_DCS == 1
-    double* dcs = reinterpret_cast<double*>(pbuf + Rc + H);        // (A/B build) [Rc] zeros read like the former diagonal couplings
-#endif
     const uint32_t pbuf_a = smem_u32(pbuf);
     uint16_t* sa_all = reinterpret_cast<uint16_t*>(smem + mat0);
     const uint32_t* sendl = reinterpret_cast<const uint32_t*>(smem + kHdr);
@@ -659,7 +622,7 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
         sb[(j - nt) * 32 + lane] = make_double2(blk.z, blk.w);
       }
     }
-    if (kTmCols) asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 
     // ---- vectors of the thread's rows in registers ----------------------------------------------
     double2 x[kClRpt], r[kClRpt];   // p lives in pbuf (its owner is the only writer)
@@ -674,9 +637,6 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
         const d4 rec = P.rp[my_row0 + lr];   // r0 = S b (k_pcg_init_vectors)
         r[k] = make_double2(rec.x, rec.y);
         pbuf[lr] = r[k];                     // first direction p = r
-#if FEA_CL_DCS == 1
-        dcs[lr] = 0.0;
-#endif
       }
     }
 #ifdef FEA_CLUSTER_PROFILE
@@ -692,7 +652,6 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
       h->it_limit = P.max_iter;
       h->rz_monitor = inf;                    // smallest true r.r found by a monitor pass
       h->mon_strikes = 0;
-      h->rz_zero = 0.0;
     }
     __syncthreads();
     int iters = 0, status = FEA_SAMPLE_NOT_RUN;
@@ -751,18 +710,8 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
         double a0 = 0.0, a1 = 0.0;
         if (ls < my_sl) {
           const double2 pk = pbuf[tid + kClT * k];   // the diagonal block of Khat is the identity
-#if FEA_CL_DCS == 1
-          const double dck = dcs[tid + kClT * k];
-          a0 = fma(dck, pk.y, pk.x);
-          a1 = fma(dck, pk.x, pk.y);
-#elif FEA_CL_DCS == 2
-          const double dck = h->rz_zero;
-          a0 = fma(dck, pk.y, pk.x);
-          a1 = fma(dck, pk.x, pk.y);
-#else
           a0 = pk.x;
           a1 = pk.y;
-#endif
           const int L = h->s_len[ls];
           const int off = h->s_off[ls];
           const uint2* sa = reinterpret_cast<const uint2*>(sa_all + h->s_aoff[ls]) + lane;   // 4 codes per load
@@ -771,7 +720,7 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
             mbar_wait(smem_u32(&h->mbarP), (phase >> 2) & 1u);
             halo_here = true;
           }
-          const int nt = kTmCols ? h->s_nt[ls] : 0;
+          const int nt = h->s_nt[ls];
           if (nt > 0) {   // leading blocks from tensor memory: their own datapath, not the L1TEX pipe
             const uint32_t tcol = tm_strip + (uint32_t)h->s_tcol[ls];
             d4 kv[4];
@@ -881,9 +830,8 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
         PROF_T(3);
         double pq, qq, rq;
         sum_records<CL>(h->partA[ab], lane, pq, qq, rq, rz);     // rz = r.r of the current residual, exact
-#if FEA_CL_ONE_DIV
         const double ipq = 1.0 / pq;                             // (started before the exit tests: it is the longest
-#endif                                                           //  scalar dependency of the iteration)
+                                                                 //  scalar dependency of the iteration)
         PROF_T(4);
         bool check = false, monitor = false;
 #ifdef FEA_CLUSTER_DEBUG
@@ -912,18 +860,11 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
           continue;
         }
         if (!(pq > 0.0 && isfinite(pq))) { status = FEA_SAMPLE_BREAKDOWN; break; }
-#if FEA_CL_ONE_DIV
-        // one division (fp64 division is ~150 cycles of dependent instructions that every warp repeats; measured
-        // 29.9 -> 28.1 ms per 400-system batch against alpha = rz / pq, beta = est / rz):
+        // one division (fp64 division is ~150 cycles of dependent instructions that every warp repeats):
         //   alpha = rz / pq;  beta = |r - alpha q|^2 / rz = 1 + (rz qq / pq - 2 rq) / pq
         const double alpha = rz * ipq;
         const double b1 = fma(fma(rz * qq, ipq, -2.0 * rq), ipq, 1.0);
         const double beta = b1 > 0.0 ? b1 : 0.0;
-#else
-        const double alpha = rz / pq;
-        const double est = fma(alpha * alpha, qq, fma(-2.0 * alpha, rq, rz));   // |r - alpha q|^2
-        const double beta = est > 0.0 ? est / rz : 0.0;
-#endif
 #pragma unroll
         for (int k = 0; k < kClRpt; ++k) {
           if (own[k]) {
@@ -1071,7 +1012,7 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
     if (tid == 0) {   // where this CTA read its blocks from (bench: bytes through the shared-memory pipe / TMEM / L2)
       long long nb[3] = {0, 0, 0};
       for (int i = 0; i < my_sl; ++i) {
-        const int L = h->s_len[i], nt = min(kTmCols ? h->s_nt[i] : 0, L);
+        const int L = h->s_len[i], nt = min(h->s_nt[i], L);
         nb[0] += 32 * nt;
         nb[h->s_off[i] >= 0 ? 1 : 2] += 32 * (L - nt);
       }
@@ -1102,10 +1043,9 @@ __global__ void __launch_bounds__(kClT, FEA_CL_CTAS_PER_SM) k_pcg_cluster(const 
 #ifdef FEA_CLUSTER_ACCOUNT
   if (tid == 0) atomicAdd(&g_cl_prof[13], (unsigned long long)(clock64() - acc_t0));
 #endif
-  if (kTmCols) {   // every CTA must give its tensor memory back: the next CTA on this SM allocates all of it
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(h->tmem_base), "n"(kTmCols > 0 ? kTmCols : 32) : "memory");
-  }
+  // every CTA must give its tensor memory back: the next CTA on this SM allocates all of it
+  __syncthreads();
+  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(h->tmem_base), "n"(kTmCols) : "memory");
 }
 
 typedef void (*cluster_fn)(const PcgPtrs*);

@@ -349,7 +349,7 @@ class Context:
 
     def set_option(self, key: str, value: int):
         """fea_ctx_set_int: "pcg_path" (0 auto / 1 streaming kernels only), "cluster_min", "cluster_halo_cap",
-        "row_order", "refine_rounds", "spmv_variant", "use_graphs" (include/fea_b200.h)."""
+        "row_order", "refine_rounds" (include/fea_b200.h)."""
         self._check(self.lib.fea_ctx_set_int(self.h, key.encode("ascii"), int(value)))
 
     def kernel_launches(self) -> int:

@@ -216,11 +216,7 @@ int  fea_ctx_wait_ctx(fea_ctx* ctx, fea_ctx* other);
  *   "cluster_halo_cap"  test knob: the largest number of rows a CTA of the on-chip path accepts
  *                   from its cluster peers (default: whatever fits its shared memory); a system
  *                   above it is handed back to the streaming kernels
- *   "cluster_prio"  tuning knob: stream urgency of the persistent kernel of each cluster class; decimal
- *                   digit k from the right = urgency 1 (least) .. 6 of the k-CTA class, 0 = default rule
- *                   (the smaller the cluster the more urgent).  It decides when a system is solved,
- *                   never its bits
- *   "spmv_variant"  tuning knob of k_pcg_spmv;  "use_graphs" 0/1 (streaming path) */
+ * any other key fails with FEA_BAD_ARG */
 int  fea_ctx_set_int(fea_ctx* ctx, const char* key, int64_t value);
 /* number of kernels this context has launched so far (graph nodes included) */
 int  fea_ctx_kernel_launches(fea_ctx* ctx, int64_t* out);

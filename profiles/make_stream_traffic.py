@@ -34,7 +34,7 @@ c3 = {}
 for r in csv.reader(open(os.path.join(here, "%s_c3_traffic.csv" % tag))):
     if len(r) > 14 and r[0].isdigit():
         c3.setdefault(re.sub(r"^void\s+|\(.*", "", r[4]), {}).setdefault(r[12], []).append(float(r[14]))
-out = {"source": "profiles/%s_c3_traffic.csv (ncu --metrics dram bytes / time, 4 iterations of tools/tune_spmv_c3.py 0 cantilever 4)" % tag}
+out = {"source": "profiles/%s_c3_traffic.csv (ncu --metrics dram bytes / time, 4 iterations of tools/tune_spmv_c3.py cantilever 4)" % tag}
 for k, m in c3.items():
     mean = lambda name: sum(m[name]) / len(m[name])
     us = mean("gpu__time_duration.sum") * 1e-3

@@ -28,7 +28,7 @@ echo "full capture rc=$?"
 ncu --set full --clock-control none --import-source on -k "regex:k_pcg_spmv|k_pcg_update" -s 40 -c 6 \
     -f -o gpurun_out/${TAG}_stream $CMD > gpurun_out/${TAG}_ncu4.log 2>&1
 echo "streaming capture rc=$?"
-C3="python tools/tune_spmv_c3.py 0 cantilever 4"
+C3="python tools/tune_spmv_c3.py cantilever 4"
 ITERS=256 $C3 > gpurun_out/${TAG}_c3_plain.log 2>&1 &&
 ITERS=256 ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum,lts__t_sectors.sum \
     --clock-control none -k "regex:k_pcg_spmv|k_pcg_update" -s 200 -c 8 --csv \

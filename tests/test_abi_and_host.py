@@ -141,14 +141,15 @@ def test_pack_layout():
 
 
 def test_every_context_option_is_documented_in_the_header():
-    """fea_ctx_set_int keys accepted by the library (csrc/fea_api.cu) are all described in include/fea_b200.h."""
+    """fea_ctx_set_int accepts exactly the five options that select a path real inputs also reach
+    (csrc/fea_api.cu), and include/fea_b200.h describes each of them."""
     import re
     root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
     src = open(os.path.join(root, "fea_diffusion_b200", "csrc", "fea_api.cu")).read()
     body = src[src.index("int fea_ctx_set_int("):]
     body = body[:body.index("\n}\n")]
     keys = set(re.findall(r'strcmp\(key, "([a-z_]+)"\)', body))
-    assert {"pcg_path", "cluster_min", "cluster_halo_cap", "row_order"} <= keys
+    assert keys == {"pcg_path", "cluster_min", "cluster_halo_cap", "row_order", "refine_rounds"}
     header = open(os.path.join(root, "include", "fea_b200.h")).read()
     missing = [k for k in sorted(keys) if '"%s"' % k not in header]
     assert not missing, missing

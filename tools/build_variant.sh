@@ -1,7 +1,8 @@
 #!/bin/bash
-# Build a variant of libfea_b200.so with extra nvcc flags for k_pcg_cluster.cu / k_pcg.cu only
-# (tuning experiments; the other objects come from the regular build).
-#   tools/build_variant.sh <name> [-DFLAG=V ...]   ->  build/variants/lib_<name>.so
+# Build an instrumented libfea_b200.so: k_pcg_cluster.cu / k_pcg.cu with extra nvcc flags, the other
+# objects from the regular build.  The flags are FEA_CLUSTER_PROFILE / ACCOUNT / TRACE / DEBUG, which
+# only observe the solver (cycle counts, per-system timeline, printf); see tools/cluster_timeline.py.
+#   tools/build_variant.sh <name> [-DFLAG ...]   ->  build/variants/lib_<name>.so
 set -e
 cd "$(dirname "$0")/.."
 name=$1; shift

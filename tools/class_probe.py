@@ -12,20 +12,15 @@ seed0 = int(sys.argv[1]) if len(sys.argv) > 1 else 0
 plates = int(sys.argv[2]) if len(sys.argv) > 2 else 100
 items, _ = build_workload(plates, 4, 64, seed0=seed0, workers=os.cpu_count() or 1)
 ctx = Context(0)
-prios = [int(v) for v in sys.argv[3:]] or [0]      # cluster_prio settings to time one after the other
-knob = os.environ.get("PROBE_KNOB", "cluster_prio")
 packed = pack([it.setup.sample for it in items], alloc=ctx.pinned_empty)
-for pr in prios:
-    ctx.set_option(knob, pr)           # (cluster_min decides the classes when the batch is created)
-    with ctx.create_batch(packed) as b:
-        b.assemble()
-        ms = []
-        for _ in range(4):
-            b.solve(1e-10, 20000)
-            ms.append(round(b.stats()["cluster_ms"], 2))
-        print("%s %d: cluster_ms %s" % (knob, pr, ms), flush=True)
-        r = b.download()
-        rounds = b.refine_rounds()
+with ctx.create_batch(packed) as b:
+    b.assemble()
+    ms = []
+    for _ in range(4):
+        b.solve(1e-10, 20000)
+        ms.append(round(b.stats()["cluster_ms"], 2))
+    r = b.download()
+    rounds = b.refine_rounds()
 nv = np.diff(packed.vtx_off)
 rows = (nv + 127) // 128 * 128
 cl = np.maximum(1, (rows + 2047) // 2048)
