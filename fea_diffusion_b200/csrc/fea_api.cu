@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 
 #include "fea_internal.cuh"
@@ -12,13 +13,6 @@
 using namespace fea;
 
 namespace {
-
-#define CK(ctx, call)                                                        \
-  do {                                                                       \
-    cudaError_t e_ = (call);                                                 \
-    if (e_ != cudaSuccess)                                                   \
-      return api_fail(ctx, e_ == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, #call, e_); \
-  } while (0)
 
 __global__ void k_gather_i32(const int32_t* __restrict__ src, const int64_t* __restrict__ idx, int n,
                              int32_t* __restrict__ dst) {
@@ -108,43 +102,40 @@ int api_batch_begin(fea_ctx* ctx, int32_t ns, int32_t npc, const int64_t* vtx_of
   return FEA_OK;
 }
 
-cudaError_t api_batch_finish(Batch& b, const int8_t* creg_local, const int32_t* conn_local) {
+int api_batch_finish(fea_ctx* ctx, Batch& b, const int8_t* creg_local, const int32_t* conn_local) {
   cudaStream_t st = b.ctx->stream;
   const int ns = b.ns;
-  cudaError_t e = cudaSuccess;
-#define A(call) if (e == cudaSuccess) e = (call)
-  A(dalloc(b, &b.conn, b.NC * b.npc));
-  A(dalloc(b, &b.cell_dreg, b.NC));
-  A(dalloc(b, &b.d_vtx_off, ns + 1));
-  A(dalloc(b, &b.d_cell_off, ns + 1));
-  A(dalloc(b, &b.d_reg_off, ns + 1));
-  A(dalloc(b, &b.vsample, b.NV));
-  A(dalloc(b, &b.flips, ns));
-  A(dalloc(b, &b.vrank, b.NV));
-  A(dalloc(b, &b.prank, b.NV));
-  A(dalloc(b, &b.n_active, ns));
-  A(dalloc(b, &b.row_base, ns + 1));
-  A(dalloc(b, &b.row_of_vertex, b.NV));
-  A(dalloc(b, &b.vertex_of_row, b.NBR));
-  A(dalloc(b, &b.sys_of_cta, b.NBR / kCtaRows));
-  A(dalloc(b, &b.cta_first, ns));
-  A(dalloc(b, &b.cta_count, ns));
-  A(dalloc(b, &b.err_flag, 4));
-  A(dalloc(b, &b.empty, ns));
-  A(dalloc(b, &b.cl_order, ns));
-  A(dalloc(b, &b.cl_counter, 24));  // queue heads of the cluster classes, restart count, scratch
-  A(cudaMemcpyAsync(b.d_vtx_off, b.vtx_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(b.d_cell_off, b.cell_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(b.d_reg_off, b.reg_off.data(), sizeof(int32_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemsetAsync(b.flips, 0, sizeof(int32_t) * ns, st));
-  A(cudaMemsetAsync(b.err_flag, 0, sizeof(int32_t) * 4, st));
-  A(cudaMemsetAsync(b.empty, 0, sizeof(int32_t) * ns, st));
-  A(cudaMemsetAsync(b.vertex_of_row, 0xFF, sizeof(int32_t) * std::max<int64_t>(1, b.NBR), st));
-  A(launch_setup(b, creg_local, conn_local));
-  A(launch_cluster_order(b));
-#undef A
+  CK(ctx, dalloc(b, &b.conn, b.NC * b.npc));
+  CK(ctx, dalloc(b, &b.cell_dreg, b.NC));
+  CK(ctx, dalloc(b, &b.d_vtx_off, ns + 1));
+  CK(ctx, dalloc(b, &b.d_cell_off, ns + 1));
+  CK(ctx, dalloc(b, &b.d_reg_off, ns + 1));
+  CK(ctx, dalloc(b, &b.vsample, b.NV));
+  CK(ctx, dalloc(b, &b.flips, ns));
+  CK(ctx, dalloc(b, &b.vrank, b.NV));
+  CK(ctx, dalloc(b, &b.prank, b.NV));
+  CK(ctx, dalloc(b, &b.n_active, ns));
+  CK(ctx, dalloc(b, &b.row_base, ns + 1));
+  CK(ctx, dalloc(b, &b.row_of_vertex, b.NV));
+  CK(ctx, dalloc(b, &b.vertex_of_row, b.NBR));
+  CK(ctx, dalloc(b, &b.sys_of_cta, b.NBR / kCtaRows));
+  CK(ctx, dalloc(b, &b.cta_first, ns));
+  CK(ctx, dalloc(b, &b.cta_count, ns));
+  CK(ctx, dalloc(b, &b.err_flag, 4));
+  CK(ctx, dalloc(b, &b.empty, ns));
+  CK(ctx, dalloc(b, &b.cl_order, ns));
+  CK(ctx, dalloc(b, &b.cl_counter, 24));  // queue heads of the cluster classes, restart count, scratch
+  CK(ctx, cudaMemcpyAsync(b.d_vtx_off, b.vtx_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(b.d_cell_off, b.cell_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(b.d_reg_off, b.reg_off.data(), sizeof(int32_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemsetAsync(b.flips, 0, sizeof(int32_t) * ns, st));
+  CK(ctx, cudaMemsetAsync(b.err_flag, 0, sizeof(int32_t) * 4, st));
+  CK(ctx, cudaMemsetAsync(b.empty, 0, sizeof(int32_t) * ns, st));
+  CK(ctx, cudaMemsetAsync(b.vertex_of_row, 0xFF, sizeof(int32_t) * std::max<int64_t>(1, b.NBR), st));
+  CK(ctx, launch_setup(b, creg_local, conn_local));
+  CK(ctx, launch_cluster_order(b));
   b.ctx->launches += 7;
-  return e;
+  return FEA_OK;
 }
 
 int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke) {
@@ -390,42 +381,35 @@ int fea_batch_create(fea_ctx* ctx, const fea_batch_desc* d, fea_batch** out) {
   *out = nullptr;
   if (!d->vtx_off || !d->cell_off || !d->reg_off || !d->xy || !d->conn || !d->cell_region || !d->D || !d->fixed || !d->rhs)
     return api_fail(ctx, FEA_BAD_ARG, "null array in fea_batch_desc");
-  fea_batch* hb = nullptr;
-  int rc = api_batch_begin(ctx, d->n_samples, d->nodes_per_cell, d->vtx_off, d->cell_off, d->reg_off, &hb);
+  fea_batch* created = nullptr;
+  int rc = api_batch_begin(ctx, d->n_samples, d->nodes_per_cell, d->vtx_off, d->cell_off, d->reg_off, &created);
   if (rc != FEA_OK) return rc;
+  std::unique_ptr<fea_batch, decltype(&api_free_batch)> hb(created, api_free_batch);
   Batch& b = hb->b;
   cudaStream_t st = ctx->c.stream;
+  Scratch scratch(st);
   int32_t* conn_local = nullptr;
   int8_t* creg_local = nullptr;
-  cudaError_t e = cudaSuccess;
-#define A(call) if (e == cudaSuccess) e = (call)
-  A(dalloc(b, &b.xy, b.NV * 2));
-  A(dalloc(b, &b.D, (int64_t)b.NREG * 9));
-  A(dalloc(b, &b.fixed, b.NV));
-  A(dalloc(b, &b.rhs, b.NV * 2));
-  A(cudaMallocAsync((void**)&conn_local, sizeof(int32_t) * std::max<int64_t>(1, b.NC * b.npc), st));
-  A(cudaMallocAsync((void**)&creg_local, std::max<int64_t>(1, b.NC), st));
-  A(cudaMemcpyAsync(b.xy, d->xy, sizeof(double) * b.NV * 2, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(conn_local, d->conn, sizeof(int32_t) * b.NC * b.npc, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(creg_local, d->cell_region, b.NC, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(b.D, d->D, sizeof(double) * 9 * b.NREG, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(b.fixed, d->fixed, b.NV, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(b.rhs, d->rhs, sizeof(double) * b.NV * 2, cudaMemcpyHostToDevice, st));
-  A(api_batch_finish(b, creg_local, conn_local));
-  if (e == cudaSuccess && b.ns == 1 && b.npc == 3) {   // a possible uniform refinement (fea_batch_set_refinement)
+  CK(ctx, dalloc(b, &b.xy, b.NV * 2));
+  CK(ctx, dalloc(b, &b.D, (int64_t)b.NREG * 9));
+  CK(ctx, dalloc(b, &b.fixed, b.NV));
+  CK(ctx, dalloc(b, &b.rhs, b.NV * 2));
+  if (b.ns == 1 && b.npc == 3) {   // a possible uniform refinement: fea_batch_set_refinement reads it until assemble
+    CK(ctx, dalloc(b, &conn_local, b.NC * b.npc));
     b.conn_given = conn_local;
-    b.allocs.push_back(conn_local);
-  } else if (conn_local) {
-    cudaFreeAsync(conn_local, st);
+  } else {
+    CK(ctx, scratch.alloc(&conn_local, b.NC * b.npc));
   }
-  if (creg_local) cudaFreeAsync(creg_local, st);
-#undef A
-  if (e != cudaSuccess) {
-    rc = api_fail(ctx, e == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, "fea_batch_create", e);
-    api_free_batch(hb);
-    return rc;
-  }
-  *out = hb;
+  CK(ctx, scratch.alloc(&creg_local, b.NC));
+  CK(ctx, cudaMemcpyAsync(b.xy, d->xy, sizeof(double) * b.NV * 2, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(conn_local, d->conn, sizeof(int32_t) * b.NC * b.npc, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(creg_local, d->cell_region, b.NC, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(b.D, d->D, sizeof(double) * 9 * b.NREG, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(b.fixed, d->fixed, b.NV, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(b.rhs, d->rhs, sizeof(double) * b.NV * 2, cudaMemcpyHostToDevice, st));
+  rc = api_batch_finish(ctx, b, creg_local, conn_local);
+  if (rc != FEA_OK) return rc;
+  *out = hb.release();
   return FEA_OK;
 }
 
@@ -530,20 +514,20 @@ int fea_batch_rasterize_flags(fea_batch* hb, const int64_t* field_off, const uin
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
   const size_t per = (size_t)b.img_size * b.img_size, tab = sizeof(int64_t) * (b.ns + 1);
-  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
-  const size_t o_fo = 0, o_go = up(tab), o_fl = o_go + up(tab), o_im = o_fl + up((size_t)n_flags), total = o_im + up(n_img * per);
-  char* d = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&d, total, st));
-  cudaError_t e = cudaMemcpyAsync(d + o_fo, field_off, tab, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_go, flag_off.data(), tab, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d + o_fl, flags, (size_t)n_flags, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = launch_raster_flags(b, n_img, (const int64_t*)(d + o_fo), (const int64_t*)(d + o_go),
-                                                (const uint8_t*)(d + o_fl), (uint8_t*)(d + o_im));
-  if (e == cudaSuccess) e = cudaMemcpyAsync(images, d + o_im, n_img * per, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // flag_off (host vector) must outlive the copy
-  cudaFreeAsync(d, st);
+  Scratch scratch(st);
+  int64_t *d_field_off = nullptr, *d_flag_off = nullptr;
+  uint8_t *d_flags = nullptr, *d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_field_off, b.ns + 1));
+  CK(ctx, scratch.alloc(&d_flag_off, b.ns + 1));
+  CK(ctx, scratch.alloc(&d_flags, n_flags));
+  CK(ctx, scratch.alloc(&d_images, n_img * (int64_t)per));
+  CK(ctx, cudaMemcpyAsync(d_field_off, field_off, tab, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_flag_off, flag_off.data(), tab, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_flags, flags, (size_t)n_flags, cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_raster_flags(b, n_img, d_field_off, d_flag_off, d_flags, d_images));
   ctx->c.launches += 1;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_rasterize_flags", e);
+  CK(ctx, cudaMemcpyAsync(images, d_images, n_img * per, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));   // flag_off (host vector) must outlive the copy
   return FEA_OK;
 }
 
@@ -554,16 +538,15 @@ int fea_batch_cell_strain_stress(fea_batch* hb, int32_t stress_region, double* s
   if (!b.solved) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_cell_strain_stress before fea_batch_solve");
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  double* d = nullptr;
-  const size_t n = (size_t)std::max<int64_t>(1, b.NC * 3);
-  CK(ctx, cudaMallocAsync((void**)&d, sizeof(double) * 2 * n, st));
-  cudaError_t e = launch_cell_strain_stress(b, stress_region, d, d + n);
-  if (e == cudaSuccess && strain) e = cudaMemcpyAsync(strain, d, sizeof(double) * 3 * b.NC, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess && stress) e = cudaMemcpyAsync(stress, d + n, sizeof(double) * 3 * b.NC, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFreeAsync(d, st);
+  Scratch scratch(st);
+  double *d_strain = nullptr, *d_stress = nullptr;
+  CK(ctx, scratch.alloc(&d_strain, b.NC * 3));
+  CK(ctx, scratch.alloc(&d_stress, b.NC * 3));
+  CK(ctx, launch_cell_strain_stress(b, stress_region, d_strain, d_stress));
   ctx->c.launches += 1;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_cell_strain_stress", e);
+  if (strain) CK(ctx, cudaMemcpyAsync(strain, d_strain, sizeof(double) * 3 * b.NC, cudaMemcpyDeviceToHost, st));
+  if (stress) CK(ctx, cudaMemcpyAsync(stress, d_stress, sizeof(double) * 3 * b.NC, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 
@@ -577,25 +560,26 @@ int fea_batch_rasterize_cell_components(fea_batch* hb, int32_t stress_region, in
     if (field_ids[f] < 0 || field_ids[f] > 3) return api_fail(ctx, FEA_BAD_ARG, "field id must be 0..3");
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  const size_t per = (size_t)b.img_size * b.img_size, nc3 = (size_t)std::max<int64_t>(1, b.NC * 3);
-  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
-  const size_t o_stress = up(sizeof(double) * nc3), o_ids = o_stress + up(sizeof(double) * nc3), o_rng = o_ids + 256,
-               o_img = o_rng + up(sizeof(double) * 2 * n_fields * b.ns), total = o_img + up((size_t)n_fields * b.ns * per);
-  char* d = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&d, total, st));
+  const size_t per = (size_t)b.img_size * b.img_size;
+  const int64_t n_img = (int64_t)n_fields * b.ns;
+  Scratch scratch(st);
+  double *d_strain = nullptr, *d_stress = nullptr, *d_ranges = nullptr;
+  int32_t* d_ids = nullptr;
+  uint8_t* d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_strain, b.NC * 3));
+  CK(ctx, scratch.alloc(&d_stress, b.NC * 3));
+  CK(ctx, scratch.alloc(&d_ids, 4));
+  CK(ctx, scratch.alloc(&d_ranges, 2 * n_img));
+  CK(ctx, scratch.alloc(&d_images, n_img * (int64_t)per));
   int32_t ids[4] = {0, 0, 0, 0};
   for (int f = 0; f < n_fields; ++f) ids[f] = field_ids[f];
-  cudaError_t e = cudaMemcpyAsync(d + o_ids, ids, sizeof(ids), cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = launch_cell_strain_stress(b, stress_region, (double*)d, (double*)(d + o_stress));
-  if (e == cudaSuccess)
-    e = launch_raster_cell_fields(b, n_fields, (const int32_t*)(d + o_ids), (const double*)d, (const double*)(d + o_stress),
-                                  value_scale, (double*)(d + o_rng), (uint8_t*)(d + o_img));
-  if (e == cudaSuccess && images) e = cudaMemcpyAsync(images, d + o_img, (size_t)n_fields * b.ns * per, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess && ranges) e = cudaMemcpyAsync(ranges, d + o_rng, sizeof(double) * 2 * n_fields * b.ns, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // ids (host array) must outlive the copy
-  cudaFreeAsync(d, st);
+  CK(ctx, cudaMemcpyAsync(d_ids, ids, sizeof(ids), cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_cell_strain_stress(b, stress_region, d_strain, d_stress));
+  CK(ctx, launch_raster_cell_fields(b, n_fields, d_ids, d_strain, d_stress, value_scale, d_ranges, d_images));
   ctx->c.launches += 3;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_rasterize_cell_components", e);
+  if (images) CK(ctx, cudaMemcpyAsync(images, d_images, (size_t)n_img * per, cudaMemcpyDeviceToHost, st));
+  if (ranges) CK(ctx, cudaMemcpyAsync(ranges, d_ranges, sizeof(double) * 2 * n_img, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));   // ids (host array) must outlive the copy
   return FEA_OK;
 }
 
@@ -618,13 +602,14 @@ int fea_batch_sample_sizes(fea_batch* hb, int64_t* n_active_dofs, int64_t* nnz) 
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
   std::vector<int32_t> na(b.ns), ap(b.ns + 1);
-  int32_t* d_tmp = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&d_tmp, sizeof(int32_t) * (b.ns + 1), st));
-  k_gather_i32<<<(b.ns + 1 + 255) / 256, 256, 0, st>>>(b.adj_ptr, b.d_vtx_off, b.ns + 1, d_tmp);
-  CK(ctx, cudaMemcpyAsync(ap.data(), d_tmp, sizeof(int32_t) * (b.ns + 1), cudaMemcpyDeviceToHost, st));
+  Scratch scratch(st);
+  int32_t* d_ap = nullptr;
+  CK(ctx, scratch.alloc(&d_ap, b.ns + 1));
+  k_gather_i32<<<(b.ns + 1 + 255) / 256, 256, 0, st>>>(b.adj_ptr, b.d_vtx_off, b.ns + 1, d_ap);
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaMemcpyAsync(ap.data(), d_ap, sizeof(int32_t) * (b.ns + 1), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaMemcpyAsync(na.data(), b.n_active, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
-  cudaFreeAsync(d_tmp, st);
   for (int s = 0; s < b.ns; ++s) {
     if (n_active_dofs) n_active_dofs[s] = 2 * (int64_t)na[s];
     if (nnz) nnz[s] = 4 * (int64_t)(ap[s + 1] - ap[s]);
@@ -638,11 +623,13 @@ int fea_batch_get_info(fea_batch* hb, fea_batch_info* out) {
   Batch& b = hb->b;
   if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_info before fea_batch_assemble");
   CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
   std::vector<int32_t> na(b.ns), fl(b.ns);
   int64_t rows = 0;
-  CK(ctx, cudaMemcpy(na.data(), b.n_active, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost));
-  CK(ctx, cudaMemcpy(fl.data(), b.flips, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost));
-  CK(ctx, cudaMemcpy(&rows, b.row_base + b.ns, sizeof(int64_t), cudaMemcpyDeviceToHost));
+  CK(ctx, cudaMemcpyAsync(na.data(), b.n_active, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(fl.data(), b.flips, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(&rows, b.row_base + b.ns, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   out->n_vertices = b.NV;
   out->n_cells = b.NC;
   out->n_active_dofs = 0;
@@ -694,12 +681,13 @@ int fea_batch_get_conn(fea_batch* hb, int32_t* conn, int32_t* n_flipped) {
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
   if (conn && b.NC) {
-    int32_t* tmp = nullptr;
-    CK(ctx, cudaMallocAsync((void**)&tmp, sizeof(int32_t) * b.NC * b.npc, st));
-    k_localize_conn<<<(unsigned)((b.NC + 255) / 256), 256, 0, st>>>(b.NC, b.npc, b.d_cell_off, b.d_vtx_off, b.ns, b.conn, tmp);
-    CK(ctx, cudaMemcpyAsync(conn, tmp, sizeof(int32_t) * b.NC * b.npc, cudaMemcpyDeviceToHost, st));
+    Scratch scratch(st);
+    int32_t* d_conn = nullptr;
+    CK(ctx, scratch.alloc(&d_conn, b.NC * b.npc));
+    k_localize_conn<<<(unsigned)((b.NC + 255) / 256), 256, 0, st>>>(b.NC, b.npc, b.d_cell_off, b.d_vtx_off, b.ns, b.conn, d_conn);
+    CK(ctx, cudaGetLastError());
+    CK(ctx, cudaMemcpyAsync(conn, d_conn, sizeof(int32_t) * b.NC * b.npc, cudaMemcpyDeviceToHost, st));
     CK(ctx, cudaStreamSynchronize(st));
-    cudaFreeAsync(tmp, st);
   }
   if (n_flipped) {
     CK(ctx, cudaMemcpyAsync(n_flipped, b.flips, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
@@ -734,22 +722,20 @@ int fea_batch_get_csr(fea_batch* hb, int32_t s, int32_t* indptr, int32_t* indice
   CK(ctx, cudaMemcpyAsync(&a1, b.adj_ptr + b.vtx_off[s + 1], sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
   const int64_t n = 2 * (int64_t)na, nnz = 4 * (int64_t)(a1 - a0);
+  Scratch scratch(st);
   int32_t *d_ip = nullptr, *d_ix = nullptr;
   double* d_dt = nullptr;
   if (indptr) {
-    CK(ctx, cudaMallocAsync((void**)&d_ip, sizeof(int32_t) * (n + 1), st));
+    CK(ctx, scratch.alloc(&d_ip, n + 1));
     CK(ctx, cudaMemsetAsync(d_ip, 0, sizeof(int32_t) * (n + 1), st));
   }
-  if (indices) CK(ctx, cudaMallocAsync((void**)&d_ix, sizeof(int32_t) * std::max<int64_t>(1, nnz), st));
-  if (data) CK(ctx, cudaMallocAsync((void**)&d_dt, sizeof(double) * std::max<int64_t>(1, nnz), st));
+  if (indices) CK(ctx, scratch.alloc(&d_ix, nnz));
+  if (data) CK(ctx, scratch.alloc(&d_dt, nnz));
   CK(ctx, launch_csr_export(b, s, d_ip, d_ix, d_dt));
   if (indptr) CK(ctx, cudaMemcpyAsync(indptr, d_ip, sizeof(int32_t) * (n + 1), cudaMemcpyDeviceToHost, st));
   if (indices) CK(ctx, cudaMemcpyAsync(indices, d_ix, sizeof(int32_t) * nnz, cudaMemcpyDeviceToHost, st));
   if (data) CK(ctx, cudaMemcpyAsync(data, d_dt, sizeof(double) * nnz, cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
-  if (d_ip) cudaFreeAsync(d_ip, st);
-  if (d_ix) cudaFreeAsync(d_ix, st);
-  if (d_dt) cudaFreeAsync(d_dt, st);
   return FEA_OK;
 }
 
@@ -765,15 +751,14 @@ int fea_batch_spmv(fea_batch* hb, int32_t s, const double* x, double* y) {
   CK(ctx, cudaMemcpyAsync(&na, b.n_active + s, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
   const int64_t n = 2 * (int64_t)na;
+  Scratch scratch(st);
   double *dx = nullptr, *dy = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&dx, sizeof(double) * std::max<int64_t>(1, n), st));
-  CK(ctx, cudaMallocAsync((void**)&dy, sizeof(double) * std::max<int64_t>(1, n), st));
+  CK(ctx, scratch.alloc(&dx, n));
+  CK(ctx, scratch.alloc(&dy, n));
   CK(ctx, cudaMemcpyAsync(dx, x, sizeof(double) * n, cudaMemcpyHostToDevice, st));
   CK(ctx, launch_plain_spmv(b, s, dx, dy));
   CK(ctx, cudaMemcpyAsync(y, dy, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
-  cudaFreeAsync(dx, st);
-  cudaFreeAsync(dy, st);
   b.solved = false;  // solver vectors were overwritten
   return FEA_OK;
 }
@@ -790,32 +775,33 @@ int fea_rasterize_fields(fea_ctx* ctx, const double* xy, int64_t n_v, const int3
     if (conn[i] < 0 || conn[i] >= n_v) return api_fail(ctx, FEA_MESH_ERROR, "connectivity index out of range");
   CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  const int64_t per = (int64_t)size * size;
-  const size_t b_xy = sizeof(double) * 2 * n_v, b_cn = sizeof(int32_t) * n_cell * nodes_per_cell,
-               b_f = sizeof(double) * n_fields * (cell_fields ? std::max<int64_t>(n_cell, 1) : n_v), b_img = (size_t)n_fields * per;
-  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
-  const size_t o_xy = 0, o_cn = o_xy + up(b_xy), o_f = o_cn + up(b_cn), o_cl = o_f + up(b_f),
-               o_af = o_cl + up(sizeof(double) * 2 * n_fields), o_co = o_af + 256, o_ow = o_co + 256,
-               o_im = o_ow + up(sizeof(int32_t) * per), total = o_im + up(b_img);
-  char* d = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&d, total, st));
+  const int64_t per = (int64_t)size * size, n_conn = n_cell * nodes_per_cell,
+                n_f = (int64_t)n_fields * (cell_fields ? std::max<int64_t>(n_cell, 1) : n_v);
+  Scratch scratch(st);
+  double *d_xy = nullptr, *d_f = nullptr, *d_clim = nullptr, *d_affine = nullptr;
+  int32_t *d_conn = nullptr, *d_owner = nullptr;
+  int64_t* d_cell_off = nullptr;
+  uint8_t* d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_xy, 2 * n_v));
+  CK(ctx, scratch.alloc(&d_conn, n_conn));
+  CK(ctx, scratch.alloc(&d_f, n_f));
+  CK(ctx, scratch.alloc(&d_clim, 2 * n_fields));
+  CK(ctx, scratch.alloc(&d_affine, 4));
+  CK(ctx, scratch.alloc(&d_cell_off, 2));
+  CK(ctx, scratch.alloc(&d_owner, per));
+  CK(ctx, scratch.alloc(&d_images, n_fields * per));
   const int64_t h_off[2] = {0, n_cell};
-  cudaError_t e = cudaMemcpyAsync(d + o_xy, xy, b_xy, cudaMemcpyHostToDevice, st);
-#define A(call) if (e == cudaSuccess) e = (call)
-  if (b_cn) A(cudaMemcpyAsync(d + o_cn, conn, b_cn, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d + o_f, fields, b_f, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d + o_cl, clim, sizeof(double) * 2 * n_fields, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d + o_af, affine, sizeof(double) * 4, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d + o_co, h_off, sizeof(h_off), cudaMemcpyHostToDevice, st));
-  A(launch_raster_fields(st, nodes_per_cell, n_v, n_cell, (const int32_t*)(d + o_cn), (const double*)(d + o_xy),
-                         (const double*)(d + o_af), (const int64_t*)(d + o_co), size, (int32_t*)(d + o_ow),
-                         (const double*)(d + o_f), n_fields, cell_fields ? 1 : 0, (const double*)(d + o_cl), (uint8_t*)(d + o_im)));
-  A(cudaMemcpyAsync(images, d + o_im, b_img, cudaMemcpyDeviceToHost, st));
-  A(cudaStreamSynchronize(st));
-#undef A
-  cudaFreeAsync(d, st);
+  CK(ctx, cudaMemcpyAsync(d_xy, xy, sizeof(double) * 2 * n_v, cudaMemcpyHostToDevice, st));
+  if (n_conn) CK(ctx, cudaMemcpyAsync(d_conn, conn, sizeof(int32_t) * n_conn, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_f, fields, sizeof(double) * n_f, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_clim, clim, sizeof(double) * 2 * n_fields, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_affine, affine, sizeof(double) * 4, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_cell_off, h_off, sizeof(h_off), cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_raster_fields(st, nodes_per_cell, n_v, n_cell, d_conn, d_xy, d_affine, d_cell_off, size, d_owner, d_f,
+                               n_fields, cell_fields ? 1 : 0, d_clim, d_images));
   ctx->c.launches += 3;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_rasterize_fields", e);
+  CK(ctx, cudaMemcpyAsync(images, d_images, (size_t)n_fields * per, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 
@@ -895,15 +881,15 @@ int fea_batch_mg_apply(fea_batch* hb, const double* r, double* z) {
   CK(ctx, cudaMemcpyAsync(&na, b.n_active, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
   const int64_t n = 2 * (int64_t)na;
-  double* d = nullptr;
-  CK(ctx, cudaMallocAsync((void**)&d, sizeof(double) * 2 * std::max<int64_t>(1, n), st));
-  cudaError_t e = cudaMemcpyAsync(d, r, sizeof(double) * n, cudaMemcpyHostToDevice, st);
-  int rc = e == cudaSuccess ? mg_apply(ctx, b, d, d + std::max<int64_t>(1, n)) : FEA_CUDA_ERROR;
-  if (rc == FEA_OK) e = cudaMemcpyAsync(z, d + std::max<int64_t>(1, n), sizeof(double) * n, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFreeAsync(d, st);
+  Scratch scratch(st);
+  double *d_r = nullptr, *d_z = nullptr;
+  CK(ctx, scratch.alloc(&d_r, n));
+  CK(ctx, scratch.alloc(&d_z, n));
+  CK(ctx, cudaMemcpyAsync(d_r, r, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  const int rc = mg_apply(ctx, b, d_r, d_z);
   if (rc != FEA_OK) return rc;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_mg_apply", e);
+  CK(ctx, cudaMemcpyAsync(z, d_z, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 

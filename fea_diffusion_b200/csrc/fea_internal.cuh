@@ -212,6 +212,13 @@ namespace fea {
 
 // error bookkeeping shared by the API translation units (fea_api.cu)
 int api_fail(fea_ctx* ctx, int code, const char* what, cudaError_t e = cudaSuccess);
+// return FEA_OUT_OF_MEMORY / FEA_CUDA_ERROR from the calling function when a CUDA call fails
+#define CK(ctx, call)                                                        \
+  do {                                                                       \
+    cudaError_t e_ = (call);                                                 \
+    if (e_ != cudaSuccess)                                                   \
+      return ::fea::api_fail(ctx, e_ == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, #call, e_); \
+  } while (0)
 void api_free_batch(fea_batch* hb);
 // host-side part of batch creation that does not depend on how the set-up arrays were produced:
 // sizes, offset tables, cluster classes.  Returns FEA_OK or a status (message set on ctx).
@@ -219,8 +226,8 @@ int api_batch_begin(fea_ctx* ctx, int32_t ns, int32_t npc, const int64_t* vtx_of
                     const int32_t* reg_off, fea_batch** out);
 // allocations of the arrays launch_setup fills, offset-table uploads, launch_setup itself and the
 // device-side ordering of the cluster queues; b.xy, b.D, b.fixed, b.rhs must be allocated and
-// (stream-ordered) filled, conn_local / creg_local are consumed.
-cudaError_t api_batch_finish(Batch& b, const int8_t* d_creg_local, const int32_t* d_conn_local);
+// (stream-ordered) filled, conn_local / creg_local are consumed.  Returns FEA_OK or a status (message set on ctx).
+int api_batch_finish(fea_ctx* ctx, Batch& b, const int8_t* d_creg_local, const int32_t* d_conn_local);
 // element stiffness (fill_ke: launch_element_stiffness, or the Galerkin product of a multigrid level),
 // topology, block-SELL matrix and solver vectors of a created batch
 int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke);
@@ -240,6 +247,30 @@ inline cudaError_t dalloc(Batch& b, T** p, int64_t n) {
   if (e == cudaSuccess) b.allocs.push_back(*p);
   return e;
 }
+
+// Temporary device memory of one scope: alloc() follows dalloc's rule (n <= 0 allocates one element), and
+// the destructor frees every allocation stream-ordered on `st`, on the error returns as well.
+class Scratch {
+ public:
+  explicit Scratch(cudaStream_t st) : st_(st) {}
+  Scratch(const Scratch&) = delete;
+  Scratch& operator=(const Scratch&) = delete;
+  ~Scratch() {
+    for (void* p : ptrs_) cudaFreeAsync(p, st_);
+  }
+  template <class T>
+  cudaError_t alloc(T** p, int64_t n) {
+    *p = nullptr;
+    if (n <= 0) n = 1;
+    cudaError_t e = cudaMallocAsync((void**)p, sizeof(T) * (size_t)n, st_);
+    if (e == cudaSuccess) ptrs_.push_back(*p);
+    return e;
+  }
+
+ private:
+  cudaStream_t st_;
+  std::vector<void*> ptrs_;
+};
 
 // ---- launchers implemented in the kernel translation units -----------------
 // All return cudaError_t of the launch (cudaGetLastError).

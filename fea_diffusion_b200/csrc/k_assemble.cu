@@ -35,12 +35,11 @@ cudaError_t launch_sell_lengths(Batch& b) {
   const int T = 256;
   if (b.n_slices == 0) return cudaSuccess;
   k_slice_len<<<(unsigned)((b.NBR + T - 1) / T), T, 0, st>>>(b.n_slices, b.vertex_of_row, b.adj_ptr, b.slice_len);
+  Scratch scratch(st);
   int64_t* tmp = nullptr;
-  cudaError_t e = cudaMallocAsync(&tmp, sizeof(int64_t) * (b.n_slices / 4096 + 4), st);
+  cudaError_t e = scratch.alloc(&tmp, b.n_slices / 4096 + 4);
   if (e != cudaSuccess) return e;
-  exclusive_scan_i32_to_i64(b.slice_len, b.slice_ptr, b.n_slices, 32, tmp, st);
-  cudaFreeAsync(tmp, st);
-  return cudaGetLastError();
+  return exclusive_scan_i32_to_i64(b.slice_len, b.slice_ptr, b.n_slices, 32, tmp, st);
 }
 
 // 2x2 block K[v][w] summed over the stiffness cells containing both, ascending cell order.

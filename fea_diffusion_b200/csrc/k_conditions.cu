@@ -19,6 +19,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <vector>
 
@@ -576,13 +577,14 @@ cudaError_t launch_classify(Batch& b, int32_t* d_floating, int32_t* d_empty) {
       return cudaGetLastError();
     }
   }
-  cudaMemsetAsync(d_floating, 0, sizeof(int32_t) * b.ns, st);
-  cudaMemsetAsync(d_empty, 0, sizeof(int32_t) * b.ns, st);
+  Scratch scratch(st);
   int32_t *parent = nullptr, *nfix = nullptr;
   cudaError_t e;
-  if ((e = cudaMallocAsync((void**)&parent, sizeof(int32_t) * std::max<int64_t>(1, b.NC), st)) != cudaSuccess) return e;
-  if ((e = cudaMallocAsync((void**)&nfix, sizeof(int32_t) * std::max<int64_t>(1, b.NC), st)) != cudaSuccess) return e;
-  cudaMemsetAsync(nfix, 0, sizeof(int32_t) * std::max<int64_t>(1, b.NC), st);
+  if ((e = cudaMemsetAsync(d_floating, 0, sizeof(int32_t) * b.ns, st)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(d_empty, 0, sizeof(int32_t) * b.ns, st)) != cudaSuccess) return e;
+  if ((e = scratch.alloc(&parent, b.NC)) != cudaSuccess) return e;
+  if ((e = scratch.alloc(&nfix, b.NC)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(nfix, 0, sizeof(int32_t) * std::max<int64_t>(1, b.NC), st)) != cudaSuccess) return e;
   if (b.NC) {
     const unsigned gc = (unsigned)((b.NC + T - 1) / T), ge = (unsigned)((b.NC * b.npc + T - 1) / T);
     k_cc_init<<<gc, T, 0, st>>>(b.NC, b.cell_dreg, parent);
@@ -592,8 +594,6 @@ cudaError_t launch_classify(Batch& b, int32_t* d_floating, int32_t* d_empty) {
   }
   if (b.NV) k_cc_vertices<<<(unsigned)((b.NV + T - 1) / T), T, 0, st>>>(b.NV, b.fixed, b.vsample, b.inc_ptr, b.inc, parent, nfix, d_empty);
   if (b.NC) k_cc_count<<<(unsigned)((b.NC + T - 1) / T), T, 0, st>>>(b.NC, b.npc, b.conn, b.vsample, parent, nfix, d_floating);
-  cudaFreeAsync(parent, st);
-  cudaFreeAsync(nfix, st);
   b.ctx->launches += 5;
   return cudaGetLastError();
 }
@@ -606,13 +606,6 @@ cudaError_t launch_classify(Batch& b, int32_t* d_floating, int32_t* d_empty) {
 using namespace fea;
 
 namespace {
-
-#define CKC(ctx, call)                                                       \
-  do {                                                                       \
-    cudaError_t e_ = (call);                                                 \
-    if (e_ != cudaSuccess)                                                   \
-      return api_fail(ctx, e_ == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, #call, e_); \
-  } while (0)
 
 // tag (1-based point tag) -> sample-local vertex index with numpy's negative wrap-around
 // ('vertex {tag-1}', coors[tag - 1]; fea_analysis.py:184-185, 198)
@@ -744,9 +737,10 @@ int fea_batch_create_from_conditions(fea_ctx* ctx, const fea_conditions_desc* d,
   const int64_t n_scalars = 2 * d->mat_coord_off[n_matreg];
   const int64_t MV = d->mesh_vtx_off[nm], MC = d->mesh_cell_off[nm];
 
-  fea_batch* hb = nullptr;
-  int rc = api_batch_begin(ctx, ns, npc, vtx_off.data(), cell_off.data(), reg_off.data(), &hb);
+  fea_batch* created = nullptr;
+  int rc = api_batch_begin(ctx, ns, npc, vtx_off.data(), cell_off.data(), reg_off.data(), &created);
   if (rc != FEA_OK) return rc;
+  std::unique_ptr<fea_batch, decltype(&api_free_batch)> hb(created, api_free_batch);
   Batch& b = hb->b;
   b.from_conditions = true;
   b.NR = NRrows;
@@ -754,13 +748,7 @@ int fea_batch_create_from_conditions(fea_ctx* ctx, const fea_conditions_desc* d,
   b.flag_off = flag_off;
   cudaStream_t st = ctx->c.stream;
   const int T = 256;
-  // scratch (freed stream-ordered at the end)
-  std::vector<void*> scratch;
-  auto salloc = [&](void** p, size_t bytes) {
-    cudaError_t e = cudaMallocAsync(p, bytes ? bytes : 1, st);
-    if (e == cudaSuccess) scratch.push_back(*p);
-    return e;
-  };
+  Scratch scratch(st);
   double2 *m_xy = nullptr;
   int32_t *m_conn = nullptr, *conn_local = nullptr, *d_mat_region = nullptr, *d_mat_first = nullptr, *combo_first = nullptr,
           *combo_id = nullptr, *d_regoff = nullptr;
@@ -771,102 +759,89 @@ int fea_batch_create_from_conditions(fea_ctx* ctx, const fea_conditions_desc* d,
   unsigned long long* tab = nullptr;
   uint8_t* v0 = nullptr;
   uint32_t *cell_member = nullptr, *combo_mask = nullptr;
-  cudaError_t e = cudaSuccess;
-#define A(call) if (e == cudaSuccess) e = (call)
-  A(dalloc(b, &b.xy, b.NV * 2));
-  A(dalloc(b, &b.D, (int64_t)b.NREG * 9));
-  A(dalloc(b, &b.fixed, b.NV));
-  A(dalloc(b, &b.rhs, b.NV * 2));
-  A(dalloc(b, &b.rflags, flag_bytes));
-  A(dalloc(b, &b.rcount, NRrows));
-  A(dalloc(b, &b.creg_local, b.NC));
-  A(dalloc(b, &b.n_reg_used, ns));
-  A(salloc((void**)&m_xy, sizeof(double) * 2 * MV));
-  A(salloc((void**)&m_conn, sizeof(int32_t) * MC * npc));
-  A(salloc((void**)&m_vtx_off, sizeof(int64_t) * (nm + 1)));
-  A(salloc((void**)&m_cell_off, sizeof(int64_t) * (nm + 1)));
-  A(salloc((void**)&d_voff, sizeof(int64_t) * (ns + 1)));
-  A(salloc((void**)&d_coff, sizeof(int64_t) * (ns + 1)));
-  A(salloc((void**)&conn_local, sizeof(int32_t) * b.NC * npc));
-  A(salloc((void**)&d_sc, sizeof(SampleCond) * ns));
-  A(salloc((void**)&d_reg, sizeof(Region) * NRrows));
-  A(salloc((void**)&d_mat_region, sizeof(int32_t) * std::max(n_matreg, 1)));
-  A(salloc((void**)&d_mat_first, sizeof(int32_t) * ns));
-  A(salloc((void**)&d_regoff, sizeof(int32_t) * (ns + 1)));
-  A(salloc((void**)&d_coord_off, sizeof(int64_t) * (n_matreg + 1)));
-  A(salloc((void**)&d_E_nu, sizeof(double) * 2 * std::max(n_matreg, 1)));
-  A(salloc((void**)&d_coords, sizeof(double) * std::max<int64_t>(n_scalars, 1)));
-  A(salloc((void**)&tab, sizeof(unsigned long long) * std::max<int64_t>(tab_slots, 1)));
-  A(salloc((void**)&v0, (size_t)flag_bytes));
-  A(salloc((void**)&cell_member, sizeof(uint32_t) * std::max<int64_t>(b.NC, 1)));
-  A(salloc((void**)&combo_mask, sizeof(uint32_t) * ns * kMaxCombo));
-  A(salloc((void**)&combo_first, sizeof(int32_t) * ns * kMaxCombo));
-  A(salloc((void**)&combo_id, sizeof(int32_t) * ns * kMaxCombo));
+  CK(ctx, dalloc(b, &b.xy, b.NV * 2));
+  CK(ctx, dalloc(b, &b.D, (int64_t)b.NREG * 9));
+  CK(ctx, dalloc(b, &b.fixed, b.NV));
+  CK(ctx, dalloc(b, &b.rhs, b.NV * 2));
+  CK(ctx, dalloc(b, &b.rflags, flag_bytes));
+  CK(ctx, dalloc(b, &b.rcount, NRrows));
+  CK(ctx, dalloc(b, &b.creg_local, b.NC));
+  CK(ctx, dalloc(b, &b.n_reg_used, ns));
+  CK(ctx, scratch.alloc(&m_xy, MV));
+  CK(ctx, scratch.alloc(&m_conn, MC * npc));
+  CK(ctx, scratch.alloc(&m_vtx_off, nm + 1));
+  CK(ctx, scratch.alloc(&m_cell_off, nm + 1));
+  CK(ctx, scratch.alloc(&d_voff, ns + 1));
+  CK(ctx, scratch.alloc(&d_coff, ns + 1));
+  CK(ctx, scratch.alloc(&conn_local, b.NC * npc));
+  CK(ctx, scratch.alloc(&d_sc, ns));
+  CK(ctx, scratch.alloc(&d_reg, NRrows));
+  CK(ctx, scratch.alloc(&d_mat_region, n_matreg));
+  CK(ctx, scratch.alloc(&d_mat_first, ns));
+  CK(ctx, scratch.alloc(&d_regoff, ns + 1));
+  CK(ctx, scratch.alloc(&d_coord_off, n_matreg + 1));
+  CK(ctx, scratch.alloc(&d_E_nu, 2 * std::max(n_matreg, 1)));
+  CK(ctx, scratch.alloc(&d_coords, n_scalars));
+  CK(ctx, scratch.alloc(&tab, tab_slots));
+  CK(ctx, scratch.alloc(&v0, flag_bytes));
+  CK(ctx, scratch.alloc(&cell_member, b.NC));
+  CK(ctx, scratch.alloc(&combo_mask, ns * kMaxCombo));
+  CK(ctx, scratch.alloc(&combo_first, ns * kMaxCombo));
+  CK(ctx, scratch.alloc(&combo_id, ns * kMaxCombo));
   // err_flag is allocated by api_batch_finish; the combination overflow is collected in a word of its own first
   int32_t* d_err = nullptr;
-  A(dalloc(b, &d_err, 1));
-  A(cudaMemsetAsync(d_err, 0, sizeof(int32_t), st));
-  A(cudaMemcpyAsync(m_xy, d->xy, sizeof(double) * 2 * MV, cudaMemcpyDefault, st));       // host or device (fea_device_upload)
-  A(cudaMemcpyAsync(m_conn, d->conn, sizeof(int32_t) * MC * npc, cudaMemcpyDefault, st));
-  A(cudaMemcpyAsync(m_vtx_off, d->mesh_vtx_off, sizeof(int64_t) * (nm + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(m_cell_off, d->mesh_cell_off, sizeof(int64_t) * (nm + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_voff, vtx_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_coff, cell_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_sc, sc.data(), sizeof(SampleCond) * ns, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_reg, reg.data(), sizeof(Region) * NRrows, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_mat_region, mat_region.data(), sizeof(int32_t) * std::max(n_matreg, 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_mat_first, mat_first.data(), sizeof(int32_t) * ns, cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_regoff, reg_off.data(), sizeof(int32_t) * (ns + 1), cudaMemcpyHostToDevice, st));
-  A(cudaMemcpyAsync(d_coord_off, d->mat_coord_off, sizeof(int64_t) * (n_matreg + 1), cudaMemcpyHostToDevice, st));
-  if (n_matreg) A(cudaMemcpyAsync(d_E_nu, d->mat_E_nu, sizeof(double) * 2 * n_matreg, cudaMemcpyHostToDevice, st));
-  if (n_scalars) A(cudaMemcpyAsync(d_coords, d->mat_coords, sizeof(double) * n_scalars, cudaMemcpyDefault, st));
-  A(cudaMemsetAsync(tab, 0xFF, sizeof(unsigned long long) * std::max<int64_t>(tab_slots, 1), st));
-  A(cudaMemsetAsync(cell_member, 0, sizeof(uint32_t) * std::max<int64_t>(b.NC, 1), st));
-  A(cudaMemsetAsync(combo_mask, 0, sizeof(uint32_t) * ns * kMaxCombo, st));
-  A(cudaMemsetAsync(combo_first, 0x7F, sizeof(int32_t) * ns * kMaxCombo, st));
-  A(cudaMemsetAsync(combo_id, 0, sizeof(int32_t) * ns * kMaxCombo, st));
-  A(cudaMemsetAsync(b.D, 0, sizeof(double) * 9 * std::max<int64_t>(b.NREG, 1), st));
-  if (e == cudaSuccess) {
-    int64_t nv_max = 0, nc_max = 0;
-    for (int s = 0; s < ns; ++s) {
-      nv_max = std::max(nv_max, vtx_off[s + 1] - vtx_off[s]);
-      nc_max = std::max(nc_max, cell_off[s + 1] - cell_off[s]);
-    }
-    const unsigned gyv = (unsigned)std::max<int64_t>(1, (nv_max + T - 1) / T), gyc = (unsigned)std::max<int64_t>(1, (nc_max + T - 1) / T),
-                   gyn = (unsigned)std::max<int64_t>(1, (nc_max * npc + T - 1) / T);
-    if (gyv > 65535u || gyn > 65535u) e = cudaErrorInvalidValue;   // > 16 M vertices in one sample
-    if (e == cudaSuccess) {
-      k_replicate_vertices<<<dim3(ns, gyv), T, 0, st>>>(d_sc, d_voff, m_vtx_off, m_xy, (double2*)b.xy);
-      k_replicate_cells<<<dim3(ns, gyn), T, 0, st>>>(d_sc, d_coff, npc, m_cell_off, m_conn, conn_local);
-      if (n_scalars)
-        k_hash_insert<<<(unsigned)((n_scalars + T - 1) / T), T, 0, st>>>(n_scalars, n_matreg, d_coord_off, d_mat_region, d_reg, d_coords, tab);
-      k_region_vertices<<<dim3((unsigned)NRrows, gyv), T, 0, st>>>(d_reg, d_voff, (const double2*)b.xy, tab, v0, b.rflags);
-      if (npc == 3) k_region_cells<3><<<dim3((unsigned)NRrows, gyc), T, 0, st>>>(d_reg, d_voff, d_coff, conn_local, v0, b.rflags, cell_member);
-      else k_region_cells<4><<<dim3((unsigned)NRrows, gyc), T, 0, st>>>(d_reg, d_voff, d_coff, conn_local, v0, b.rflags, cell_member);
-      k_region_count<<<(unsigned)NRrows, T, 0, st>>>(d_reg, d_voff, b.rflags, b.rcount);
-      k_fixed_rhs<<<dim3(ns, gyv), T, 0, st>>>(d_sc, d_reg, d_voff, b.rflags, b.rcount, b.fixed, (double2*)b.rhs);
-      k_cell_region<<<dim3(ns, gyc), T, 0, st>>>(d_sc, d_coff, cell_member, combo_mask, combo_first, b.creg_local, d_err);
-      k_material_table<<<(ns + 127) / 128, 128, 0, st>>>(ns, d_sc, d_regoff, d_E_nu, d_mat_first, combo_mask, combo_first,
-                                                        combo_id, b.D, b.n_reg_used);
-      k_cell_region_combos<<<dim3(ns, gyc), T, 0, st>>>(d_coff, combo_id, b.creg_local);
-      e = cudaGetLastError();
-    }
+  CK(ctx, dalloc(b, &d_err, 1));
+  CK(ctx, cudaMemsetAsync(d_err, 0, sizeof(int32_t), st));
+  CK(ctx, cudaMemcpyAsync(m_xy, d->xy, sizeof(double) * 2 * MV, cudaMemcpyDefault, st));       // host or device (fea_device_upload)
+  CK(ctx, cudaMemcpyAsync(m_conn, d->conn, sizeof(int32_t) * MC * npc, cudaMemcpyDefault, st));
+  CK(ctx, cudaMemcpyAsync(m_vtx_off, d->mesh_vtx_off, sizeof(int64_t) * (nm + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(m_cell_off, d->mesh_cell_off, sizeof(int64_t) * (nm + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_voff, vtx_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_coff, cell_off.data(), sizeof(int64_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_sc, sc.data(), sizeof(SampleCond) * ns, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_reg, reg.data(), sizeof(Region) * NRrows, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_mat_region, mat_region.data(), sizeof(int32_t) * std::max(n_matreg, 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_mat_first, mat_first.data(), sizeof(int32_t) * ns, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_regoff, reg_off.data(), sizeof(int32_t) * (ns + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_coord_off, d->mat_coord_off, sizeof(int64_t) * (n_matreg + 1), cudaMemcpyHostToDevice, st));
+  if (n_matreg) CK(ctx, cudaMemcpyAsync(d_E_nu, d->mat_E_nu, sizeof(double) * 2 * n_matreg, cudaMemcpyHostToDevice, st));
+  if (n_scalars) CK(ctx, cudaMemcpyAsync(d_coords, d->mat_coords, sizeof(double) * n_scalars, cudaMemcpyDefault, st));
+  CK(ctx, cudaMemsetAsync(tab, 0xFF, sizeof(unsigned long long) * std::max<int64_t>(tab_slots, 1), st));
+  CK(ctx, cudaMemsetAsync(cell_member, 0, sizeof(uint32_t) * std::max<int64_t>(b.NC, 1), st));
+  CK(ctx, cudaMemsetAsync(combo_mask, 0, sizeof(uint32_t) * ns * kMaxCombo, st));
+  CK(ctx, cudaMemsetAsync(combo_first, 0x7F, sizeof(int32_t) * ns * kMaxCombo, st));
+  CK(ctx, cudaMemsetAsync(combo_id, 0, sizeof(int32_t) * ns * kMaxCombo, st));
+  CK(ctx, cudaMemsetAsync(b.D, 0, sizeof(double) * 9 * std::max<int64_t>(b.NREG, 1), st));
+  int64_t nv_max = 0, nc_max = 0;
+  for (int s = 0; s < ns; ++s) {
+    nv_max = std::max(nv_max, vtx_off[s + 1] - vtx_off[s]);
+    nc_max = std::max(nc_max, cell_off[s + 1] - cell_off[s]);
   }
+  const unsigned gyv = (unsigned)std::max<int64_t>(1, (nv_max + T - 1) / T), gyc = (unsigned)std::max<int64_t>(1, (nc_max + T - 1) / T),
+                 gyn = (unsigned)std::max<int64_t>(1, (nc_max * npc + T - 1) / T);
+  if (gyv > 65535u || gyn > 65535u)
+    return api_fail(ctx, FEA_CUDA_ERROR, "more than 16 M vertices or cell corners in one sample");
+  k_replicate_vertices<<<dim3(ns, gyv), T, 0, st>>>(d_sc, d_voff, m_vtx_off, m_xy, (double2*)b.xy);
+  k_replicate_cells<<<dim3(ns, gyn), T, 0, st>>>(d_sc, d_coff, npc, m_cell_off, m_conn, conn_local);
+  if (n_scalars)
+    k_hash_insert<<<(unsigned)((n_scalars + T - 1) / T), T, 0, st>>>(n_scalars, n_matreg, d_coord_off, d_mat_region, d_reg, d_coords, tab);
+  k_region_vertices<<<dim3((unsigned)NRrows, gyv), T, 0, st>>>(d_reg, d_voff, (const double2*)b.xy, tab, v0, b.rflags);
+  if (npc == 3) k_region_cells<3><<<dim3((unsigned)NRrows, gyc), T, 0, st>>>(d_reg, d_voff, d_coff, conn_local, v0, b.rflags, cell_member);
+  else k_region_cells<4><<<dim3((unsigned)NRrows, gyc), T, 0, st>>>(d_reg, d_voff, d_coff, conn_local, v0, b.rflags, cell_member);
+  k_region_count<<<(unsigned)NRrows, T, 0, st>>>(d_reg, d_voff, b.rflags, b.rcount);
+  k_fixed_rhs<<<dim3(ns, gyv), T, 0, st>>>(d_sc, d_reg, d_voff, b.rflags, b.rcount, b.fixed, (double2*)b.rhs);
+  k_cell_region<<<dim3(ns, gyc), T, 0, st>>>(d_sc, d_coff, cell_member, combo_mask, combo_first, b.creg_local, d_err);
+  k_material_table<<<(ns + 127) / 128, 128, 0, st>>>(ns, d_sc, d_regoff, d_E_nu, d_mat_first, combo_mask, combo_first,
+                                                    combo_id, b.D, b.n_reg_used);
+  k_cell_region_combos<<<dim3(ns, gyc), T, 0, st>>>(d_coff, combo_id, b.creg_local);
+  CK(ctx, cudaGetLastError());
   ctx->c.launches += 10;
-  A(api_batch_finish(b, b.creg_local, conn_local));
+  rc = api_batch_finish(ctx, b, b.creg_local, conn_local);
+  if (rc != FEA_OK) return rc;
   // material-combination overflow found by k_cell_region -> bit 2 of the batch's error word (read by assemble)
-  if (e == cudaSuccess) {
-    k_merge_err<<<1, 1, 0, st>>>(d_err, b.err_flag + 2);
-    e = cudaGetLastError();
-  }
-#undef A
-  for (void* p : scratch) cudaFreeAsync(p, st);
-  if (e != cudaSuccess) {
-    rc = api_fail(ctx, e == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, "fea_batch_create_from_conditions", e);
-    api_free_batch(hb);
-    return rc;
-  }
-  *out = hb;
+  k_merge_err<<<1, 1, 0, st>>>(d_err, b.err_flag + 2);
+  CK(ctx, cudaGetLastError());
+  *out = hb.release();
   return FEA_OK;
 }
 
@@ -876,26 +851,26 @@ int fea_batch_get_setup(fea_batch* hb, uint8_t* fixed, int8_t* cell_region, doub
   fea_ctx* ctx = hb->owner;
   Batch& b = hb->b;
   if (!b.from_conditions) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_setup needs a batch made by fea_batch_create_from_conditions");
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  if (fixed) CKC(ctx, cudaMemcpyAsync(fixed, b.fixed, (size_t)b.NV, cudaMemcpyDeviceToHost, st));
-  if (cell_region) CKC(ctx, cudaMemcpyAsync(cell_region, b.creg_local, (size_t)b.NC, cudaMemcpyDeviceToHost, st));
-  if (rhs) CKC(ctx, cudaMemcpyAsync(rhs, b.rhs, sizeof(double) * 2 * b.NV, cudaMemcpyDeviceToHost, st));
+  if (fixed) CK(ctx, cudaMemcpyAsync(fixed, b.fixed, (size_t)b.NV, cudaMemcpyDeviceToHost, st));
+  if (cell_region) CK(ctx, cudaMemcpyAsync(cell_region, b.creg_local, (size_t)b.NC, cudaMemcpyDeviceToHost, st));
+  if (rhs) CK(ctx, cudaMemcpyAsync(rhs, b.rhs, sizeof(double) * 2 * b.NV, cudaMemcpyDeviceToHost, st));
   std::vector<int32_t> cnt;
   if (region_count) {
     cnt.resize((size_t)b.NR);
-    CKC(ctx, cudaMemcpyAsync(cnt.data(), b.rcount, sizeof(int32_t) * b.NR, cudaMemcpyDeviceToHost, st));
+    CK(ctx, cudaMemcpyAsync(cnt.data(), b.rcount, sizeof(int32_t) * b.NR, cudaMemcpyDeviceToHost, st));
   }
   if (region_flags) {   // every sample's block without its trailing plate-mask row
     size_t o = 0;
     for (int s = 0; s < b.ns; ++s) {
       const size_t nv = (size_t)(b.vtx_off[s + 1] - b.vtx_off[s]);
       const size_t bytes = (size_t)(b.sreg_off[s + 1] - b.sreg_off[s] - 1) * nv;
-      if (bytes) CKC(ctx, cudaMemcpyAsync(region_flags + o, b.rflags + b.flag_off[s], bytes, cudaMemcpyDeviceToHost, st));
+      if (bytes) CK(ctx, cudaMemcpyAsync(region_flags + o, b.rflags + b.flag_off[s], bytes, cudaMemcpyDeviceToHost, st));
       o += bytes;
     }
   }
-  CKC(ctx, cudaStreamSynchronize(st));
+  CK(ctx, cudaStreamSynchronize(st));
   if (region_count) {
     size_t o = 0;
     for (int s = 0; s < b.ns; ++s)
@@ -908,15 +883,15 @@ int fea_batch_get_materials(fea_batch* hb, int32_t* reg_off, int32_t* n_used, do
   if (!hb) return FEA_BAD_ARG;
   fea_ctx* ctx = hb->owner;
   Batch& b = hb->b;
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
   if (reg_off) memcpy(reg_off, b.reg_off.data(), sizeof(int32_t) * (b.ns + 1));
   if (n_used) {
-    if (b.n_reg_used) CKC(ctx, cudaMemcpyAsync(n_used, b.n_reg_used, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+    if (b.n_reg_used) CK(ctx, cudaMemcpyAsync(n_used, b.n_reg_used, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
     else for (int s = 0; s < b.ns; ++s) n_used[s] = b.reg_off[s + 1] - b.reg_off[s];
   }
-  if (D && b.NREG) CKC(ctx, cudaMemcpyAsync(D, b.D, sizeof(double) * 9 * b.NREG, cudaMemcpyDeviceToHost, st));
-  CKC(ctx, cudaStreamSynchronize(st));
+  if (D && b.NREG) CK(ctx, cudaMemcpyAsync(D, b.D, sizeof(double) * 9 * b.NREG, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 
@@ -931,21 +906,21 @@ int fea_batch_rasterize_regions(fea_batch* hb, const uint8_t* with_plate_mask, u
     field_off[s + 1] = field_off[s] + (b.sreg_off[s + 1] - b.sreg_off[s] - 1) + ((with_plate_mask && with_plate_mask[s]) ? 1 : 0);
   const int64_t n_img = field_off[b.ns];
   if (n_img == 0) return FEA_OK;
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
   const size_t per = (size_t)b.img_size * b.img_size, tabb = sizeof(int64_t) * (b.ns + 1);
-  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
-  const size_t o_go = up(tabb), o_im = o_go + up(tabb), total = o_im + up(n_img * per);
-  char* dv = nullptr;
-  CKC(ctx, cudaMallocAsync((void**)&dv, total, st));
-  cudaError_t e = cudaMemcpyAsync(dv, field_off.data(), tabb, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(dv + o_go, b.flag_off.data(), tabb, cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = launch_raster_flags(b, n_img, (const int64_t*)dv, (const int64_t*)(dv + o_go), b.rflags, (uint8_t*)(dv + o_im));
-  if (e == cudaSuccess) e = cudaMemcpyAsync(images, dv + o_im, n_img * per, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // field_off (host vector) must outlive the copy
-  cudaFreeAsync(dv, st);
+  Scratch scratch(st);
+  int64_t *d_field_off = nullptr, *d_flag_off = nullptr;
+  uint8_t* d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_field_off, b.ns + 1));
+  CK(ctx, scratch.alloc(&d_flag_off, b.ns + 1));
+  CK(ctx, scratch.alloc(&d_images, n_img * (int64_t)per));
+  CK(ctx, cudaMemcpyAsync(d_field_off, field_off.data(), tabb, cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_flag_off, b.flag_off.data(), tabb, cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_raster_flags(b, n_img, d_field_off, d_flag_off, b.rflags, d_images));
   ctx->c.launches += 1;
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_rasterize_regions", e);
+  CK(ctx, cudaMemcpyAsync(images, d_images, n_img * per, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));   // field_off (host vector) must outlive the copy
   return FEA_OK;
 }
 
@@ -954,16 +929,15 @@ int fea_batch_classify(fea_batch* hb, int32_t* floating_parts, int32_t* empty_ve
   fea_ctx* ctx = hb->owner;
   Batch& b = hb->b;
   if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_classify before fea_batch_assemble");
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
+  Scratch scratch(st);
   int32_t* dv = nullptr;
-  CKC(ctx, cudaMallocAsync((void**)&dv, sizeof(int32_t) * 2 * b.ns, st));
-  cudaError_t e = launch_classify(b, dv, dv + b.ns);
-  if (e == cudaSuccess && floating_parts) e = cudaMemcpyAsync(floating_parts, dv, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess && empty_vertices) e = cudaMemcpyAsync(empty_vertices, dv + b.ns, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  cudaFreeAsync(dv, st);
-  if (e != cudaSuccess) return api_fail(ctx, FEA_CUDA_ERROR, "fea_batch_classify", e);
+  CK(ctx, scratch.alloc(&dv, 2 * (int64_t)b.ns));
+  CK(ctx, launch_classify(b, dv, dv + b.ns));
+  if (floating_parts) CK(ctx, cudaMemcpyAsync(floating_parts, dv, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  if (empty_vertices) CK(ctx, cudaMemcpyAsync(empty_vertices, dv + b.ns, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 
@@ -975,28 +949,33 @@ int fea_batch_stage_outputs(fea_batch* hb, const uint8_t* with_plate_mask) {
   fea_ctx* ctx = hb->owner;
   Batch& b = hb->b;
   if (!b.rasterized) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_stage_outputs before fea_batch_rasterize");
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  if (!b.ev_staged) CKC(ctx, cudaEventCreateWithFlags(&b.ev_staged, cudaEventDisableTiming));
-  if (b.from_conditions && !b.stage_class) {
-    b.stage_field_off.assign(b.ns + 1, 0);
+  if (!b.ev_staged) CK(ctx, cudaEventCreateWithFlags(&b.ev_staged, cudaEventDisableTiming));
+  if (b.from_conditions && !b.stage_class) {   // committed to b last, so that a failed call is staged again in full
+    std::vector<int64_t> field_off(b.ns + 1, 0);
     for (int s = 0; s < b.ns; ++s)
-      b.stage_field_off[s + 1] = b.stage_field_off[s] + (b.sreg_off[s + 1] - b.sreg_off[s] - 1) + ((with_plate_mask && with_plate_mask[s]) ? 1 : 0);
-    const int64_t n_img = b.stage_field_off[b.ns];
+      field_off[s + 1] = field_off[s] + (b.sreg_off[s + 1] - b.sreg_off[s] - 1) + ((with_plate_mask && with_plate_mask[s]) ? 1 : 0);
+    const int64_t n_img = field_off[b.ns];
     const size_t per = (size_t)b.img_size * b.img_size;
-    CKC(ctx, dalloc(b, &b.stage_class, (int64_t)2 * b.ns));
-    CKC(ctx, launch_classify(b, b.stage_class, b.stage_class + b.ns));
+    int32_t* cls = nullptr;
+    uint8_t* regions = nullptr;
+    CK(ctx, dalloc(b, &cls, (int64_t)2 * b.ns));
+    CK(ctx, launch_classify(b, cls, cls + b.ns));
     if (n_img > 0) {
       int64_t* tab = nullptr;
-      CKC(ctx, dalloc(b, &tab, (int64_t)2 * (b.ns + 1)));
-      CKC(ctx, dalloc(b, &b.stage_regions, (int64_t)(n_img * per)));
-      CKC(ctx, cudaMemcpyAsync(tab, b.stage_field_off.data(), sizeof(int64_t) * (b.ns + 1), cudaMemcpyHostToDevice, st));
-      CKC(ctx, cudaMemcpyAsync(tab + b.ns + 1, b.flag_off.data(), sizeof(int64_t) * (b.ns + 1), cudaMemcpyHostToDevice, st));
-      CKC(ctx, launch_raster_flags(b, n_img, tab, tab + b.ns + 1, b.rflags, b.stage_regions));
+      CK(ctx, dalloc(b, &tab, (int64_t)2 * (b.ns + 1)));
+      CK(ctx, dalloc(b, &regions, (int64_t)(n_img * per)));
+      CK(ctx, cudaMemcpyAsync(tab, field_off.data(), sizeof(int64_t) * (b.ns + 1), cudaMemcpyHostToDevice, st));
+      CK(ctx, cudaMemcpyAsync(tab + b.ns + 1, b.flag_off.data(), sizeof(int64_t) * (b.ns + 1), cudaMemcpyHostToDevice, st));
+      CK(ctx, launch_raster_flags(b, n_img, tab, tab + b.ns + 1, b.rflags, regions));
       ctx->c.launches += 1;
     }
+    b.stage_class = cls;
+    b.stage_regions = regions;
+    b.stage_field_off = std::move(field_off);
   }
-  CKC(ctx, cudaEventRecord(b.ev_staged, st));
+  CK(ctx, cudaEventRecord(b.ev_staged, st));
   return FEA_OK;
 }
 
@@ -1016,21 +995,21 @@ int fea_batch_fetch_outputs(fea_batch* hb, fea_ctx* copy_ctx, double* u, double*
   if ((region_images || floating_parts || empty_vertices) && !b.stage_class)
     return api_fail(ctx, FEA_BAD_STATE, "region images / classifier need a batch made by fea_batch_create_from_conditions");
   if (ctx->c.device != hb->owner->c.device) return api_fail(ctx, FEA_BAD_ARG, "copy context on another device");
-  CKC(ctx, cudaSetDevice(ctx->c.device));
+  CK(ctx, cudaSetDevice(ctx->c.device));
   cudaStream_t st = ctx->c.stream;
-  CKC(ctx, cudaStreamWaitEvent(st, b.ev_staged, 0));
+  CK(ctx, cudaStreamWaitEvent(st, b.ev_staged, 0));
   const size_t per = (size_t)b.img_size * b.img_size;
-  if (u) CKC(ctx, cudaMemcpyAsync(u, b.u, sizeof(double) * 2 * b.NV, cudaMemcpyDeviceToHost, st));
-  if (ranges) CKC(ctx, cudaMemcpyAsync(ranges, b.ranges, sizeof(double) * 4 * b.ns, cudaMemcpyDeviceToHost, st));
-  if (iters) CKC(ctx, cudaMemcpyAsync(iters, b.sc.iters, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
-  if (relres) CKC(ctx, cudaMemcpyAsync(relres, b.relres, sizeof(double) * b.ns, cudaMemcpyDeviceToHost, st));
-  if (status) CKC(ctx, cudaMemcpyAsync(status, b.sc.status, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
-  if (images) CKC(ctx, cudaMemcpyAsync(images, b.images, (size_t)b.ns * 2 * per, cudaMemcpyDeviceToHost, st));
+  if (u) CK(ctx, cudaMemcpyAsync(u, b.u, sizeof(double) * 2 * b.NV, cudaMemcpyDeviceToHost, st));
+  if (ranges) CK(ctx, cudaMemcpyAsync(ranges, b.ranges, sizeof(double) * 4 * b.ns, cudaMemcpyDeviceToHost, st));
+  if (iters) CK(ctx, cudaMemcpyAsync(iters, b.sc.iters, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  if (relres) CK(ctx, cudaMemcpyAsync(relres, b.relres, sizeof(double) * b.ns, cudaMemcpyDeviceToHost, st));
+  if (status) CK(ctx, cudaMemcpyAsync(status, b.sc.status, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  if (images) CK(ctx, cudaMemcpyAsync(images, b.images, (size_t)b.ns * 2 * per, cudaMemcpyDeviceToHost, st));
   if (region_images && b.stage_regions)
-    CKC(ctx, cudaMemcpyAsync(region_images, b.stage_regions, (size_t)b.stage_field_off[b.ns] * per, cudaMemcpyDeviceToHost, st));
-  if (floating_parts) CKC(ctx, cudaMemcpyAsync(floating_parts, b.stage_class, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
-  if (empty_vertices) CKC(ctx, cudaMemcpyAsync(empty_vertices, b.stage_class + b.ns, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
-  CKC(ctx, cudaStreamSynchronize(st));
+    CK(ctx, cudaMemcpyAsync(region_images, b.stage_regions, (size_t)b.stage_field_off[b.ns] * per, cudaMemcpyDeviceToHost, st));
+  if (floating_parts) CK(ctx, cudaMemcpyAsync(floating_parts, b.stage_class, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  if (empty_vertices) CK(ctx, cudaMemcpyAsync(empty_vertices, b.stage_class + b.ns, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 

@@ -19,6 +19,7 @@
 // Dot products: one partial per CTA, summed by one block in a fixed order (bitwise reproducible).
 #include <cmath>
 #include <cstdio>
+#include <memory>
 #include <vector>
 
 #include "fea_internal.cuh"
@@ -671,13 +672,6 @@ void accumulate_level_ms(Mg& mg) {
   }
 }
 
-#define MGCK(call)                                                                                              \
-  do {                                                                                                          \
-    cudaError_t e_ = (call);                                                                                    \
-    if (e_ != cudaSuccess)                                                                                      \
-      return api_fail(ctx, e_ == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, #call, e_);    \
-  } while (0)
-
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------
@@ -688,7 +682,7 @@ int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels) {
     if (nc % 4 != 0 || nc == 0) return api_fail(ctx, FEA_MESH_ERROR, "cell count is not that of a uniform refinement");
     nc /= 4;
   }
-  Mg* mg = new Mg();
+  std::unique_ptr<Mg> mg(new Mg());
   mg->levels = levels;
   mg->lev.resize(levels + 1);
   MgLevel& top = mg->lev[levels];
@@ -697,72 +691,51 @@ int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels) {
   top.nc = b.NC;
   top.conn = b.conn_given;
   top.creg = b.cell_dreg;
+  Scratch scratch(st);
   int32_t* flag = nullptr;
   unsigned long long* key = nullptr;
   int32_t* tmp = nullptr;
-  cudaError_t e = cudaSuccess;
-  int rc = FEA_OK;
-#define A(call) if (e == cudaSuccess) e = (call)
-  A(cudaMallocAsync((void**)&flag, 2 * sizeof(int32_t), st));
-  A(cudaMallocAsync((void**)&key, sizeof(unsigned long long) * std::max<int64_t>(1, b.NV), st));
-  A(cudaMallocAsync((void**)&tmp, sizeof(int32_t) * (b.NV / 4096 + 4), st));
-  for (int l = levels; l >= 1 && e == cudaSuccess && rc == FEA_OK; --l) {
+  CK(ctx, scratch.alloc(&flag, 2));
+  CK(ctx, scratch.alloc(&key, b.NV));
+  CK(ctx, scratch.alloc(&tmp, b.NV / 4096 + 4));
+  for (int l = levels; l >= 1; --l) {
     MgLevel& F = mg->lev[l];
     MgLevel& C = mg->lev[l - 1];
     C.nc = F.nc / 4;
-    A(dalloc(b, &C.conn, C.nc * 3));
-    A(dalloc(b, &C.creg, C.nc));
-    A(dalloc(b, &C.creg8, C.nc));
-    A(dalloc(b, &F.par, F.nv));
-    A(cudaMemsetAsync(flag, 0, 2 * sizeof(int32_t), st));
-    A(cudaMemsetAsync(key, 0xFF, sizeof(unsigned long long) * F.nv, st));
-    if (e != cudaSuccess) break;
+    CK(ctx, dalloc(b, &C.conn, C.nc * 3));
+    CK(ctx, dalloc(b, &C.creg, C.nc));
+    CK(ctx, dalloc(b, &C.creg8, C.nc));
+    CK(ctx, dalloc(b, &F.par, F.nv));
+    CK(ctx, cudaMemsetAsync(flag, 0, 2 * sizeof(int32_t), st));
+    CK(ctx, cudaMemsetAsync(key, 0xFF, sizeof(unsigned long long) * F.nv, st));
     k_mg_derive<<<(unsigned)((C.nc + 255) / 256), 256, 0, st>>>(C.nc, F.nv, F.conn, F.creg, b.xy, C.conn, C.creg, C.creg8, key, flag);
     int32_t h[2] = {0, 0};
-    A(cudaMemcpyAsync(h, flag, sizeof(h), cudaMemcpyDeviceToHost, st));
-    A(cudaStreamSynchronize(st));
-    if (e != cudaSuccess) break;
-    if (h[0]) {
-      rc = api_fail(ctx, FEA_MESH_ERROR, (h[0] & 1) ? "children of a cell are not those of a uniform red refinement"
-                                         : (h[0] & 2) ? "a midpoint is shared by two different edges"
-                                                      : "a midpoint is not at the middle of its edge (bit for bit)");
-      break;
-    }
+    CK(ctx, cudaMemcpyAsync(h, flag, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CK(ctx, cudaStreamSynchronize(st));
+    if (h[0])
+      return api_fail(ctx, FEA_MESH_ERROR, (h[0] & 1) ? "children of a cell are not those of a uniform red refinement"
+                                           : (h[0] & 2) ? "a midpoint is shared by two different edges"
+                                                        : "a midpoint is not at the middle of its edge (bit for bit)");
     C.nv = (int64_t)h[1] + 1;
-    A(dalloc(b, &F.child_ptr, C.nv + 1));
-    A(dalloc(b, &F.child, 2 * (F.nv - C.nv)));
+    CK(ctx, dalloc(b, &F.child_ptr, C.nv + 1));
+    CK(ctx, dalloc(b, &F.child, 2 * (F.nv - C.nv)));
     int32_t* cnt = nullptr;
-    A(cudaMallocAsync((void**)&cnt, sizeof(int32_t) * (C.nv + 1), st));
-    A(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
-    if (e != cudaSuccess) break;
+    CK(ctx, scratch.alloc(&cnt, C.nv + 1));
+    CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
     k_mg_parents<<<(unsigned)((F.nv + 255) / 256), 256, 0, st>>>(F.nv, (int)C.nv, key, F.par, cnt, flag);
     // the midpoint lists are built from par: only once every vertex from n_c on is known to be a midpoint
-    A(cudaMemcpyAsync(h, flag, sizeof(h), cudaMemcpyDeviceToHost, st));
-    A(cudaStreamSynchronize(st));
-    if (e == cudaSuccess && h[0]) {
-      cudaFreeAsync(cnt, st);
-      rc = api_fail(ctx, FEA_MESH_ERROR, "vertices are not numbered coarse vertices first, then one midpoint per coarse edge");
-      break;
-    }
-    A(exclusive_scan_i32(cnt, F.child_ptr, C.nv, tmp, st));
-    A(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
-    if (F.nv > C.nv && e == cudaSuccess)
+    CK(ctx, cudaMemcpyAsync(h, flag, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CK(ctx, cudaStreamSynchronize(st));
+    if (h[0]) return api_fail(ctx, FEA_MESH_ERROR, "vertices are not numbered coarse vertices first, then one midpoint per coarse edge");
+    CK(ctx, exclusive_scan_i32(cnt, F.child_ptr, C.nv, tmp, st));
+    CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
+    if (F.nv > C.nv)
       k_mg_child_fill<<<(unsigned)((F.nv - C.nv + 255) / 256), 256, 0, st>>>(F.nv, (int)C.nv, F.par, F.child_ptr, cnt, F.child);
-    if (e == cudaSuccess) k_mg_child_sort<<<(unsigned)((C.nv + 255) / 256), 256, 0, st>>>((int)C.nv, F.child_ptr, F.child);
-    A(cudaGetLastError());
-    if (cnt) cudaFreeAsync(cnt, st);
+    k_mg_child_sort<<<(unsigned)((C.nv + 255) / 256), 256, 0, st>>>((int)C.nv, F.child_ptr, F.child);
+    CK(ctx, cudaGetLastError());
     ctx->c.launches += 5;
   }
-#undef A
-  if (flag) cudaFreeAsync(flag, st);
-  if (key) cudaFreeAsync(key, st);
-  if (tmp) cudaFreeAsync(tmp, st);
-  if (e != cudaSuccess) rc = api_fail(ctx, e == cudaErrorMemoryAllocation ? FEA_OUT_OF_MEMORY : FEA_CUDA_ERROR, "fea_batch_set_refinement", e);
-  if (rc != FEA_OK) {
-    delete mg;
-    return rc;
-  }
-  b.mg = mg;
+  b.mg = mg.release();
   return FEA_OK;
 }
 
@@ -779,15 +752,15 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
     if (rc != FEA_OK) return rc;
     Batch& cb = C.hb->b;
     C.b = &cb;
-    MGCK(dalloc(cb, &cb.xy, cb.NV * 2));
-    MGCK(dalloc(cb, &cb.D, (int64_t)cb.NREG * 9));
-    MGCK(dalloc(cb, &cb.fixed, cb.NV));
-    MGCK(dalloc(cb, &cb.rhs, cb.NV * 2));
-    MGCK(cudaMemcpyAsync(cb.xy, b.xy, sizeof(double) * 2 * cb.NV, cudaMemcpyDeviceToDevice, st));   // a prefix of the finest
-    MGCK(cudaMemcpyAsync(cb.D, b.D, sizeof(double) * 9 * cb.NREG, cudaMemcpyDeviceToDevice, st));
-    MGCK(cudaMemcpyAsync(cb.fixed, b.fixed, cb.NV, cudaMemcpyDeviceToDevice, st));
-    MGCK(cudaMemsetAsync(cb.rhs, 0, sizeof(double) * 2 * cb.NV, st));
-    MGCK(api_batch_finish(cb, C.creg8, C.conn));
+    CK(ctx, dalloc(cb, &cb.xy, cb.NV * 2));
+    CK(ctx, dalloc(cb, &cb.D, (int64_t)cb.NREG * 9));
+    CK(ctx, dalloc(cb, &cb.fixed, cb.NV));
+    CK(ctx, dalloc(cb, &cb.rhs, cb.NV * 2));
+    CK(ctx, cudaMemcpyAsync(cb.xy, b.xy, sizeof(double) * 2 * cb.NV, cudaMemcpyDeviceToDevice, st));   // a prefix of the finest
+    CK(ctx, cudaMemcpyAsync(cb.D, b.D, sizeof(double) * 9 * cb.NREG, cudaMemcpyDeviceToDevice, st));
+    CK(ctx, cudaMemcpyAsync(cb.fixed, b.fixed, cb.NV, cudaMemcpyDeviceToDevice, st));
+    CK(ctx, cudaMemsetAsync(cb.rhs, 0, sizeof(double) * 2 * cb.NV, st));
+    if ((rc = api_batch_finish(ctx, cb, C.creg8, C.conn)) != FEA_OK) return rc;
     const Batch& fb = *F.b;
     const int2* par = F.par;
     rc = api_batch_assemble(ctx, cb, [&fb, par](Batch& c) -> cudaError_t {
@@ -799,29 +772,29 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
   }
   // vectors: outer CG on the finest level, V-cycle state on every smoothed level
   const int64_t nbr = b.NBR;
-  MGCK(dalloc(b, &mg.r, nbr));
-  MGCK(dalloc(b, &mg.p, nbr));
-  MGCK(dalloc(b, &mg.q, nbr));
-  MGCK(dalloc(b, &mg.partA, nbr / kT));
-  MGCK(dalloc(b, &mg.partB, nbr / kT));
-  MGCK(dalloc(b, &mg.sc, kScCount + 2 * kLanczos));
-  MGCK(cudaMemsetAsync(mg.sc, 0, sizeof(double) * (kScCount + 2 * kLanczos), st));
+  CK(ctx, dalloc(b, &mg.r, nbr));
+  CK(ctx, dalloc(b, &mg.p, nbr));
+  CK(ctx, dalloc(b, &mg.q, nbr));
+  CK(ctx, dalloc(b, &mg.partA, nbr / kT));
+  CK(ctx, dalloc(b, &mg.partB, nbr / kT));
+  CK(ctx, dalloc(b, &mg.sc, kScCount + 2 * kLanczos));
+  CK(ctx, cudaMemsetAsync(mg.sc, 0, sizeof(double) * (kScCount + 2 * kLanczos), st));
   for (int l = 1; l <= mg.levels; ++l) {
     MgLevel& L = mg.lev[l];
     const int64_t n = L.b->NBR;
     double2** v[5] = {&L.x, &L.r, &L.d[0], &L.d[1], &L.bv};   // the finest level's b is the outer CG's r
     for (double2** p : v) {
       if (p == &L.bv && l == mg.levels) continue;
-      MGCK(dalloc(b, p, n));
-      MGCK(cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st));
+      CK(ctx, dalloc(b, p, n));
+      CK(ctx, cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st));
     }
   }
-  if (!mg.h_sc) MGCK(cudaHostAlloc((void**)&mg.h_sc, sizeof(double) * kScCount, cudaHostAllocDefault));
+  if (!mg.h_sc) CK(ctx, cudaHostAlloc((void**)&mg.h_sc, sizeof(double) * kScCount, cudaHostAllocDefault));
   if (mg.ev.empty()) {
     mg.ev.resize(4 * (mg.levels + 1) + 2);
-    for (auto& ev : mg.ev) MGCK(cudaEventCreate(&ev));
+    for (auto& ev : mg.ev) CK(ctx, cudaEventCreate(&ev));
   }
-  for (int l = 0; l <= mg.levels; ++l) MGCK(estimate_lmax(b, mg.lev[l]));
+  for (int l = 0; l <= mg.levels; ++l) CK(ctx, estimate_lmax(b, mg.lev[l]));
   return FEA_OK;
 }
 
@@ -832,11 +805,11 @@ int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z) {
   if (!g) return FEA_OK;
   for (auto& L : mg.lev) L.ms = 0.0;
   k_mg_load<<<g, kT, 0, st>>>(side_of(b), b.vrank, d_r, mg.r);
-  MGCK(vcycle_top(ctx, b, mg.r));
+  CK(ctx, vcycle_top(ctx, b, mg.r));
   k_mg_store<<<g, kT, 0, st>>>(side_of(b), b.vrank, mg.lev[mg.levels].x, d_z);
   ctx->c.launches += 2;
-  MGCK(cudaGetLastError());
-  MGCK(cudaStreamSynchronize(st));
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaStreamSynchronize(st));
   accumulate_level_ms(mg);
   return FEA_OK;
 }
@@ -857,27 +830,27 @@ int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
   b.t_update.clear();
   for (auto& L : mg.lev) L.ms = 0.0;
   const int64_t launches0 = c.launches;
-  MGCK(cudaEventRecord(ev0, st));
+  CK(ctx, cudaEventRecord(ev0, st));
   int32_t empty = 0;
-  MGCK(cudaMemcpyAsync(&empty, b.empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(&empty, b.empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 0, mg.partA);
-  MGCK(reduce(b, mg.partA, nullptr, np, kRedStore, kScRZ0));
-  MGCK(cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
-  MGCK(cudaStreamSynchronize(st));
+  CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScRZ0));
+  CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
   const double rz0 = h[kScRZ0], tol2 = rtol * rtol * rz0;
   int status = FEA_SAMPLE_NOT_RUN, it = 0, restarts = 0, first = 1;
   double rr = rz0;
   if (empty) status = FEA_SAMPLE_EMPTY_ROW;
   else if (!(rz0 > 0.0)) status = std::isfinite(rz0) ? FEA_SAMPLE_CONVERGED : FEA_SAMPLE_BREAKDOWN;
   if (status == FEA_SAMPLE_CONVERGED) {
-    MGCK(cudaMemcpyAsync(mg.sc + kScTrue, &rz0, sizeof(double), cudaMemcpyHostToDevice, st));
+    CK(ctx, cudaMemcpyAsync(mg.sc + kScTrue, &rz0, sizeof(double), cudaMemcpyHostToDevice, st));
   }
   while (status == FEA_SAMPLE_NOT_RUN) {
     if (rr <= tol2) {   // recursive residual met the tolerance: decide on the TRUE residual
       k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 2, mg.partA);
-      MGCK(reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
-      MGCK(cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
-      MGCK(cudaStreamSynchronize(st));
+      CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
+      CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
+      CK(ctx, cudaStreamSynchronize(st));
       c.launches += 2;
       rr = h[kScTrue];
       if (rr <= tol2) { status = FEA_SAMPLE_CONVERGED; break; }
@@ -886,17 +859,17 @@ int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
       first = 1;   // restart from the true residual (p = q = 0)
     }
     if (it >= max_iter) { status = FEA_SAMPLE_MAX_ITER; break; }
-    MGCK(vcycle_top(ctx, b, mg.r));
+    CK(ctx, vcycle_top(ctx, b, mg.r));
     const double2* z = mg.lev[mg.levels].x;
     k_mg_fcg_dots<<<g, kT, 0, st>>>(z, mg.r, mg.q, mg.partA, mg.partB);
-    MGCK(reduce(b, mg.partA, mg.partB, np, kRedDots, 0, first));
+    CK(ctx, reduce(b, mg.partA, mg.partB, np, kRedDots, 0, first));
     k_mg_fcg_dir<<<g, kT, 0, st>>>(z, mg.p, mg.sc);
     k_mg_fcg_spmv<<<g, kT, 0, st>>>(A, mg.p, mg.q, mg.partA);
-    MGCK(reduce(b, mg.partA, nullptr, np, kRedPQ));
+    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedPQ));
     k_mg_fcg_update<<<g, kT, 0, st>>>(x, mg.r, mg.p, mg.q, mg.sc, mg.partA);
-    MGCK(reduce(b, mg.partA, nullptr, np, kRedStore, kScRR));
-    MGCK(cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
-    MGCK(cudaStreamSynchronize(st));   // one host poll per outer iteration (the coarse solve polls anyway)
+    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScRR));
+    CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
+    CK(ctx, cudaStreamSynchronize(st));   // one host poll per outer iteration (the coarse solve polls anyway)
     c.launches += 8;
     accumulate_level_ms(mg);
     if (!(h[kScPQ] > 0.0) || !std::isfinite(h[kScPQ]) || !std::isfinite(h[kScAlpha]) || !std::isfinite(h[kScRR])) {
@@ -904,7 +877,7 @@ int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
       // relres are those of the last sound iterate
       status = FEA_SAMPLE_BREAKDOWN;
       k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 1, mg.partA);
-      MGCK(reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
+      CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
       break;
     }
     ++it;
@@ -913,13 +886,13 @@ int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
   }
   if (status == FEA_SAMPLE_MAX_ITER || status == FEA_SAMPLE_STAGNATED) {
     k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 1, mg.partA);
-    MGCK(reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
+    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
   }
   k_mg_finish<<<1, 32, 0, st>>>(b.sc, b.rz_last, mg.sc, status, it);
-  MGCK(cudaGetLastError());
-  MGCK(launch_finalize(b));
-  MGCK(cudaEventRecord(ev1, st));
-  MGCK(cudaStreamSynchronize(st));
+  CK(ctx, cudaGetLastError());
+  CK(ctx, launch_finalize(b));
+  CK(ctx, cudaEventRecord(ev1, st));
+  CK(ctx, cudaStreamSynchronize(st));
   b.stats.iterations = it;
   b.stats.n_converged = status == FEA_SAMPLE_CONVERGED ? 1 : 0;
   b.stats.refined_systems = restarts > 0 ? 1 : 0;

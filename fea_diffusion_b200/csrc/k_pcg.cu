@@ -609,9 +609,16 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
   if ((e = cudaEventRecord(c.ev_t1, st)) != cudaSuccess) return e;
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
   // statistics
-  std::vector<int32_t> it(b.ns), stt(b.ns);
+  std::vector<int32_t> it(b.ns), stt(b.ns), order(n_cluster > 0 ? b.cl_off[8] + b.cl_cnt[8] : 0);
+  int32_t h_restarts = 0;
+  long long h_reads[3] = {0, 0, 0};
   if ((e = cudaMemcpyAsync(it.data(), b.sc.iters, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
   if ((e = cudaMemcpyAsync(stt.data(), b.sc.status, sizeof(int32_t) * b.ns, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+  if (n_cluster > 0) {
+    if ((e = cudaMemcpyAsync(order.data(), b.cl_order, sizeof(int32_t) * order.size(), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&h_restarts, b.cl_counter, sizeof(int32_t), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(h_reads, b.cl_counter + 16, sizeof(h_reads), cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+  }
   if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
   int itmax = 0, nconv = 0;
   for (int s = 0; s < b.ns; ++s) {
@@ -621,8 +628,6 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
   b.stats.iterations = itmax;
   b.stats.n_converged = nconv;
   if (n_cluster > 0) {
-    std::vector<int32_t> order(b.cl_off[8] + b.cl_cnt[8]);
-    if ((e = cudaMemcpy(order.data(), b.cl_order, sizeof(int32_t) * order.size(), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
     int64_t tot = 0;
     int nclusters = 0;
     int best = 1;
@@ -637,11 +642,7 @@ cudaError_t run_pcg(Batch& b, double rtol, int max_iter) {
     b.stats.cluster_count = nclusters;
     b.stats.cluster_iterations = tot;
     cudaEventElapsedTime(&b.stats.cluster_ms, c.ev_c0, c.ev_c1);
-    int32_t h_restarts = 0;
-    if ((e = cudaMemcpy(&h_restarts, b.cl_counter, sizeof(int32_t), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
     b.stats.refined_systems += h_restarts;
-    long long h_reads[3] = {0, 0, 0};
-    if ((e = cudaMemcpy(h_reads, b.cl_counter + 16, sizeof(h_reads), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
     b.stats.cluster_block_reads_tmem = h_reads[0];
     b.stats.cluster_block_reads_smem = h_reads[1];
     b.stats.cluster_block_reads_l2 = h_reads[2];

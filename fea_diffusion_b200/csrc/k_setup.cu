@@ -420,12 +420,12 @@ cudaError_t launch_cluster_order(Batch& b) {
   if (n_out == 0) return cudaSuccess;
   int n2 = 2;
   while (n2 < b.ns) n2 <<= 1;
+  Scratch scratch(st);
   unsigned long long* keys = nullptr;
-  cudaError_t e = cudaMallocAsync((void**)&keys, sizeof(unsigned long long) * n2, st);
+  cudaError_t e = scratch.alloc(&keys, n2);
   if (e != cudaSuccess) return e;
   k_cluster_order<<<1, 1024, 0, st>>>(b.ns, n2, b.d_vtx_off, b.n_active, pcg_cluster_rows_per_cta(), b.ctx->cluster_min, 8,
                                       keys, n_out, b.cl_order);
-  cudaFreeAsync(keys, st);
   return cudaGetLastError();
 }
 
@@ -565,18 +565,19 @@ cudaError_t launch_topology_counts(Batch& b) {
   const int T = 256;
   const unsigned gv = (unsigned)((b.NV + T - 1) / T), gc = (unsigned)((b.NC + T - 1) / T);
   // scratch: cnt [NV+1], tmp for scans
+  Scratch scratch(st);
   int32_t* cnt = nullptr;
   int32_t* tmp = nullptr;
   cudaError_t e;
-  if ((e = cudaMallocAsync(&cnt, sizeof(int32_t) * (b.NV + 1), st)) != cudaSuccess) return e;
-  if ((e = cudaMallocAsync(&tmp, sizeof(int64_t) * (b.NV / kScanTile + 4), st)) != cudaSuccess) return e;
-  cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (b.NV + 1), st);
+  if ((e = scratch.alloc(&cnt, b.NV + 1)) != cudaSuccess) return e;
+  if ((e = scratch.alloc(&tmp, b.NV / kScanTile + 4)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (b.NV + 1), st)) != cudaSuccess) return e;
   if (b.NC) {
     if (b.npc == 3) k_inc_count<3><<<gc, T, 0, st>>>(b.conn, b.cell_dreg, b.NC, cnt);
     else k_inc_count<4><<<gc, T, 0, st>>>(b.conn, b.cell_dreg, b.NC, cnt);
   }
-  exclusive_scan_i32(cnt, b.inc_ptr, b.NV, tmp, st);
-  cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (b.NV + 1), st);
+  if ((e = exclusive_scan_i32(cnt, b.inc_ptr, b.NV, tmp, st)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (b.NV + 1), st)) != cudaSuccess) return e;
   if (b.NC) {
     if (b.npc == 3) k_inc_fill<3><<<gc, T, 0, st>>>(b.conn, b.cell_dreg, b.NC, b.inc_ptr, cnt, b.inc);
     else k_inc_fill<4><<<gc, T, 0, st>>>(b.conn, b.cell_dreg, b.NC, b.inc_ptr, cnt, b.inc);
@@ -589,10 +590,7 @@ cudaError_t launch_topology_counts(Batch& b) {
     else
       k_adj_count<4><<<gv, T, 0, st>>>(b.NV, b.inc_ptr, b.inc, b.conn, b.vrank, cnt, max_len, b.err_flag);
   }
-  exclusive_scan_i32(cnt, b.adj_ptr, b.NV, tmp, st);
-  cudaFreeAsync(cnt, st);
-  cudaFreeAsync(tmp, st);
-  return cudaGetLastError();
+  return exclusive_scan_i32(cnt, b.adj_ptr, b.NV, tmp, st);
 }
 
 cudaError_t launch_topology_fill(Batch& b) {
