@@ -834,6 +834,49 @@ int fea_batch_set_refinement(fea_batch* hb, int32_t levels) {
   return mg_set_refinement(ctx, b, levels);
 }
 
+int fea_batch_set_coarse_meshes(fea_batch* hb, const fea_batch_desc* d) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_set_coarse_meshes after fea_batch_assemble");
+  if (b.mg)
+    return api_fail(ctx, FEA_BAD_STATE, b.mg->nonnested ? "the batch already has its coarse meshes"
+                                                        : "the batch already declared its refinement");
+  if (b.ns != 1 || b.npc != 3) return api_fail(ctx, FEA_BAD_ARG, "a multigrid hierarchy needs one sample of triangles");
+  if (!d) return api_fail(ctx, FEA_BAD_ARG, "null coarse mesh description");
+  if (d->n_samples < 1 || d->n_samples > 8) return api_fail(ctx, FEA_BAD_ARG, "1..8 coarse meshes");
+  if (d->nodes_per_cell != 3) return api_fail(ctx, FEA_BAD_ARG, "coarse meshes must be made of triangles");
+  if (!d->vtx_off || !d->cell_off || !d->reg_off || !d->xy || !d->conn || !d->cell_region || !d->D || !d->fixed)
+    return api_fail(ctx, FEA_BAD_ARG, "null array in the coarse mesh description");
+  const int n = d->n_samples;
+  if (d->vtx_off[0] != 0 || d->cell_off[0] != 0 || d->reg_off[0] != 0) return api_fail(ctx, FEA_BAD_ARG, "offset tables must start at 0");
+  for (int s = 0; s < n; ++s) {
+    if (d->cell_off[s + 1] < d->cell_off[s] || d->reg_off[s + 1] < d->reg_off[s])
+      return api_fail(ctx, FEA_BAD_ARG, "offset tables must be non-decreasing");
+    const int64_t nv = d->vtx_off[s + 1] - d->vtx_off[s];
+    const int64_t finer = s + 1 < n ? d->vtx_off[s + 2] - d->vtx_off[s + 1] : b.NV;
+    if (nv < 1 || nv >= finer) {
+      char msg[160];
+      snprintf(msg, sizeof msg, "level %d has %lld vertices, not fewer than level %d's %lld", s, (long long)nv, s + 1,
+               (long long)finer);
+      return api_fail(ctx, FEA_BAD_ARG, msg);
+    }
+  }
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  return mg_set_coarse_meshes(ctx, b, d);
+}
+
+int fea_batch_get_level_transfer(fea_batch* hb, int32_t level, int32_t* indptr, int32_t* indices, double* data) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch has no multigrid hierarchy");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_level_transfer before fea_batch_assemble");
+  if (level < 1 || level > b.mg->levels) return api_fail(ctx, FEA_BAD_ARG, "level out of range");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  return mg_level_transfer(ctx, b, level, indptr, indices, data);
+}
+
 int fea_batch_get_mg_levels(fea_batch* hb, int32_t cap, fea_mg_level* out, int32_t* n_out) {
   if (!hb || !n_out || cap < 0 || (cap > 0 && !out)) return FEA_BAD_ARG;
   fea_ctx* ctx = hb->owner;

@@ -166,7 +166,8 @@ struct Batch {
   Mg* mg = nullptr;
 };
 
-// One level of the multigrid hierarchy of a uniformly refined single-sample batch (DESIGN.md section 3.9).
+// One level of the multigrid hierarchy of a single-sample batch: a uniform refinement (DESIGN.md section
+// 3.9) or a mesh with coarser meshes of the same domain (section 3.10).
 // Level 0 is the coarsest mesh, level `levels` the batch itself.  Vectors are in the level's scaled
 // row space (Khat = S^T K S, rows in the level batch's solver order).
 struct MgLevel {
@@ -178,7 +179,12 @@ struct MgLevel {
   int8_t* creg8 = nullptr;       // [nc] the same as the int8 input of a coarse level batch
   int2* par = nullptr;           // [nv] levels >= 1: (v, -1) for a vertex of level l-1, else the edge's two ends
   int32_t* child_ptr = nullptr;  // [nv(l-1)+1] levels >= 1: vertex of level l-1 -> the midpoints of level l
-  int32_t* child = nullptr;      //   that have it as an end, ascending
+  int32_t* child = nullptr;      //   that have it as an end, ascending (non-nested: every vertex of level l
+                                 //   that has it as a parent, ascending)
+  // non-nested hierarchies only (levels >= 1): up to 3 parents of level l-1 per vertex, -1 = none
+  int32_t* par3 = nullptr;       // [nv*3]
+  double* w3 = nullptr;          // [nv*3] their interpolation weights
+  double* child_w = nullptr;     // weights of the child entries
   double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};   // levels >= 1
   double lmax = 0.0;             // power-iteration estimate of the largest eigenvalue of Khat
   double inv_theta = 0.0, c1[2] = {0.0, 0.0}, c2[2] = {0.0, 0.0};   // Chebyshev coefficients
@@ -186,6 +192,7 @@ struct MgLevel {
 };
 struct Mg {
   int levels = 0;
+  bool nonnested = false;        // coarse levels are the caller's meshes (fea_batch_set_coarse_meshes)
   bool failed = false;           // building the hierarchy failed in fea_batch_assemble: the batch cannot be solved
   std::vector<MgLevel> lev;      // [levels + 1]
   double2 *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, finest row space (x = Batch::x)
@@ -238,6 +245,10 @@ int mg_assemble(fea_ctx* ctx, Batch& b);                     // coarse level bat
 int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter);   // flexible CG preconditioned by V-cycles
 int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z);   // one V-cycle, active-DOF vectors
 void mg_release(Batch& b);
+// non-nested hierarchy (k_mg_nonnested.cu): coarse level batches from `coarse`, point location, transfers
+int mg_set_coarse_meshes(fea_ctx* ctx, Batch& b, const fea_batch_desc* coarse);
+// P_level as CSR over active DOFs (either kind of hierarchy, assembled batch); any array may be NULL
+int mg_level_transfer(fea_ctx* ctx, Batch& b, int level, int32_t* indptr, int32_t* indices, double* data);
 
 template <class T>
 inline cudaError_t dalloc(Batch& b, T** p, int64_t n) {

@@ -17,6 +17,8 @@
 //   coarsest  : run_pcg on the level-0 batch to rtol 1e-4; the inexact coarse solve makes the outer
 //               iteration flexible CG, beta = z+.(r+ - r) / (r.z) = -alpha z+.q / (r.z).
 // Dot products: one partial per CTA, summed by one block in a fixed order (bitwise reproducible).
+// A non-nested hierarchy (fea_batch_set_coarse_meshes, k_mg_nonnested.cu; DESIGN.md section 3.10) runs the same
+// V-cycle and outer CG with rediscretised coarse operators and the k_mgn_* transfers (up to 3 weighted parents).
 #include <cmath>
 #include <cstdio>
 #include <memory>
@@ -441,6 +443,60 @@ __global__ void __launch_bounds__(kT) k_mg_prolong(Side F, Side Cs, const int2* 
   xf[row] = xv;
 }
 
+// non-nested hierarchies (k_mg_nonnested.cu): the same two transfers with up to 3 weighted parents per vertex.
+// Restriction gathers over a coarse vertex's (fine vertex, weight) list, ascending in the fine vertex.
+__global__ void __launch_bounds__(kT) k_mgn_restrict(Side F, Side Cs, const double2* __restrict__ ru,
+                                                     const int32_t* __restrict__ child_ptr, const int32_t* __restrict__ child,
+                                                     const double* __restrict__ child_w, double2* __restrict__ bc,
+                                                     double2* __restrict__ xc, double2* __restrict__ rc, double2* __restrict__ dc,
+                                                     double inv_theta, double2* __restrict__ rhs0) {
+  const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
+  const int j = Cs.vertex_of_row[row];
+  double2 acc = make_double2(0.0, 0.0);
+  if (j >= 0) {
+    for (int i = child_ptr[j]; i < child_ptr[j + 1]; ++i) {
+      const int fr = F.row_of_vertex[child[i]];
+      if (fr < 0) continue;
+      const double w = child_w[i];
+      const double2 t = ru[fr];
+      acc.x = fma(w, t.x, acc.x);
+      acc.y = fma(w, t.y, acc.y);
+    }
+  }
+  if (rhs0) {
+    if (j >= 0) rhs0[j] = acc;
+    return;
+  }
+  const double2 h = j >= 0 ? mul_St(Cs.dscale, Cs.scoup, row, acc) : make_double2(0.0, 0.0);
+  bc[row] = h;
+  rc[row] = h;
+  dc[row] = make_double2(h.x * inv_theta, h.y * inv_theta);
+  xc[row] = make_double2(0.0, 0.0);
+}
+__global__ void __launch_bounds__(kT) k_mgn_prolong(Side F, Side Cs, const int32_t* __restrict__ par3, const double* __restrict__ w3,
+                                                    const double2* __restrict__ xc, double2* __restrict__ xf) {
+  const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
+  const int f = F.vertex_of_row[row];
+  if (f < 0) return;
+  double2 e = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const int p = par3[3 * (int64_t)f + k];
+    if (p < 0) continue;
+    const int r = Cs.row_of_vertex[p];
+    if (r < 0) continue;   // a Dirichlet vertex of the coarse level: no column
+    const double w = w3[3 * (int64_t)f + k];
+    const double2 t = mul_S(Cs.dscale, Cs.scoup, r, xc[r]);
+    e.x = fma(w, t.x, e.x);
+    e.y = fma(w, t.y, e.y);
+  }
+  const double2 c = solve_S(F.dscale, F.scoup, row, e);
+  double2 xv = xf[row];
+  xv.x += c.x;
+  xv.y += c.y;
+  xf[row] = xv;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // outer flexible CG on the finest level
 // r = S^T b (true = 0) or S^T b - Khat x (true = 1); true = 0 also clears x, p, q.  Partials of r.r.
@@ -635,14 +691,20 @@ cudaError_t vcycle(fea_ctx* ctx, Batch& fine, int l) {
   k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], L.d[1], L.x, L.r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
   k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[1], L.d[0], L.x, L.r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
   k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], nullptr, L.x, L.r, 0.0, 0.0, b.dscale, b.scoup, L.d[1]);
-  if (gc)
+  if (gc && mg.nonnested)
+    k_mgn_restrict<<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), L.d[1], L.child_ptr, L.child, L.child_w, C.bv, C.x, C.r,
+                                      C.d[0], C.inv_theta, l == 1 ? (double2*)C.b->rhs : nullptr);
+  else if (gc)
     k_mg_restrict<<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), L.d[1], L.child_ptr, L.child, C.bv, C.x, C.r, C.d[0],
                                      C.inv_theta, l == 1 ? (double2*)C.b->rhs : nullptr);
   cudaEventRecord(ev[1], st);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   if ((e = vcycle(ctx, fine, l - 1)) != cudaSuccess) return e;
   cudaEventRecord(ev[2], st);
-  k_mg_prolong<<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par, l == 1 ? (const double2*)C.b->x : C.x, L.x);
+  if (mg.nonnested)
+    k_mgn_prolong<<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par3, L.w3, l == 1 ? (const double2*)C.b->x : C.x, L.x);
+  else
+    k_mg_prolong<<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par, l == 1 ? (const double2*)C.b->x : C.x, L.x);
   k_mg_resid<<<g, kT, 0, st>>>(A, L.x, L.bv, L.r, L.d[0], L.inv_theta);
   k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], L.d[1], L.x, L.r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
   k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[1], L.d[0], L.x, L.r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
@@ -742,9 +804,16 @@ int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels) {
 int mg_assemble(fea_ctx* ctx, Batch& b) {
   Mg& mg = *b.mg;
   cudaStream_t st = ctx->c.stream;
-  // coarse level batches, finest-but-one first: each one's matrices are the Galerkin product of the next finer
+  // coarse level batches, finest-but-one first: each one's matrices are the Galerkin product of the next finer.
+  // A non-nested hierarchy's coarse batches exist already (mg_set_coarse_meshes) and are rediscretised:
+  // each level's operator is its own mesh's stiffness matrix.
   for (int l = mg.levels - 1; l >= 0; --l) {
     MgLevel& C = mg.lev[l];
+    if (mg.nonnested) {
+      const int rc = fea_batch_assemble(C.hb);
+      if (rc != FEA_OK) return rc;
+      continue;
+    }
     const MgLevel& F = mg.lev[l + 1];
     const int64_t vo[2] = {0, C.nv}, co[2] = {0, C.nc};
     const int32_t ro[2] = {0, b.NREG};

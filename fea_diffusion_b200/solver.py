@@ -690,6 +690,25 @@ class Batch:
         self.ctx._check(self.ctx.lib.fea_batch_get_level_csr(self.h, int(level), ptr(indptr), ptr(indices), ptr(data)))
         return sp.csr_matrix((data, indices, indptr), shape=(n, n))
 
+    def set_coarse_meshes(self, packed: PackedBatch):
+        """Declare coarser meshes of the same domain, ``pack([Sample, ...])`` coarsest first (1..8; their rhs is
+        not read): assemble then builds a non-nested hierarchy (point location, linear interpolation,
+        rediscretised coarse operators) and solve runs multigrid-preconditioned CG."""
+        self.ctx._check(self.ctx.lib.fea_batch_set_coarse_meshes(self.h, C.byref(packed.desc)))
+        return self
+
+    def level_transfer(self, level: int):
+        """scipy CSR of P_level (level-1 -> level) over active DOFs, in the numbering of ``csr``."""
+        import scipy.sparse as sp
+        lv = self.mg_levels()
+        n, m = int(lv[level]["n_active_dofs"]), int(lv[level - 1]["n_active_dofs"])
+        indptr = np.empty(n + 1, np.int32)
+        self.ctx._check(self.ctx.lib.fea_batch_get_level_transfer(self.h, int(level), ptr(indptr), None, None))
+        nnz = int(indptr[-1])
+        indices, data = np.empty(nnz, np.int32), np.empty(nnz)
+        self.ctx._check(self.ctx.lib.fea_batch_get_level_transfer(self.h, int(level), None, ptr(indices), ptr(data)))
+        return sp.csr_matrix((data, indices, indptr), shape=(n, m))
+
     def mg_apply(self, r: np.ndarray) -> np.ndarray:
         """z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as ``spmv``)."""
         r = np.ascontiguousarray(r, dtype=np.float64)

@@ -169,3 +169,59 @@ def large_case(name: str, levels: int, fixtures_path: str = None):
     for v, m in loads:
         s.rhs[v] += m
     return setup, len(c0)
+
+
+def jittered_case(name: str, levels: int, fraction: float = 0.15, seed: int = 0):
+    """``large_case(name, levels)`` with every interior, unconstrained vertex of the last refinement moved by a
+    deterministic jitter of at most ``fraction`` x its shortest incident edge: the mesh is then no uniform
+    refinement, while ``large_case(name, l)`` for l < levels stay meshes of the same domain.  Returns
+    (Sample, n_coarse_vertices); ``levels`` >= 1."""
+    setup, n0 = large_case(name, levels)
+    s = setup.sample
+    co = s.coors.copy()
+    conn = np.asarray(s.conn, dtype=np.int64)
+    n_prev = len(large_case(name, levels - 1)[0].coors)   # vertices that the last refinement did not add
+    e = np.concatenate([conn[:, [0, 1]], conn[:, [1, 2]], conn[:, [2, 0]]])
+    e = np.sort(e, axis=1)
+    key, cnt = np.unique(e[:, 0] * len(co) + e[:, 1], return_counts=True)
+    e0, e1 = key // len(co), key % len(co)
+    boundary = np.zeros(len(co), bool)
+    boundary[e0[cnt == 1]] = boundary[e1[cnt == 1]] = True
+    length = np.linalg.norm(co[e0] - co[e1], axis=1)
+    shortest = np.full(len(co), np.inf)
+    np.minimum.at(shortest, e0, length)
+    np.minimum.at(shortest, e1, length)
+    move = np.flatnonzero((np.arange(len(co)) >= n_prev) & ~boundary & ~s.fixed.astype(bool))
+    rng = np.random.default_rng(seed)
+    ang = rng.uniform(0.0, 2.0 * np.pi, len(move))
+    rad = fraction * shortest[move] * rng.uniform(0.0, 1.0, len(move))
+    co[move, 0] += rad * np.cos(ang)
+    co[move, 1] += rad * np.sin(ang)
+    from .solver import Sample
+    return Sample(np.ascontiguousarray(co), s.conn, s.cell_region, s.D, s.fixed, s.rhs), n0
+
+
+def plate_meshes(seed: int, sizes, max_tries: int = 50):
+    """One random plate geometry (``PlateGenerator``, seeded) meshed at each of ``sizes``:
+    ([(coors, conn) per size], ptags, ltags).  The geometry's corners keep their ids at every size, so
+    tag-based conditions mean the same on every mesh."""
+    from .plates import GeometryRejected, PlateGenerator
+    gen = PlateGenerator(random_seed=seed)
+    for _ in range(max_tries):
+        g = gen.normalize_geometry(gen.generate_geometry())
+        try:
+            meshes = []
+            for h in sizes:
+                ptags, ltags = gen.generate_mesh(g, h)
+                meshes.append(gen.mesh)
+            return meshes, ptags, ltags
+        except GeometryRejected:
+            continue
+    raise RuntimeError("no plate meshable at every size after %d tries (seed %d)" % (max_tries, seed))
+
+
+def plate_condition(ptags, ltags) -> Dict:
+    """A well-posed condition in the plate's tags: the first exterior edge clamped, a point load at the
+    exterior corner after it (FEAnalysis keyword arguments; the default material everywhere)."""
+    edge = next(iter(ltags[-1].values()))
+    return dict(constraints_edges_tags=[edge], force_vertex_tags_magnitudes=[(ptags[-1][2], (0.0, -1000.0))])

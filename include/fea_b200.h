@@ -374,6 +374,29 @@ int  fea_batch_get_level_csr(fea_batch* b, int32_t level, int32_t* indptr, int32
 /* z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as fea_batch_spmv) */
 int  fea_batch_mg_apply(fea_batch* b, const double* r, double* z);
 
+/* ---- multigrid-preconditioned solve of a mesh with coarser meshes of the same domain ------------
+ * The batch's only sample (P1 triangles) is the finest level of a hierarchy whose coarser levels are the samples
+ * of `coarse`, coarsest first (1..8 levels): meshes of the same domain, each with its own cell_region, D and
+ * fixed mask (rhs is not read). Before fea_batch_assemble.  Accepted on batches from fea_batch_create and from
+ * fea_batch_create_from_conditions.  Each vertex of level l is located in level l-1 on the device: the
+ * lowest-index triangle that contains it (edge-inclusive), or, if it lies outside every triangle by at most
+ * 1e-10 * the longest bounding-box side of level l-1, the nearest triangle with barycentric weights clamped to
+ * [0, 1] and renormalised.  P_l interpolates linearly from those triangles; Dirichlet vertices have neither
+ * rows nor columns.  Coarse operators are the coarse meshes' own stiffness matrices (rediscretised, not
+ * Galerkin); smoothers, the coarsest solve, the outer flexible CG and every output are those of
+ * fea_batch_set_refinement, and fea_batch_get_mg_levels / get_level_csr / mg_apply keep their meaning.
+ * FEA_BAD_ARG: more than one sample, quads, 0 or more than 8 coarse meshes, a level without fewer vertices than
+ * the next finer one, a null array.  FEA_BAD_STATE: after fea_batch_assemble, fea_batch_set_refinement or an
+ * earlier successful fea_batch_set_coarse_meshes.  FEA_MESH_ERROR: a vertex of level l farther than the
+ * tolerance from every triangle of level l-1 (the message names the level and the vertex), or a coarse
+ * connectivity index out of range.  If fea_batch_assemble then fails to build the coarse levels, the batch
+ * stays unassembled: a second fea_batch_assemble returns FEA_BAD_STATE. */
+int  fea_batch_set_coarse_meshes(fea_batch* b, const fea_batch_desc* coarse);
+/* P_l (level l-1 -> level l) as CSR over active DOFs, unscaled: rows = active DOFs of level l, columns = active DOFs
+ * of level l-1, same numbering rule as fea_batch_get_csr; level 1..levels; for either kind of hierarchy.  After
+ * fea_batch_assemble; any pointer may be NULL (indptr [rows+1] alone gives nnz = indptr[rows]). */
+int  fea_batch_get_level_transfer(fea_batch* b, int32_t level, int32_t* indptr, int32_t* indices, double* data);
+
 /* ---- scalar-field images of one mesh ----------------------------------------
  * The point-scalar renders of FEAnalysis.save_input_image / save_region_images (reference
  * fea_analysis.py:472-524: the constant field "1" and the 0/1 region flags of regions.vtk) and the
