@@ -912,6 +912,21 @@ int fea_batch_get_level_csr(fea_batch* hb, int32_t level, int32_t* indptr, int32
   return fea_batch_get_csr(lb, 0, indptr, indices, data);
 }
 
+int fea_batch_solve_load_cases(fea_batch* hb, int32_t n_cases, const double* rhs, double rtol, int32_t max_iter,
+                               double* u, double* ranges, int32_t* iters, double* relres, int32_t* status,
+                               fea_solve_stats* stats) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch has no multigrid hierarchy");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_solve_load_cases before fea_batch_assemble");
+  if (n_cases < 1 || n_cases > kMaxCases) return api_fail(ctx, FEA_BAD_ARG, "n_cases must be 1..8");
+  if (!rhs) return api_fail(ctx, FEA_BAD_ARG, "null rhs");
+  if (!(rtol >= 0.0) || max_iter < 1) return api_fail(ctx, FEA_BAD_ARG, "rtol must be >= 0 and max_iter >= 1");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  return mg_solve_load_cases(ctx, b, n_cases, rhs, rtol, max_iter, u, ranges, iters, relres, status, stats);
+}
+
 int fea_batch_mg_apply(fea_batch* hb, const double* r, double* z) {
   if (!hb || !r || !z) return FEA_BAD_ARG;
   fea_ctx* ctx = hb->owner;

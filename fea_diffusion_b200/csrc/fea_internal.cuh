@@ -188,8 +188,9 @@ struct MgLevel {
   double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};   // levels >= 1
   double lmax = 0.0;             // power-iteration estimate of the largest eigenvalue of Khat
   double inv_theta = 0.0, c1[2] = {0.0, 0.0}, c2[2] = {0.0, 0.0};   // Chebyshev coefficients
-  double ms = 0.0;               // V-cycle time spent on the level in the last solve
+  double ms = 0.0;               // V-cycle time spent on the level in the last solve (of either kind)
 };
+constexpr int kMaxCases = 8;     // load cases of one fea_batch_solve_load_cases call
 struct Mg {
   int levels = 0;
   bool nonnested = false;        // coarse levels are the caller's meshes (fea_batch_set_coarse_meshes)
@@ -198,8 +199,11 @@ struct Mg {
   double2 *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, finest row space (x = Batch::x)
   double *partA = nullptr, *partB = nullptr;          // per-CTA partial sums
   double* sc = nullptr;          // device scalars (kSc* slots, k_mg.cu)
-  double* h_sc = nullptr;        // pinned copy
+  double* h_sc = nullptr;        // pinned copy, room for kMaxCases cases
   std::vector<cudaEvent_t> ev;   // 4 per level + 2 around the solve
+  // coarsest batches of load-case solves: coarse[K] has K samples, each a copy of level 0 (built on first use)
+  fea_batch* coarse[kMaxCases + 1] = {};
+  int64_t case_rows = 0;         // block rows of one sample of those batches
 };
 
 }  // namespace fea
@@ -244,6 +248,9 @@ int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels);   // derive and valid
 int mg_assemble(fea_ctx* ctx, Batch& b);                     // coarse level batches, Galerkin operators, smoothers
 int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter);   // flexible CG preconditioned by V-cycles
 int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z);   // one V-cycle, active-DOF vectors
+// n_cases (1..kMaxCases) loads [n_cases][NV*2] solved together; host outputs as fea_batch_solve_load_cases
+int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int n_cases, const double* rhs, double rtol, int max_iter, double* u,
+                        double* ranges, int32_t* iters, double* relres, int32_t* status, fea_solve_stats* stats);
 void mg_release(Batch& b);
 // non-nested hierarchy (k_mg_nonnested.cu): coarse level batches from `coarse`, point location, transfers
 int mg_set_coarse_meshes(fea_ctx* ctx, Batch& b, const fea_batch_desc* coarse);
@@ -305,6 +312,9 @@ int pcg_cluster_rows_per_cta();                               // block rows a CT
 struct PcgPtrs;
 cudaError_t launch_pcg_cluster(Ctx& c, const PcgPtrs* dP, int n_systems, int cl, cudaStream_t st);
 cudaError_t launch_finalize(Batch& b);                        // u, ranges, max-iter status
+// the same three kernels on a solution x [NBR*2] and per-sample arrays other than the batch's own
+cudaError_t launch_finalize_to(Batch& b, const double* x, const int32_t* status, const double* rz_last, const double* rz0,
+                               double* u, double* ranges, double* relres);
 cudaError_t launch_plain_spmv(Batch& b, int32_t s, const double* d_x, double* d_y);
 cudaError_t launch_raster(Batch& b, double value_scale);
 cudaError_t launch_raster_flags(Batch& b, int64_t n_img, const int64_t* d_field_off, const int64_t* d_flag_off,

@@ -19,9 +19,13 @@
 // Dot products: one partial per CTA, summed by one block in a fixed order (bitwise reproducible).
 // A non-nested hierarchy (fea_batch_set_coarse_meshes, k_mg_nonnested.cu; DESIGN.md section 3.10) runs the same
 // V-cycle and outer CG with rediscretised coarse operators and the k_mgn_* transfers (up to 3 weighted parents).
+// Both solve K = 1..8 load cases at once (fea_batch_solve_load_cases; DESIGN.md section 3.11): the V-cycle and
+// outer-CG kernels are templates on the number of columns they carry (a group of at most 4 cases), and
+// fea_batch_solve is the case K = 1.
 #include <cmath>
 #include <cstdio>
 #include <memory>
+#include <type_traits>
 #include <vector>
 
 #include "fea_internal.cuh"
@@ -48,41 +52,68 @@ struct MgOp {   // block-SELL matrix of one level (identity diagonal blocks not 
 };
 MgOp op_of(const Batch& b) { return MgOp{b.slice_len, b.slice_ptr, (const d4*)b.val, b.col}; }
 
-// (Khat v)[row]; row's lane in its slice = threadIdx.x & 31
-__device__ __forceinline__ double2 khat_row(const MgOp& A, int64_t row, const double2* __restrict__ v) {
+// A kernel carries K columns (load cases; a group of at most 4, see each_group), interleaved per block row:
+// column k of row r is v[r * K + k], so one gathered neighbour brings all K columns.  Every kernel below does,
+// per column, exactly the arithmetic of
+// K = 1 in the same order (the same fma chains, the same per-CTA partials): a column's bits do not depend on
+// K or on the other columns.
+// (Khat v)[row] of the K columns; row's lane in its slice = threadIdx.x & 31
+template <int K>
+__device__ __forceinline__ void khat_row(const MgOp& A, int64_t row, const double2* __restrict__ v, double2 (&out)[K]) {
   const int lane = threadIdx.x & 31;
   const int64_t slice = row >> 5;
   const int L = A.slice_len[slice];
   const int64_t base = A.slice_ptr[slice];
   const d4* __restrict__ vt = A.val + base + lane;
   const int32_t* __restrict__ cp = A.col + base + lane;
-  const double2 own = v[row];
-  double a0 = own.x, a1 = own.y;
+  double a0[K], a1[K];
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const double2 own = v[row * K + q];
+    a0[q] = own.x;
+    a1[q] = own.y;
+  }
   for (int j = 0; j < L; ++j) {
     const int c = ld_stream_i32(cp + j * 32);
     const d4 k = ld_stream_d4(vt + j * 32);
-    const double2 xj = __ldg(v + c);
-    a0 = fma(k.x, xj.x, a0);
-    a0 = fma(k.y, xj.y, a0);
-    a1 = fma(k.z, xj.x, a1);
-    a1 = fma(k.w, xj.y, a1);
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+      const double2 xj = __ldg(v + (int64_t)c * K + q);
+      a0[q] = fma(k.x, xj.x, a0[q]);
+      a0[q] = fma(k.y, xj.y, a0[q]);
+      a1[q] = fma(k.z, xj.x, a1[q]);
+      a1[q] = fma(k.w, xj.y, a1[q]);
+    }
   }
-  return make_double2(a0, a1);
+#pragma unroll
+  for (int q = 0; q < K; ++q) out[q] = make_double2(a0[q], a1[q]);
 }
 
-// deterministic block sum, result written by thread 0 to part[blockIdx.x]
-__device__ __forceinline__ void block_partial(double v, double* __restrict__ part) {
-  __shared__ double sm[kT / 32];
-  v = warp_sum(v);
-  if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = v;
+// deterministic block sums of K columns, written by thread 0 to part[q * gridDim.x + blockIdx.x]
+template <int K>
+__device__ __forceinline__ void block_partial(const double (&v)[K], double* __restrict__ part) {
+  __shared__ double sm[K][kT / 32];
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const double s = warp_sum(v[q]);
+    if ((threadIdx.x & 31) == 0) sm[q][threadIdx.x >> 5] = s;
+  }
   __syncthreads();
   if (threadIdx.x == 0) {
-    double t = 0.0;
 #pragma unroll
-    for (int w = 0; w < kT / 32; ++w) t += sm[w];
-    part[blockIdx.x] = t;
+    for (int q = 0; q < K; ++q) {
+      double t = 0.0;
+#pragma unroll
+      for (int w = 0; w < kT / 32; ++w) t += sm[q][w];
+      part[(int64_t)q * gridDim.x + blockIdx.x] = t;
+    }
   }
 }
+__device__ __forceinline__ void block_partial(double v, double* __restrict__ part) {
+  const double a[1] = {v};
+  block_partial<1>(a, part);
+}
+__device__ __forceinline__ bool on(unsigned mask, int q) { return (mask >> q) & 1u; }
 
 __device__ __forceinline__ double dot2(double2 a, double2 b) { return fma(a.x, b.x, a.y * b.y); }
 
@@ -244,11 +275,21 @@ __global__ void k_mg_galerkin(int64_t nc, const int32_t* __restrict__ conn_f, co
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// reductions: one block sums the partials in a fixed order, then updates the scalars
+// reductions: one block per case sums that case's partials in a fixed order, then updates its scalars (the
+// kScCount slots from sc + case * kScCount; out, if given, advances by the same stride).  Cases outside
+// `mask` are left alone; bit q of `first` is case q's first-iteration flag.
 enum { kRedStore = 0, kRedDots = 1, kRedPQ = 2 };
 __global__ void __launch_bounds__(1024) k_mg_reduce(const double* __restrict__ pa, const double* __restrict__ pb, int n,
-                                                    double* __restrict__ sc, int mode, double* __restrict__ out, int first) {
+                                                    double* __restrict__ sc, int mode, double* __restrict__ out,
+                                                    unsigned first_bits, unsigned mask) {
   __shared__ double sa[32], sb[32];
+  const int q = blockIdx.x;
+  if (!on(mask, q)) return;
+  pa += (int64_t)q * n;
+  if (pb) pb += (int64_t)q * n;
+  sc += q * kScCount;
+  out += q * kScCount;
+  const int first = on(first_bits, q);
   double a = 0.0, b = 0.0;
   for (int i = threadIdx.x; i < n; i += 1024) {
     a += pa[i];
@@ -297,9 +338,10 @@ __global__ void __launch_bounds__(kT) k_mg_lz_init(const int32_t* __restrict__ v
 __global__ void __launch_bounds__(kT) k_mg_lz_apply(MgOp A, const double2* __restrict__ v, double2* __restrict__ w,
                                                     double* __restrict__ part) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 t = khat_row(A, row, v);
-  w[row] = t;
-  block_partial(dot2(v[row], t), part);
+  double2 t[1];
+  khat_row<1>(A, row, v, t);
+  w[row] = t[0];
+  block_partial(dot2(v[row], t[0]), part);
 }
 __global__ void __launch_bounds__(kT) k_mg_lz_orth(const double2* __restrict__ v, const double2* __restrict__ vp,
                                                    double2* __restrict__ w, const double* __restrict__ alpha,
@@ -329,49 +371,73 @@ __global__ void __launch_bounds__(kT) k_mg_lz_next(double2* __restrict__ v, doub
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// V-cycle kernels of one level (state: x, r, d where d is not yet added to x)
+// V-cycle kernels of one level, K columns (state: x, r, d where d is not yet added to x)
 // Chebyshev step: x += d_in; r -= Khat d_in; d_out = c1 d_in + c2 r.  The last step of the pre-smoother
 // (d_out == nullptr) leaves the unscaled residual S^-T r in ru for the restriction instead.
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_cheb_step(MgOp A, const double2* __restrict__ din, double2* __restrict__ dout,
                                                      double2* __restrict__ x, double2* __restrict__ r, double c1, double c2,
                                                      const double* __restrict__ ds, const double* __restrict__ scp,
                                                      double2* __restrict__ ru) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 ad = khat_row(A, row, din);
-  const double2 d = din[row];
-  double2 xv = x[row], rv = r[row];
-  xv.x += d.x;
-  xv.y += d.y;
-  rv.x -= ad.x;
-  rv.y -= ad.y;
-  x[row] = xv;
-  r[row] = rv;
-  if (dout) dout[row] = make_double2(fma(c1, d.x, c2 * rv.x), fma(c1, d.y, c2 * rv.y));
-  else ru[row] = ds[2 * row] > 0.0 ? solve_St(ds, scp, row, rv) : make_double2(0.0, 0.0);   // padding rows: 0
+  double2 ad[K];
+  khat_row<K>(A, row, din, ad);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 d = din[i];
+    double2 xv = x[i], rv = r[i];
+    xv.x += d.x;
+    xv.y += d.y;
+    rv.x -= ad[q].x;
+    rv.y -= ad[q].y;
+    x[i] = xv;
+    r[i] = rv;
+    if (dout) dout[i] = make_double2(fma(c1, d.x, c2 * rv.x), fma(c1, d.y, c2 * rv.y));
+    else ru[i] = ds[2 * row] > 0.0 ? solve_St(ds, scp, row, rv) : make_double2(0.0, 0.0);   // padding rows: 0
+  }
 }
 // after the coarse correction: r = b - Khat x, d = r / theta
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_resid(MgOp A, const double2* __restrict__ x, const double2* __restrict__ b,
                                                  double2* __restrict__ r, double2* __restrict__ d, double inv_theta) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 ax = khat_row(A, row, x);
-  const double2 bv = b[row];
-  const double2 rv = make_double2(bv.x - ax.x, bv.y - ax.y);
-  r[row] = rv;
-  d[row] = make_double2(rv.x * inv_theta, rv.y * inv_theta);
+  double2 ax[K];
+  khat_row<K>(A, row, x, ax);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 bv = b[i];
+    const double2 rv = make_double2(bv.x - ax[q].x, bv.y - ax[q].y);
+    r[i] = rv;
+    d[i] = make_double2(rv.x * inv_theta, rv.y * inv_theta);
+  }
 }
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_add(double2* __restrict__ x, const double2* __restrict__ d) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 a = x[row], b = d[row];
-  x[row] = make_double2(a.x + b.x, a.y + b.y);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 a = x[i], b = d[i];
+    x[i] = make_double2(a.x + b.x, a.y + b.y);
+  }
 }
-// entry of the finest level: r = b, d = b / theta, x = 0
+// entry of the finest level: r = b, d = b / theta, x = 0; a column outside `mask` (a finished case) enters
+// with b = 0, so its coarse system is zero and it costs the coarse solve nothing
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_top_init(const double2* __restrict__ b, double2* __restrict__ x,
-                                                    double2* __restrict__ r, double2* __restrict__ d, double inv_theta) {
+                                                    double2* __restrict__ r, double2* __restrict__ d, double inv_theta,
+                                                    unsigned mask) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 bv = b[row];
-  r[row] = bv;
-  d[row] = make_double2(bv.x * inv_theta, bv.y * inv_theta);
-  x[row] = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 bv = on(mask, q) ? b[i] : make_double2(0.0, 0.0);
+    r[i] = bv;
+    d[i] = make_double2(bv.x * inv_theta, bv.y * inv_theta);
+    x[i] = make_double2(0.0, 0.0);
+  }
 }
 
 struct Side {   // one level's maps and scaling
@@ -382,103 +448,157 @@ struct Side {   // one level's maps and scaling
 };
 Side side_of(const Batch& b) { return Side{b.vertex_of_row, b.row_of_vertex, b.dscale, b.scoup}; }
 
+// Where column k of a coarse-level vector lives.  A smoothed level interleaves: (row, k) at row * K + k.
+// The coarsest level is a batch with one sample per case, each a copy of level 0: case k's row r is row
+// r + k * rows_per_sample of that batch, and its vertex v is vertex v + k * n_vertices (the restriction writes
+// the batch's rhs by vertex).
+struct ColMap {
+  int64_t row_stride, col_stride;
+};
+
 // restriction, one thread per coarse row: r_c = P^T S_f^-T r^_f at the coarse vertex (ru = S_f^-T r^_f).  Into a smoothed level:
 // b = r = S_c^T r_c, d = b / theta, x = 0; into the coarsest level: its unscaled load vector rhs[vertex].
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_restrict(Side F, Side Cs, const double2* __restrict__ ru,
                                                     const int32_t* __restrict__ child_ptr, const int32_t* __restrict__ child,
                                                     double2* __restrict__ bc, double2* __restrict__ xc, double2* __restrict__ rc,
-                                                    double2* __restrict__ dc, double inv_theta, double2* __restrict__ rhs0) {
+                                                    double2* __restrict__ dc, double inv_theta, double2* __restrict__ rhs0,
+                                                    int64_t rhs0_stride) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
   const int j = Cs.vertex_of_row[row];
-  double2 acc = make_double2(0.0, 0.0);
+  double2 acc[K];
+#pragma unroll
+  for (int q = 0; q < K; ++q) acc[q] = make_double2(0.0, 0.0);
   if (j >= 0) {
     const int fr = F.row_of_vertex[j];
-    if (fr >= 0) acc = ru[fr];
+    if (fr >= 0) {
+#pragma unroll
+      for (int q = 0; q < K; ++q) acc[q] = ru[(int64_t)fr * K + q];
+    }
     for (int i = child_ptr[j]; i < child_ptr[j + 1]; ++i) {
       const int m = child[i];
       const int mr = F.row_of_vertex[m];
       if (mr < 0) continue;
-      const double2 t = ru[mr];
-      acc.x = fma(0.5, t.x, acc.x);
-      acc.y = fma(0.5, t.y, acc.y);
+#pragma unroll
+      for (int q = 0; q < K; ++q) {
+        const double2 t = ru[(int64_t)mr * K + q];
+        acc[q].x = fma(0.5, t.x, acc[q].x);
+        acc[q].y = fma(0.5, t.y, acc[q].y);
+      }
     }
   }
   if (rhs0) {
-    if (j >= 0) rhs0[j] = acc;
+    if (j >= 0) {
+#pragma unroll
+      for (int q = 0; q < K; ++q) rhs0[j + q * rhs0_stride] = acc[q];
+    }
     return;
   }
-  const double2 h = j >= 0 ? mul_St(Cs.dscale, Cs.scoup, row, acc) : make_double2(0.0, 0.0);
-  bc[row] = h;
-  rc[row] = h;
-  dc[row] = make_double2(h.x * inv_theta, h.y * inv_theta);
-  xc[row] = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 h = j >= 0 ? mul_St(Cs.dscale, Cs.scoup, row, acc[q]) : make_double2(0.0, 0.0);
+    bc[i] = h;
+    rc[i] = h;
+    dc[i] = make_double2(h.x * inv_theta, h.y * inv_theta);
+    xc[i] = make_double2(0.0, 0.0);
+  }
 }
 
-// prolongation-add, one thread per fine row: x^_f += S_f^-1 P S_c x^_c
+// prolongation-add, one thread per fine row: x^_f += S_f^-1 P S_c x^_c (Cs: the coarse level's maps and scaling;
+// column k of its row r at xc[r * cm.row_stride + k * cm.col_stride])
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_prolong(Side F, Side Cs, const int2* __restrict__ par, const double2* __restrict__ xc,
-                                                   double2* __restrict__ xf) {
+                                                   ColMap cm, double2* __restrict__ xf) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
   const int f = F.vertex_of_row[row];
   if (f < 0) return;
   const int2 pr = par[f];
-  double2 e = make_double2(0.0, 0.0);
+  double2 e[K];
+#pragma unroll
+  for (int q = 0; q < K; ++q) e[q] = make_double2(0.0, 0.0);
   const int r0 = Cs.row_of_vertex[pr.x];
   const double w = pr.y < 0 ? 1.0 : 0.5;
   if (r0 >= 0) {
-    const double2 t = mul_S(Cs.dscale, Cs.scoup, r0, xc[r0]);
-    e = make_double2(w * t.x, w * t.y);
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+      const double2 t = mul_S(Cs.dscale, Cs.scoup, r0, xc[r0 * cm.row_stride + q * cm.col_stride]);
+      e[q] = make_double2(w * t.x, w * t.y);
+    }
   }
   if (pr.y >= 0) {
     const int r1 = Cs.row_of_vertex[pr.y];
     if (r1 >= 0) {
-      const double2 t = mul_S(Cs.dscale, Cs.scoup, r1, xc[r1]);
-      e.x = fma(0.5, t.x, e.x);
-      e.y = fma(0.5, t.y, e.y);
+#pragma unroll
+      for (int q = 0; q < K; ++q) {
+        const double2 t = mul_S(Cs.dscale, Cs.scoup, r1, xc[r1 * cm.row_stride + q * cm.col_stride]);
+        e[q].x = fma(0.5, t.x, e[q].x);
+        e[q].y = fma(0.5, t.y, e[q].y);
+      }
     }
   }
-  const double2 c = solve_S(F.dscale, F.scoup, row, e);
-  double2 xv = xf[row];
-  xv.x += c.x;
-  xv.y += c.y;
-  xf[row] = xv;
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const double2 c = solve_S(F.dscale, F.scoup, row, e[q]);
+    double2 xv = xf[row * K + q];
+    xv.x += c.x;
+    xv.y += c.y;
+    xf[row * K + q] = xv;
+  }
 }
 
 // non-nested hierarchies (k_mg_nonnested.cu): the same two transfers with up to 3 weighted parents per vertex.
 // Restriction gathers over a coarse vertex's (fine vertex, weight) list, ascending in the fine vertex.
+template <int K>
 __global__ void __launch_bounds__(kT) k_mgn_restrict(Side F, Side Cs, const double2* __restrict__ ru,
                                                      const int32_t* __restrict__ child_ptr, const int32_t* __restrict__ child,
                                                      const double* __restrict__ child_w, double2* __restrict__ bc,
                                                      double2* __restrict__ xc, double2* __restrict__ rc, double2* __restrict__ dc,
-                                                     double inv_theta, double2* __restrict__ rhs0) {
+                                                     double inv_theta, double2* __restrict__ rhs0, int64_t rhs0_stride) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
   const int j = Cs.vertex_of_row[row];
-  double2 acc = make_double2(0.0, 0.0);
+  double2 acc[K];
+#pragma unroll
+  for (int q = 0; q < K; ++q) acc[q] = make_double2(0.0, 0.0);
   if (j >= 0) {
     for (int i = child_ptr[j]; i < child_ptr[j + 1]; ++i) {
       const int fr = F.row_of_vertex[child[i]];
       if (fr < 0) continue;
       const double w = child_w[i];
-      const double2 t = ru[fr];
-      acc.x = fma(w, t.x, acc.x);
-      acc.y = fma(w, t.y, acc.y);
+#pragma unroll
+      for (int q = 0; q < K; ++q) {
+        const double2 t = ru[(int64_t)fr * K + q];
+        acc[q].x = fma(w, t.x, acc[q].x);
+        acc[q].y = fma(w, t.y, acc[q].y);
+      }
     }
   }
   if (rhs0) {
-    if (j >= 0) rhs0[j] = acc;
+    if (j >= 0) {
+#pragma unroll
+      for (int q = 0; q < K; ++q) rhs0[j + q * rhs0_stride] = acc[q];
+    }
     return;
   }
-  const double2 h = j >= 0 ? mul_St(Cs.dscale, Cs.scoup, row, acc) : make_double2(0.0, 0.0);
-  bc[row] = h;
-  rc[row] = h;
-  dc[row] = make_double2(h.x * inv_theta, h.y * inv_theta);
-  xc[row] = make_double2(0.0, 0.0);
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const int64_t i = row * K + q;
+    const double2 h = j >= 0 ? mul_St(Cs.dscale, Cs.scoup, row, acc[q]) : make_double2(0.0, 0.0);
+    bc[i] = h;
+    rc[i] = h;
+    dc[i] = make_double2(h.x * inv_theta, h.y * inv_theta);
+    xc[i] = make_double2(0.0, 0.0);
+  }
 }
+template <int K>
 __global__ void __launch_bounds__(kT) k_mgn_prolong(Side F, Side Cs, const int32_t* __restrict__ par3, const double* __restrict__ w3,
-                                                    const double2* __restrict__ xc, double2* __restrict__ xf) {
+                                                    const double2* __restrict__ xc, ColMap cm, double2* __restrict__ xf) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
   const int f = F.vertex_of_row[row];
   if (f < 0) return;
-  double2 e = make_double2(0.0, 0.0);
+  double2 e[K];
+#pragma unroll
+  for (int q = 0; q < K; ++q) e[q] = make_double2(0.0, 0.0);
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
     const int p = par3[3 * (int64_t)f + k];
@@ -486,88 +606,153 @@ __global__ void __launch_bounds__(kT) k_mgn_prolong(Side F, Side Cs, const int32
     const int r = Cs.row_of_vertex[p];
     if (r < 0) continue;   // a Dirichlet vertex of the coarse level: no column
     const double w = w3[3 * (int64_t)f + k];
-    const double2 t = mul_S(Cs.dscale, Cs.scoup, r, xc[r]);
-    e.x = fma(w, t.x, e.x);
-    e.y = fma(w, t.y, e.y);
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+      const double2 t = mul_S(Cs.dscale, Cs.scoup, r, xc[r * cm.row_stride + q * cm.col_stride]);
+      e[q].x = fma(w, t.x, e[q].x);
+      e[q].y = fma(w, t.y, e[q].y);
+    }
   }
-  const double2 c = solve_S(F.dscale, F.scoup, row, e);
-  double2 xv = xf[row];
-  xv.x += c.x;
-  xv.y += c.y;
-  xf[row] = xv;
+#pragma unroll
+  for (int q = 0; q < K; ++q) {
+    const double2 c = solve_S(F.dscale, F.scoup, row, e[q]);
+    double2 xv = xf[row * K + q];
+    xv.x += c.x;
+    xv.y += c.y;
+    xf[row * K + q] = xv;
+  }
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// outer flexible CG on the finest level
-// r = S^T b (true = 0) or S^T b - Khat x (true = 1); true = 0 also clears x, p, q.  Partials of r.r.
-__global__ void __launch_bounds__(kT) k_mg_fcg_residual(MgOp A, Side F, const double* __restrict__ rhs, double2* __restrict__ x,
-                                                        double2* __restrict__ r, double2* __restrict__ p, double2* __restrict__ q,
-                                                        int true_res, double* __restrict__ part) {
+// outer flexible CG on the finest level, K cases; x, r, p and q change only in the columns of `mask` (the cases
+// still iterating), so a finished case keeps its last iterate and its p and q
+// r = S^T b (mode 0) or S^T b - Khat x (modes 1, 2); mode 0 also clears x, modes 0 and 2 (a restart) p and q.
+// b of case k: the full-DOF load rhs + k * rhs_stride.  Partials of r.r.
+template <int K>
+__global__ void __launch_bounds__(kT) k_mg_fcg_residual(MgOp A, Side F, const double* __restrict__ rhs, int64_t rhs_stride,
+                                                        double2* __restrict__ x, double2* __restrict__ r, double2* __restrict__ p,
+                                                        double2* __restrict__ q, int mode, unsigned mask, double* __restrict__ part) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
   const int v = F.vertex_of_row[row];
-  double2 bv = make_double2(0.0, 0.0);
-  if (v >= 0) bv = mul_St(F.dscale, F.scoup, row, make_double2(rhs[2 * (int64_t)v], rhs[2 * (int64_t)v + 1]));
-  if (true_res) {
-    const double2 ax = khat_row(A, row, x);
-    bv.x -= ax.x;
-    bv.y -= ax.y;
-  } else {
-    x[row] = make_double2(0.0, 0.0);
+  double2 bv[K];
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    bv[c] = make_double2(0.0, 0.0);
+    const double* rc = rhs + c * rhs_stride;
+    if (v >= 0) bv[c] = mul_St(F.dscale, F.scoup, row, make_double2(rc[2 * (int64_t)v], rc[2 * (int64_t)v + 1]));
   }
-  if (!true_res || true_res == 2) {   // (re)start: p = q = 0
-    p[row] = make_double2(0.0, 0.0);
-    q[row] = make_double2(0.0, 0.0);
+  if (mode) {
+    double2 ax[K];
+    khat_row<K>(A, row, x, ax);
+#pragma unroll
+    for (int c = 0; c < K; ++c) {
+      bv[c].x -= ax[c].x;
+      bv[c].y -= ax[c].y;
+    }
   }
-  r[row] = bv;
-  block_partial(dot2(bv, bv), part);
+  double rr[K];
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    const int64_t i = row * K + c;
+    if (on(mask, c)) {
+      if (!mode) x[i] = make_double2(0.0, 0.0);
+      if (mode != 1) {   // (re)start: p = q = 0
+        p[i] = make_double2(0.0, 0.0);
+        q[i] = make_double2(0.0, 0.0);
+      }
+      r[i] = bv[c];
+    }
+    rr[c] = dot2(bv[c], bv[c]);
+  }
+  block_partial<K>(rr, part);
 }
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_fcg_dots(const double2* __restrict__ z, const double2* __restrict__ r,
                                                     const double2* __restrict__ q, double* __restrict__ pa, double* __restrict__ pb) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 zv = z[row];
-  block_partial(dot2(zv, r[row]), pa);
+  double zr[K], zq[K];
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    const int64_t i = row * K + c;
+    const double2 zv = z[i];
+    zr[c] = dot2(zv, r[i]);
+    zq[c] = dot2(zv, q[i]);
+  }
+  block_partial<K>(zr, pa);
   __syncthreads();
-  block_partial(dot2(zv, q[row]), pb);
+  block_partial<K>(zq, pb);
 }
-__global__ void __launch_bounds__(kT) k_mg_fcg_dir(const double2* __restrict__ z, double2* __restrict__ p, const double* __restrict__ sc) {
+template <int K>
+__global__ void __launch_bounds__(kT) k_mg_fcg_dir(const double2* __restrict__ z, double2* __restrict__ p, const double* __restrict__ sc,
+                                                   unsigned mask) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double beta = sc[kScBeta];
-  const double2 zv = z[row], pv = p[row];
-  p[row] = make_double2(fma(beta, pv.x, zv.x), fma(beta, pv.y, zv.y));
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    if (!on(mask, c)) continue;
+    const int64_t i = row * K + c;
+    const double beta = sc[c * kScCount + kScBeta];
+    const double2 zv = z[i], pv = p[i];
+    p[i] = make_double2(fma(beta, pv.x, zv.x), fma(beta, pv.y, zv.y));
+  }
 }
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_fcg_spmv(MgOp A, const double2* __restrict__ p, double2* __restrict__ q,
-                                                    double* __restrict__ part) {
+                                                    unsigned mask, double* __restrict__ part) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double2 qv = khat_row(A, row, p);
-  q[row] = qv;
-  block_partial(dot2(p[row], qv), part);
+  double2 qv[K];
+  khat_row<K>(A, row, p, qv);
+  double pq[K];
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    const int64_t i = row * K + c;
+    if (on(mask, c)) q[i] = qv[c];
+    pq[c] = dot2(p[i], qv[c]);
+  }
+  block_partial<K>(pq, part);
 }
+template <int K>
 __global__ void __launch_bounds__(kT) k_mg_fcg_update(double2* __restrict__ x, double2* __restrict__ r, const double2* __restrict__ p,
-                                                      const double2* __restrict__ q, const double* __restrict__ sc,
+                                                      const double2* __restrict__ q, const double* __restrict__ sc, unsigned mask,
                                                       double* __restrict__ part) {
   const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
-  const double alpha = sc[kScAlpha], pq = sc[kScPQ];
-  double2 rv = r[row];
-  // p.q <= 0 or a non-finite step: breakdown (the host stops), x and r keep the last sound iterate
-  if (pq > 0.0 && isfinite(pq) && isfinite(alpha)) {
-    const double2 pv = p[row], qv = q[row];
-    double2 xv = x[row];
-    xv.x = fma(alpha, pv.x, xv.x);
-    xv.y = fma(alpha, pv.y, xv.y);
-    rv.x = fma(-alpha, qv.x, rv.x);
-    rv.y = fma(-alpha, qv.y, rv.y);
-    x[row] = xv;
-    r[row] = rv;
+  double rr[K];
+#pragma unroll
+  for (int c = 0; c < K; ++c) {
+    const int64_t i = row * K + c;
+    const double alpha = sc[c * kScCount + kScAlpha], pq = sc[c * kScCount + kScPQ];
+    double2 rv = r[i];
+    // p.q <= 0 or a non-finite step: breakdown (the host stops the case), x and r keep the last sound iterate
+    if (on(mask, c) && pq > 0.0 && isfinite(pq) && isfinite(alpha)) {
+      const double2 pv = p[i], qv = q[i];
+      double2 xv = x[i];
+      xv.x = fma(alpha, pv.x, xv.x);
+      xv.y = fma(alpha, pv.y, xv.y);
+      rv.x = fma(-alpha, qv.x, rv.x);
+      rv.y = fma(-alpha, qv.y, rv.y);
+      x[i] = xv;
+      r[i] = rv;
+    }
+    rr[c] = dot2(rv, rv);
   }
-  block_partial(dot2(rv, rv), part);
+  block_partial<K>(rr, part);
 }
-// what launch_finalize and fea_batch_download read
-__global__ void k_mg_finish(SysScalars s, double* __restrict__ rz_last, const double* __restrict__ sc, int status, int iters) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  s.status[0] = status;
-  s.iters[0] = iters;
-  s.rz0[0] = sc[kScRZ0];
-  rz_last[0] = sc[kScTrue];
+// what launch_finalize and fea_batch_download read, per case
+struct CaseInts {
+  int32_t v[kMaxCases];
+};
+__global__ void k_mg_finish(int n, int32_t* __restrict__ status, int32_t* __restrict__ iters, double* __restrict__ rz0,
+                            double* __restrict__ rz_last, const double* __restrict__ sc, CaseInts st, CaseInts it) {
+  const int c = threadIdx.x;
+  if (blockIdx.x != 0 || c >= n) return;
+  status[c] = st.v[c];
+  iters[c] = it.v[c];
+  rz0[c] = sc[c * kScCount + kScRZ0];
+  rz_last[c] = sc[c * kScCount + kScTrue];
+}
+// column c of a K-column vector, contiguous (the layout launch_finalize_to reads)
+__global__ void __launch_bounds__(kT) k_mg_column(const double2* __restrict__ v, int K, int c, double2* __restrict__ out) {
+  const int64_t row = (int64_t)blockIdx.x * kT + threadIdx.x;
+  out[row] = v[row * K + c];
 }
 
 // active-DOF vector (unscaled) <-> scaled rows of the finest level
@@ -595,9 +780,10 @@ __global__ void __launch_bounds__(kT) k_mg_store(Side F, const int32_t* __restri
 
 unsigned grid_rows(const Batch& b) { return (unsigned)(b.NBR / kT); }
 
-cudaError_t reduce(Batch& fine, const double* pa, const double* pb, int n, int mode, int slot = 0, int first = 0,
-                   double* out = nullptr) {
-  k_mg_reduce<<<1, 1024, 0, fine.ctx->stream>>>(pa, pb, n, fine.mg->sc, mode, out ? out : fine.mg->sc + slot, first);
+// the partials of n CTAs per case into the scalars sc of the cases in `mask` (slot: kRedStore's destination)
+cudaError_t reduce(const Batch& fine, double* sc, int n_cases, const double* pa, const double* pb, int n, int mode,
+                   int slot = 0, unsigned first = 0, unsigned mask = 1, double* out = nullptr) {
+  k_mg_reduce<<<n_cases, 1024, 0, fine.ctx->stream>>>(pa, pb, n, sc, mode, out ? out : sc + slot, first, mask);
   return cudaGetLastError();
 }
 
@@ -636,13 +822,13 @@ cudaError_t estimate_lmax(Batch& fine, MgLevel& L) {
   double2 *v = mg.p, *vp = mg.q, *w = mg.r;
   double* lz = mg.sc + kScCount;   // [2 kLanczos]: alpha_k, beta_k^2
   k_mg_lz_init<<<g, kT, 0, st>>>(b.vertex_of_row, w, mg.partA);
-  cudaError_t e = reduce(fine, mg.partA, nullptr, (int)g, kRedStore, kScNrm);
+  cudaError_t e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, kScNrm);
   if (e == cudaSuccess) k_mg_lz_next<<<g, kT, 0, st>>>(v, vp, w, mg.sc + kScNrm);
   for (int k = 0; k < kLanczos && e == cudaSuccess; ++k) {
     k_mg_lz_apply<<<g, kT, 0, st>>>(op_of(b), v, w, mg.partA);
-    e = reduce(fine, mg.partA, nullptr, (int)g, kRedStore, 0, 0, lz + 2 * k);
+    e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k);
     k_mg_lz_orth<<<g, kT, 0, st>>>(v, vp, w, lz + 2 * k, k ? lz + 2 * k - 1 : nullptr, mg.partA);
-    if (e == cudaSuccess) e = reduce(fine, mg.partA, nullptr, (int)g, kRedStore, 0, 0, lz + 2 * k + 1);
+    if (e == cudaSuccess) e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k + 1);
     k_mg_lz_next<<<g, kT, 0, st>>>(v, vp, w, lz + 2 * k + 1);
   }
   std::vector<double> h(2 * kLanczos, 0.0);
@@ -670,58 +856,141 @@ cudaError_t estimate_lmax(Batch& fine, MgLevel& L) {
   return e;
 }
 
+// Column groups.  The kernels run on at most kGroup columns at once: K <= kGroup cases are one group, more are
+// split into two groups of ceil(K/2) and floor(K/2).  A K-column vector over n block rows holds group (c0, G) at
+// v + c0 * n, interleaved G columns per row.  Measured on a B200 (plate at h = 0.000625, 18 V-cycles): a
+// single 8-column group ran the finest level 7.8x slower than one column, 4 columns 2.45x (DESIGN.md section
+// 3.11).  A group's columns do the K = 1 arithmetic, so the split changes no bit.
+constexpr int kGroup = 4;
+constexpr int groups_of(int K) { return K > kGroup ? 2 : 1; }
+template <int K, class F>
+void each_group(F&& f) {
+  constexpr int G0 = K <= kGroup ? K : (K + 1) / 2;
+  f(std::integral_constant<int, G0>{}, 0);
+  if constexpr (K > G0) f(std::integral_constant<int, K - G0>{}, G0);
+}
+template <class T>
+T* at(T* v, int64_t n, int c0) { return v ? v + c0 * n : v; }
+
+// The vectors of one solve of K cases.  fea_batch_solve and fea_batch_mg_apply (K = 1) use the hierarchy's own
+// (mg.r/p/q/sc, MgLevel x/bv/r/d, the batch's x) and level 0's batch as the coarsest; a load-case call takes
+// them from a Scratch and, for K > 1, solves the coarsest systems in a batch of K copies of level 0.
+struct Vecs {
+  double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};
+};
+struct Work {
+  std::vector<Vecs> v;                    // [levels + 1]: V-cycle state of levels >= 1
+  double2 *x = nullptr, *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, K columns in groups (at)
+  double *partA = nullptr, *partB = nullptr;                        // [K][CTAs]
+  double* sc = nullptr;                   // [K][kScCount]
+  const double* rhs = nullptr;            // full-DOF loads, case k at rhs + k * rhs_stride
+  int64_t rhs_stride = 0;
+  Batch* coarse = nullptr;                // coarsest batch: its sample k solves case k
+  ColMap coarse_map{1, 0};                // case k's rows in coarse->x
+  int64_t coarse_nv = 0;                  // vertices per sample of the coarsest batch
+};
+
+Work own_work(Batch& b) {
+  Mg& mg = *b.mg;
+  Work w;
+  w.v.resize(mg.levels + 1);
+  for (int l = 1; l <= mg.levels; ++l) {
+    const MgLevel& L = mg.lev[l];
+    w.v[l].x = L.x;
+    w.v[l].bv = L.bv;
+    w.v[l].r = L.r;
+    w.v[l].d[0] = L.d[0];
+    w.v[l].d[1] = L.d[1];
+  }
+  w.x = (double2*)b.x;
+  w.r = mg.r;
+  w.p = mg.p;
+  w.q = mg.q;
+  w.partA = mg.partA;
+  w.partB = mg.partB;
+  w.sc = mg.sc;
+  w.rhs = b.rhs;
+  w.coarse = mg.lev[0].b;
+  w.coarse_nv = mg.lev[0].b->NV;
+  return w;
+}
+
 // one V-cycle from level l down; level l's b, r, d[0], x are set up by the caller (restriction / top init)
-cudaError_t vcycle(fea_ctx* ctx, Batch& fine, int l) {
+template <int K>
+cudaError_t vcycle(fea_ctx* ctx, Batch& fine, Work& w, int l) {
   Mg& mg = *fine.mg;
   Ctx& c = ctx->c;
   cudaStream_t st = c.stream;
   MgLevel& L = mg.lev[l];
   cudaEvent_t* ev = mg.ev.data() + 4 * l;
   cudaError_t e;
-  if (l == 0) {   // coarsest: block-Jacobi CG of the level-0 batch on the restricted residual
+  if (l == 0) {   // coarsest: block-Jacobi CG of the coarsest batch on the restricted residuals
     if ((e = cudaEventRecord(ev[0], st)) != cudaSuccess) return e;
-    if ((e = run_pcg(*L.b, kCoarseRtol, kCoarseMaxIter)) != cudaSuccess) return e;
+    if ((e = run_pcg(*w.coarse, kCoarseRtol, kCoarseMaxIter)) != cudaSuccess) return e;
     return cudaEventRecord(ev[1], st);
   }
   const Batch& b = *L.b;
   MgLevel& C = mg.lev[l - 1];
+  Vecs& V = w.v[l];
+  Vecs& Cv = w.v[l - 1];   // unused below level 1: the coarsest batch holds its own vectors
   const unsigned g = grid_rows(b), gc = grid_rows(*C.b);
+  const int64_t n = b.NBR, nc = C.b->NBR;
   const MgOp A = op_of(b);
+  double2* rhs0 = l == 1 ? (double2*)w.coarse->rhs : nullptr;
   cudaEventRecord(ev[0], st);
-  k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], L.d[1], L.x, L.r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
-  k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[1], L.d[0], L.x, L.r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
-  k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], nullptr, L.x, L.r, 0.0, 0.0, b.dscale, b.scoup, L.d[1]);
-  if (gc && mg.nonnested)
-    k_mgn_restrict<<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), L.d[1], L.child_ptr, L.child, L.child_w, C.bv, C.x, C.r,
-                                      C.d[0], C.inv_theta, l == 1 ? (double2*)C.b->rhs : nullptr);
-  else if (gc)
-    k_mg_restrict<<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), L.d[1], L.child_ptr, L.child, C.bv, C.x, C.r, C.d[0],
-                                     C.inv_theta, l == 1 ? (double2*)C.b->rhs : nullptr);
+  each_group<K>([&](auto width, int c0) {
+    constexpr int G = decltype(width)::value;
+    double2 *d0 = at(V.d[0], n, c0), *d1 = at(V.d[1], n, c0), *x = at(V.x, n, c0), *r = at(V.r, n, c0);
+    k_mg_cheb_step<G><<<g, kT, 0, st>>>(A, d0, d1, x, r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
+    k_mg_cheb_step<G><<<g, kT, 0, st>>>(A, d1, d0, x, r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
+    k_mg_cheb_step<G><<<g, kT, 0, st>>>(A, d0, nullptr, x, r, 0.0, 0.0, b.dscale, b.scoup, d1);
+    double2* r0 = rhs0 ? rhs0 + c0 * w.coarse_nv : nullptr;
+    if (gc && mg.nonnested)
+      k_mgn_restrict<G><<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), d1, L.child_ptr, L.child, L.child_w, at(Cv.bv, nc, c0),
+                                           at(Cv.x, nc, c0), at(Cv.r, nc, c0), at(Cv.d[0], nc, c0), C.inv_theta, r0,
+                                           w.coarse_nv);
+    else if (gc)
+      k_mg_restrict<G><<<gc, kT, 0, st>>>(side_of(b), side_of(*C.b), d1, L.child_ptr, L.child, at(Cv.bv, nc, c0),
+                                          at(Cv.x, nc, c0), at(Cv.r, nc, c0), at(Cv.d[0], nc, c0), C.inv_theta, r0,
+                                          w.coarse_nv);
+  });
   cudaEventRecord(ev[1], st);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  if ((e = vcycle(ctx, fine, l - 1)) != cudaSuccess) return e;
+  if ((e = vcycle<K>(ctx, fine, w, l - 1)) != cudaSuccess) return e;
   cudaEventRecord(ev[2], st);
-  if (mg.nonnested)
-    k_mgn_prolong<<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par3, L.w3, l == 1 ? (const double2*)C.b->x : C.x, L.x);
-  else
-    k_mg_prolong<<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par, l == 1 ? (const double2*)C.b->x : C.x, L.x);
-  k_mg_resid<<<g, kT, 0, st>>>(A, L.x, L.bv, L.r, L.d[0], L.inv_theta);
-  k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[0], L.d[1], L.x, L.r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
-  k_mg_cheb_step<<<g, kT, 0, st>>>(A, L.d[1], L.d[0], L.x, L.r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
-  k_mg_add<<<g, kT, 0, st>>>(L.x, L.d[0]);
+  each_group<K>([&](auto width, int c0) {
+    constexpr int G = decltype(width)::value;
+    double2 *d0 = at(V.d[0], n, c0), *d1 = at(V.d[1], n, c0), *x = at(V.x, n, c0), *r = at(V.r, n, c0);
+    const double2* xc = l == 1 ? (const double2*)w.coarse->x + c0 * w.coarse_map.col_stride : at(Cv.x, nc, c0);
+    const ColMap cm = l == 1 ? w.coarse_map : ColMap{G, 1};
+    if (mg.nonnested)
+      k_mgn_prolong<G><<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par3, L.w3, xc, cm, x);
+    else
+      k_mg_prolong<G><<<g, kT, 0, st>>>(side_of(b), side_of(*C.b), L.par, xc, cm, x);
+    k_mg_resid<G><<<g, kT, 0, st>>>(A, x, at(V.bv, n, c0), r, d0, L.inv_theta);
+    k_mg_cheb_step<G><<<g, kT, 0, st>>>(A, d0, d1, x, r, L.c1[0], L.c2[0], nullptr, nullptr, nullptr);
+    k_mg_cheb_step<G><<<g, kT, 0, st>>>(A, d1, d0, x, r, L.c1[1], L.c2[1], nullptr, nullptr, nullptr);
+    k_mg_add<G><<<g, kT, 0, st>>>(x, d0);
+  });
   cudaEventRecord(ev[3], st);
-  c.launches += 9;
+  c.launches += 9 * groups_of(K);
   return cudaGetLastError();
 }
 
-// z = V(rhs) on the finest level: the result is in lev[levels].x
-cudaError_t vcycle_top(fea_ctx* ctx, Batch& fine, const double2* rhs) {
+// z = V(rhs) on the finest level for the cases in `mask` (the others get z = V(0)): the result is in v[levels].x
+template <int K>
+cudaError_t vcycle_top(fea_ctx* ctx, Batch& fine, Work& w, const double2* rhs, unsigned mask) {
   Mg& mg = *fine.mg;
-  MgLevel& L = mg.lev[mg.levels];
-  L.bv = const_cast<double2*>(rhs);
-  k_mg_top_init<<<grid_rows(fine), kT, 0, ctx->c.stream>>>(rhs, L.x, L.r, L.d[0], L.inv_theta);
-  ctx->c.launches += 1;
-  return vcycle(ctx, fine, mg.levels);
+  Vecs& V = w.v[mg.levels];
+  V.bv = const_cast<double2*>(rhs);
+  const int64_t n = fine.NBR;
+  each_group<K>([&](auto width, int c0) {
+    constexpr int G = decltype(width)::value;
+    k_mg_top_init<G><<<grid_rows(fine), kT, 0, ctx->c.stream>>>(rhs + c0 * n, at(V.x, n, c0), at(V.r, n, c0), at(V.d[0], n, c0),
+                                                                 mg.lev[mg.levels].inv_theta, mask >> c0);
+  });
+  ctx->c.launches += groups_of(K);
+  return vcycle<K>(ctx, fine, w, mg.levels);
 }
 
 void accumulate_level_ms(Mg& mg) {
@@ -732,6 +1001,244 @@ void accumulate_level_ms(Mg& mg) {
     if (l > 0) cudaEventElapsedTime(&b, ev[2], ev[3]);
     mg.lev[l].ms += (double)a + (double)b;
   }
+}
+
+// device outputs of a solve, per case: what fea_batch_download reads (status, iters, rz0, r.r at exit, u,
+// ranges, relres); col [NBR] holds one case's x for the finalize kernels when K > 1
+struct Out {
+  int32_t *status, *iters;
+  double *rz0, *rz_last, *u, *ranges, *relres;
+  double2* col;
+};
+
+// Flexible CG preconditioned by one V-cycle per iteration, for K cases at once.  Per case, every decision is
+// that of a single solve: its own status, iteration count, first-iteration flag, restarts from the true residual
+// (kMaxRestarts) and breakdown test.  A finished case is frozen (x and r no longer change, and it enters the
+// V-cycle with a zero right-hand side); the loop ends when every case has finished.  One host poll per outer
+// iteration serves all cases.
+template <int K>
+int solve(fea_ctx* ctx, Batch& b, Work& w, double rtol, int max_iter, const Out& o, fea_solve_stats& stats) {
+  Mg& mg = *b.mg;
+  Ctx& c = ctx->c;
+  cudaStream_t st = c.stream;
+  const unsigned g = grid_rows(b);
+  const int np = (int)g;
+  const MgOp A = op_of(b);
+  const Side F = side_of(b);
+  double* h = mg.h_sc;
+  cudaEvent_t ev0 = mg.ev[4 * (mg.levels + 1)], ev1 = mg.ev[4 * (mg.levels + 1) + 1];
+  const unsigned all = (1u << K) - 1;
+  stats = fea_solve_stats{};
+  for (auto& L : mg.lev) L.ms = 0.0;
+  const int64_t launches0 = c.launches;
+  CK(ctx, cudaEventRecord(ev0, st));
+  int32_t empty = 0;
+  CK(ctx, cudaMemcpyAsync(&empty, b.empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  const int64_t n = b.NBR;
+  auto residual = [&](int mode, unsigned mask, int slot) -> cudaError_t {
+    each_group<K>([&](auto width, int c0) {
+      constexpr int G = decltype(width)::value;
+      k_mg_fcg_residual<G><<<g, kT, 0, st>>>(A, F, w.rhs + c0 * w.rhs_stride, w.rhs_stride, at(w.x, n, c0), at(w.r, n, c0),
+                                             at(w.p, n, c0), at(w.q, n, c0), mode, mask >> c0, w.partA + c0 * np);
+    });
+    return reduce(b, w.sc, K, w.partA, nullptr, np, kRedStore, slot, 0, mask);
+  };
+  auto poll = [&]() -> cudaError_t {
+    cudaError_t e = cudaMemcpyAsync(h, w.sc, sizeof(double) * K * kScCount, cudaMemcpyDeviceToHost, st);
+    return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
+  };
+  CK(ctx, residual(0, all, kScRZ0));
+  CK(ctx, poll());
+  CaseInts status, it;
+  int restarts[K], first[K];
+  double rr[K], tol2[K], rz0[K];
+  for (int q = 0; q < K; ++q) {
+    const double* hq = h + q * kScCount;
+    rz0[q] = hq[kScRZ0];
+    tol2[q] = rtol * rtol * rz0[q];
+    rr[q] = rz0[q];
+    status.v[q] = FEA_SAMPLE_NOT_RUN;
+    it.v[q] = restarts[q] = 0;
+    first[q] = 1;
+    if (empty) status.v[q] = FEA_SAMPLE_EMPTY_ROW;
+    else if (!(rz0[q] > 0.0)) status.v[q] = std::isfinite(rz0[q]) ? FEA_SAMPLE_CONVERGED : FEA_SAMPLE_BREAKDOWN;
+    if (status.v[q] == FEA_SAMPLE_CONVERGED)
+      CK(ctx, cudaMemcpyAsync(w.sc + q * kScCount + kScTrue, &rz0[q], sizeof(double), cudaMemcpyHostToDevice, st));
+  }
+  for (;;) {
+    // recursive residuals that met the tolerance: decide on the TRUE residual
+    unsigned check = 0;
+    for (int q = 0; q < K; ++q)
+      if (status.v[q] == FEA_SAMPLE_NOT_RUN && rr[q] <= tol2[q]) check |= 1u << q;
+    if (check) {
+      CK(ctx, residual(2, check, kScTrue));
+      CK(ctx, poll());
+      c.launches += 2;
+      for (int q = 0; q < K; ++q) {
+        if (!((check >> q) & 1u)) continue;
+        rr[q] = h[q * kScCount + kScTrue];
+        if (rr[q] <= tol2[q]) status.v[q] = FEA_SAMPLE_CONVERGED;
+        else if (!std::isfinite(rr[q])) status.v[q] = FEA_SAMPLE_BREAKDOWN;
+        else if (++restarts[q] > kMaxRestarts) status.v[q] = FEA_SAMPLE_STAGNATED;
+        else first[q] = 1;   // restart from the true residual (p = q = 0)
+      }
+    }
+    unsigned act = 0, first_bits = 0;
+    for (int q = 0; q < K; ++q) {
+      if (status.v[q] != FEA_SAMPLE_NOT_RUN) continue;
+      if (it.v[q] >= max_iter) {
+        status.v[q] = FEA_SAMPLE_MAX_ITER;
+        continue;
+      }
+      act |= 1u << q;
+      if (first[q]) first_bits |= 1u << q;
+    }
+    if (!act) break;
+    CK(ctx, vcycle_top<K>(ctx, b, w, w.r, act));
+    const double2* z = w.v[mg.levels].x;
+    each_group<K>([&](auto width, int c0) {
+      constexpr int G = decltype(width)::value;
+      k_mg_fcg_dots<G><<<g, kT, 0, st>>>(at(z, n, c0), at(w.r, n, c0), at(w.q, n, c0), w.partA + c0 * np, w.partB + c0 * np);
+    });
+    CK(ctx, reduce(b, w.sc, K, w.partA, w.partB, np, kRedDots, 0, first_bits, act));
+    each_group<K>([&](auto width, int c0) {
+      constexpr int G = decltype(width)::value;
+      k_mg_fcg_dir<G><<<g, kT, 0, st>>>(at(z, n, c0), at(w.p, n, c0), w.sc + c0 * kScCount, act >> c0);
+      k_mg_fcg_spmv<G><<<g, kT, 0, st>>>(A, at(w.p, n, c0), at(w.q, n, c0), act >> c0, w.partA + c0 * np);
+    });
+    CK(ctx, reduce(b, w.sc, K, w.partA, nullptr, np, kRedPQ, 0, 0, act));
+    each_group<K>([&](auto width, int c0) {
+      constexpr int G = decltype(width)::value;
+      k_mg_fcg_update<G><<<g, kT, 0, st>>>(at(w.x, n, c0), at(w.r, n, c0), at(w.p, n, c0), at(w.q, n, c0),
+                                           w.sc + c0 * kScCount, act >> c0, w.partA + c0 * np);
+    });
+    CK(ctx, reduce(b, w.sc, K, w.partA, nullptr, np, kRedStore, kScRR, 0, act));
+    CK(ctx, poll());   // one host poll per outer iteration (the coarse solve polls anyway)
+    c.launches += 4 + 4 * groups_of(K);
+    accumulate_level_ms(mg);
+    unsigned broke = 0;
+    for (int q = 0; q < K; ++q) {
+      if (!((act >> q) & 1u)) continue;
+      const double* hq = h + q * kScCount;
+      if (!(hq[kScPQ] > 0.0) || !std::isfinite(hq[kScPQ]) || !std::isfinite(hq[kScAlpha]) || !std::isfinite(hq[kScRR])) {
+        // not SPD on this Krylov space (or a non-finite step): k_mg_fcg_update left x and r alone, so u and
+        // relres are those of the last sound iterate
+        status.v[q] = FEA_SAMPLE_BREAKDOWN;
+        broke |= 1u << q;
+        continue;
+      }
+      ++it.v[q];
+      first[q] = 0;
+      rr[q] = hq[kScRR];
+    }
+    if (broke) CK(ctx, residual(1, broke, kScTrue));
+  }
+  unsigned unfinished = 0;
+  for (int q = 0; q < K; ++q)
+    if (status.v[q] == FEA_SAMPLE_MAX_ITER || status.v[q] == FEA_SAMPLE_STAGNATED) unfinished |= 1u << q;
+  if (unfinished) CK(ctx, residual(1, unfinished, kScTrue));
+  k_mg_finish<<<1, 32, 0, st>>>(K, o.status, o.iters, o.rz0, o.rz_last, w.sc, status, it);
+  CK(ctx, cudaGetLastError());
+  for (int q = 0; q < K; ++q) {
+    const double* xq = (const double*)w.x;
+    if (K > 1) {
+      each_group<K>([&](auto width, int c0) {
+        constexpr int G = decltype(width)::value;
+        if (q >= c0 && q < c0 + G) k_mg_column<<<g, kT, 0, st>>>(at(w.x, n, c0), G, q - c0, o.col);
+      });
+      xq = (const double*)o.col;
+    }
+    CK(ctx, launch_finalize_to(b, xq, o.status + q, o.rz_last + q, o.rz0 + q, o.u + 2 * b.NV * q, o.ranges + 4 * q,
+                               o.relres + q));
+  }
+  CK(ctx, cudaEventRecord(ev1, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  for (int q = 0; q < K; ++q) {
+    stats.iterations = std::max(stats.iterations, it.v[q]);
+    stats.n_converged += status.v[q] == FEA_SAMPLE_CONVERGED;
+    stats.refined_systems += restarts[q] > 0;
+  }
+  cudaEventElapsedTime(&stats.solve_ms, ev0, ev1);
+  c.launches += 1 + groups_of(K) + 3 * K + (K > 1 ? K : 0) + 3;
+  stats.kernel_launches = c.launches - launches0;
+  return FEA_OK;
+}
+
+// cells of level 0 replicated per case: case k's cell c is cell c of level 0 with its vertices shifted by
+// k * vertex_shift; creg (if given) gets level 0's region as the int8 input of api_batch_finish
+__global__ void k_mg_replicate_cells(int64_t nc, int n_cases, const int32_t* __restrict__ conn0, const int32_t* __restrict__ creg0,
+                                     int64_t vertex_shift, int32_t* __restrict__ conn, int8_t* __restrict__ creg) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nc * n_cases) return;
+  const int k = (int)(i / nc);
+  const int64_t cell = i - k * nc;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) conn[3 * i + a] = (int32_t)(conn0[3 * cell + a] + k * vertex_shift);
+  if (creg) creg[i] = (int8_t)creg0[cell];
+}
+
+// The coarsest batch of a solve of K > 1 cases: K samples, each a copy of level 0 -- mesh, fixed mask, D and
+// its matrices ke (copied, not recomputed; Galerkin or rediscretised alike) -- so that each of its systems is
+// bit for bit level 0's.  Built once per K and kept in mg.coarse[K].
+int coarse_for_cases(fea_ctx* ctx, Batch& b, int K) {
+  Mg& mg = *b.mg;
+  if (mg.coarse[K]) return FEA_OK;
+  const Batch& c0 = *mg.lev[0].b;
+  cudaStream_t st = ctx->c.stream;
+  const int64_t nv = c0.NV, nc = c0.NC;
+  const int32_t nr = c0.NREG;
+  std::vector<int64_t> vo(K + 1), co(K + 1);
+  std::vector<int32_t> ro(K + 1);
+  for (int k = 0; k <= K; ++k) {
+    vo[k] = k * nv;
+    co[k] = k * nc;
+    ro[k] = k * nr;
+  }
+  fea_batch* created = nullptr;
+  int rc = api_batch_begin(ctx, K, 3, vo.data(), co.data(), ro.data(), &created);
+  if (rc != FEA_OK) return rc;
+  std::unique_ptr<fea_batch, decltype(&api_free_batch)> hb(created, api_free_batch);
+  Batch& kb = hb->b;
+  CK(ctx, dalloc(kb, &kb.xy, kb.NV * 2));
+  CK(ctx, dalloc(kb, &kb.D, (int64_t)kb.NREG * 9));
+  CK(ctx, dalloc(kb, &kb.fixed, kb.NV));
+  CK(ctx, dalloc(kb, &kb.rhs, kb.NV * 2));
+  for (int k = 0; k < K; ++k) {
+    CK(ctx, cudaMemcpyAsync(kb.xy + 2 * nv * k, c0.xy, sizeof(double) * 2 * nv, cudaMemcpyDeviceToDevice, st));
+    CK(ctx, cudaMemcpyAsync(kb.D + 9 * (int64_t)nr * k, c0.D, sizeof(double) * 9 * nr, cudaMemcpyDeviceToDevice, st));
+    CK(ctx, cudaMemcpyAsync(kb.fixed + nv * k, c0.fixed, nv, cudaMemcpyDeviceToDevice, st));
+  }
+  CK(ctx, cudaMemsetAsync(kb.rhs, 0, sizeof(double) * 2 * kb.NV, st));
+  const unsigned gcell = (unsigned)((std::max<int64_t>(kb.NC, 1) + 255) / 256);
+  {
+    Scratch scratch(st);
+    int32_t* conn = nullptr;
+    int8_t* creg = nullptr;
+    CK(ctx, scratch.alloc(&conn, kb.NC * 3));
+    CK(ctx, scratch.alloc(&creg, kb.NC));
+    k_mg_replicate_cells<<<gcell, 256, 0, st>>>(nc, K, c0.conn, c0.cell_dreg, 0, conn, creg);
+    CK(ctx, cudaGetLastError());
+    if ((rc = api_batch_finish(ctx, kb, creg, conn)) != FEA_OK) return rc;
+  }
+  // level 0's cells are oriented already: take them exactly as they are, whatever the orientation test made of them
+  k_mg_replicate_cells<<<gcell, 256, 0, st>>>(nc, K, c0.conn, c0.cell_dreg, nv, kb.conn, nullptr);
+  CK(ctx, cudaGetLastError());
+  rc = api_batch_assemble(ctx, kb, [&c0, K](Batch& x) -> cudaError_t {
+    for (int k = 0; k < K; ++k) {
+      const cudaError_t e = cudaMemcpyAsync(x.ke + 36 * c0.NC * k, c0.ke, sizeof(double) * 36 * c0.NC, cudaMemcpyDeviceToDevice,
+                                            x.ctx->stream);
+      if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+  });
+  if (rc != FEA_OK) return rc;
+  int64_t rows = 0;   // block rows of one sample (every sample has level 0's)
+  CK(ctx, cudaMemcpyAsync(&rows, kb.row_base + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  mg.case_rows = rows;
+  ctx->c.launches += 2;
+  mg.coarse[K] = hb.release();
+  return FEA_OK;
 }
 
 }  // namespace
@@ -858,7 +1365,7 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
       CK(ctx, cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st));
     }
   }
-  if (!mg.h_sc) CK(ctx, cudaHostAlloc((void**)&mg.h_sc, sizeof(double) * kScCount, cudaHostAllocDefault));
+  if (!mg.h_sc) CK(ctx, cudaHostAlloc((void**)&mg.h_sc, sizeof(double) * kScCount * kMaxCases, cudaHostAllocDefault));
   if (mg.ev.empty()) {
     mg.ev.resize(4 * (mg.levels + 1) + 2);
     for (auto& ev : mg.ev) CK(ctx, cudaEventCreate(&ev));
@@ -873,9 +1380,10 @@ int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z) {
   const unsigned g = grid_rows(b);
   if (!g) return FEA_OK;
   for (auto& L : mg.lev) L.ms = 0.0;
+  Work w = own_work(b);
   k_mg_load<<<g, kT, 0, st>>>(side_of(b), b.vrank, d_r, mg.r);
-  CK(ctx, vcycle_top(ctx, b, mg.r));
-  k_mg_store<<<g, kT, 0, st>>>(side_of(b), b.vrank, mg.lev[mg.levels].x, d_z);
+  CK(ctx, vcycle_top<1>(ctx, b, w, mg.r, 1u));
+  k_mg_store<<<g, kT, 0, st>>>(side_of(b), b.vrank, w.v[mg.levels].x, d_z);
   ctx->c.launches += 2;
   CK(ctx, cudaGetLastError());
   CK(ctx, cudaStreamSynchronize(st));
@@ -884,90 +1392,85 @@ int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z) {
 }
 
 int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
-  Mg& mg = *b.mg;
-  Ctx& c = ctx->c;
-  cudaStream_t st = c.stream;
-  const unsigned g = grid_rows(b);
-  const int np = (int)g;
-  const MgOp A = op_of(b);
-  const Side F = side_of(b);
-  double2* x = (double2*)b.x;
-  double* h = mg.h_sc;
-  cudaEvent_t ev0 = mg.ev[4 * (mg.levels + 1)], ev1 = mg.ev[4 * (mg.levels + 1) + 1];
-  b.stats = fea_solve_stats{};
+  Work w = own_work(b);
   b.t_spmv.clear();
   b.t_update.clear();
-  for (auto& L : mg.lev) L.ms = 0.0;
-  const int64_t launches0 = c.launches;
-  CK(ctx, cudaEventRecord(ev0, st));
-  int32_t empty = 0;
-  CK(ctx, cudaMemcpyAsync(&empty, b.empty, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 0, mg.partA);
-  CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScRZ0));
-  CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
+  const Out o{b.sc.status, b.sc.iters, b.sc.rz0, b.rz_last, b.u, b.ranges, b.relres, nullptr};
+  return solve<1>(ctx, b, w, rtol, max_iter, o, b.stats);
+}
+
+int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int K, const double* rhs, double rtol, int max_iter, double* u, double* ranges,
+                        int32_t* iters, double* relres, int32_t* status, fea_solve_stats* stats) {
+  Mg& mg = *b.mg;
+  cudaStream_t st = ctx->c.stream;
+  Work w;
+  if (K == 1) {
+    w.coarse = mg.lev[0].b;
+  } else {
+    const int rc = coarse_for_cases(ctx, b, K);
+    if (rc != FEA_OK) return rc;
+    w.coarse = &mg.coarse[K]->b;
+    w.coarse_map = ColMap{1, mg.case_rows};
+  }
+  w.coarse_nv = mg.lev[0].b->NV;
+  Scratch scratch(st);
+  auto zeroed = [&](double2** p, int64_t n) -> cudaError_t {
+    cudaError_t e = scratch.alloc(p, n);
+    return e == cudaSuccess ? cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st) : e;
+  };
+  w.v.resize(mg.levels + 1);
+  for (int l = 1; l <= mg.levels; ++l) {
+    const int64_t n = mg.lev[l].b->NBR * K;
+    Vecs& V = w.v[l];
+    CK(ctx, zeroed(&V.x, n));
+    CK(ctx, zeroed(&V.r, n));
+    CK(ctx, zeroed(&V.d[0], n));
+    CK(ctx, zeroed(&V.d[1], n));
+    if (l < mg.levels) CK(ctx, zeroed(&V.bv, n));   // the finest level's b is the outer CG's r
+  }
+  const int64_t nbr = b.NBR, np = nbr / kT;
+  CK(ctx, zeroed(&w.x, nbr * K));
+  CK(ctx, zeroed(&w.r, nbr * K));
+  CK(ctx, zeroed(&w.p, nbr * K));
+  CK(ctx, zeroed(&w.q, nbr * K));
+  CK(ctx, scratch.alloc(&w.partA, np * K));
+  CK(ctx, scratch.alloc(&w.partB, np * K));
+  CK(ctx, scratch.alloc(&w.sc, (int64_t)kScCount * K));
+  CK(ctx, cudaMemsetAsync(w.sc, 0, sizeof(double) * kScCount * K, st));
+  double* d_rhs = nullptr;
+  CK(ctx, scratch.alloc(&d_rhs, 2 * b.NV * K));
+  CK(ctx, cudaMemcpyAsync(d_rhs, rhs, sizeof(double) * 2 * b.NV * K, cudaMemcpyHostToDevice, st));
+  w.rhs = d_rhs;
+  w.rhs_stride = 2 * b.NV;
+  Out o{};
+  CK(ctx, scratch.alloc(&o.status, K));
+  CK(ctx, scratch.alloc(&o.iters, K));
+  CK(ctx, scratch.alloc(&o.rz0, K));
+  CK(ctx, scratch.alloc(&o.rz_last, K));
+  CK(ctx, scratch.alloc(&o.u, 2 * b.NV * K));
+  CK(ctx, scratch.alloc(&o.ranges, 4 * K));
+  CK(ctx, scratch.alloc(&o.relres, K));
+  if (K > 1) CK(ctx, scratch.alloc(&o.col, nbr));
+  fea_solve_stats s{};
+  int rc = FEA_BAD_ARG;
+  switch (K) {
+    case 1: rc = solve<1>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 2: rc = solve<2>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 3: rc = solve<3>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 4: rc = solve<4>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 5: rc = solve<5>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 6: rc = solve<6>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 7: rc = solve<7>(ctx, b, w, rtol, max_iter, o, s); break;
+    case 8: rc = solve<8>(ctx, b, w, rtol, max_iter, o, s); break;
+  }
+  if (rc != FEA_OK) return rc;
+  if (u) CK(ctx, cudaMemcpyAsync(u, o.u, sizeof(double) * 2 * b.NV * K, cudaMemcpyDeviceToHost, st));
+  if (ranges) CK(ctx, cudaMemcpyAsync(ranges, o.ranges, sizeof(double) * 4 * K, cudaMemcpyDeviceToHost, st));
+  if (iters) CK(ctx, cudaMemcpyAsync(iters, o.iters, sizeof(int32_t) * K, cudaMemcpyDeviceToHost, st));
+  if (relres) CK(ctx, cudaMemcpyAsync(relres, o.relres, sizeof(double) * K, cudaMemcpyDeviceToHost, st));
+  if (status) CK(ctx, cudaMemcpyAsync(status, o.status, sizeof(int32_t) * K, cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
-  const double rz0 = h[kScRZ0], tol2 = rtol * rtol * rz0;
-  int status = FEA_SAMPLE_NOT_RUN, it = 0, restarts = 0, first = 1;
-  double rr = rz0;
-  if (empty) status = FEA_SAMPLE_EMPTY_ROW;
-  else if (!(rz0 > 0.0)) status = std::isfinite(rz0) ? FEA_SAMPLE_CONVERGED : FEA_SAMPLE_BREAKDOWN;
-  if (status == FEA_SAMPLE_CONVERGED) {
-    CK(ctx, cudaMemcpyAsync(mg.sc + kScTrue, &rz0, sizeof(double), cudaMemcpyHostToDevice, st));
-  }
-  while (status == FEA_SAMPLE_NOT_RUN) {
-    if (rr <= tol2) {   // recursive residual met the tolerance: decide on the TRUE residual
-      k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 2, mg.partA);
-      CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
-      CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
-      CK(ctx, cudaStreamSynchronize(st));
-      c.launches += 2;
-      rr = h[kScTrue];
-      if (rr <= tol2) { status = FEA_SAMPLE_CONVERGED; break; }
-      if (!std::isfinite(rr)) { status = FEA_SAMPLE_BREAKDOWN; break; }
-      if (++restarts > kMaxRestarts) { status = FEA_SAMPLE_STAGNATED; break; }
-      first = 1;   // restart from the true residual (p = q = 0)
-    }
-    if (it >= max_iter) { status = FEA_SAMPLE_MAX_ITER; break; }
-    CK(ctx, vcycle_top(ctx, b, mg.r));
-    const double2* z = mg.lev[mg.levels].x;
-    k_mg_fcg_dots<<<g, kT, 0, st>>>(z, mg.r, mg.q, mg.partA, mg.partB);
-    CK(ctx, reduce(b, mg.partA, mg.partB, np, kRedDots, 0, first));
-    k_mg_fcg_dir<<<g, kT, 0, st>>>(z, mg.p, mg.sc);
-    k_mg_fcg_spmv<<<g, kT, 0, st>>>(A, mg.p, mg.q, mg.partA);
-    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedPQ));
-    k_mg_fcg_update<<<g, kT, 0, st>>>(x, mg.r, mg.p, mg.q, mg.sc, mg.partA);
-    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScRR));
-    CK(ctx, cudaMemcpyAsync(h, mg.sc, sizeof(double) * kScCount, cudaMemcpyDeviceToHost, st));
-    CK(ctx, cudaStreamSynchronize(st));   // one host poll per outer iteration (the coarse solve polls anyway)
-    c.launches += 8;
-    accumulate_level_ms(mg);
-    if (!(h[kScPQ] > 0.0) || !std::isfinite(h[kScPQ]) || !std::isfinite(h[kScAlpha]) || !std::isfinite(h[kScRR])) {
-      // not SPD on this Krylov space (or a non-finite step): k_mg_fcg_update left x and r alone, so u and
-      // relres are those of the last sound iterate
-      status = FEA_SAMPLE_BREAKDOWN;
-      k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 1, mg.partA);
-      CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
-      break;
-    }
-    ++it;
-    first = 0;
-    rr = h[kScRR];
-  }
-  if (status == FEA_SAMPLE_MAX_ITER || status == FEA_SAMPLE_STAGNATED) {
-    k_mg_fcg_residual<<<g, kT, 0, st>>>(A, F, b.rhs, x, mg.r, mg.p, mg.q, 1, mg.partA);
-    CK(ctx, reduce(b, mg.partA, nullptr, np, kRedStore, kScTrue));
-  }
-  k_mg_finish<<<1, 32, 0, st>>>(b.sc, b.rz_last, mg.sc, status, it);
-  CK(ctx, cudaGetLastError());
-  CK(ctx, launch_finalize(b));
-  CK(ctx, cudaEventRecord(ev1, st));
-  CK(ctx, cudaStreamSynchronize(st));
-  b.stats.iterations = it;
-  b.stats.n_converged = status == FEA_SAMPLE_CONVERGED ? 1 : 0;
-  b.stats.refined_systems = restarts > 0 ? 1 : 0;
-  cudaEventElapsedTime(&b.stats.solve_ms, ev0, ev1);
-  c.launches += 8;
-  b.stats.kernel_launches = c.launches - launches0;
+  if (stats) *stats = s;
   return FEA_OK;
 }
 
@@ -976,6 +1479,8 @@ void mg_release(Batch& b) {
   Mg* mg = b.mg;
   for (auto& L : mg->lev)
     if (L.hb) api_free_batch(L.hb);
+  for (fea_batch* cb : mg->coarse)
+    if (cb) api_free_batch(cb);
   for (auto& ev : mg->ev) cudaEventDestroy(ev);
   if (mg->h_sc) cudaFreeHost(mg->h_sc);
   delete mg;

@@ -751,15 +751,20 @@ __global__ void k_relres(int ns, const double* __restrict__ rz_last, const doubl
   relres[s] = rz0[s] > 0.0 ? sqrt(rz_last[s] / rz0[s]) : 0.0;
 }
 
-cudaError_t launch_finalize(Batch& b) {
+cudaError_t launch_finalize_to(Batch& b, const double* x, const int32_t* status, const double* rz_last, const double* rz0,
+                               double* u, double* ranges, double* relres) {
   cudaStream_t st = b.ctx->stream;
   const int T = 256;
   if (b.NV)
     k_unscale_scatter<<<(unsigned)((b.NV + T - 1) / T), T, 0, st>>>(b.NV, b.vsample, b.row_of_vertex, b.dscale, b.scoup,
-                                                                   (const double2*)b.x, b.sc.status, (double2*)b.u);
-  k_minmax<<<b.ns, 256, 0, st>>>(b.d_vtx_off, (const double2*)b.u, b.ranges);
-  k_relres<<<(b.ns + T - 1) / T, T, 0, st>>>(b.ns, b.rz_last, b.sc.rz0, b.relres);
+                                                                   (const double2*)x, status, (double2*)u);
+  k_minmax<<<b.ns, 256, 0, st>>>(b.d_vtx_off, (const double2*)u, ranges);
+  k_relres<<<(b.ns + T - 1) / T, T, 0, st>>>(b.ns, rz_last, rz0, relres);
   return cudaGetLastError();
+}
+
+cudaError_t launch_finalize(Batch& b) {
+  return launch_finalize_to(b, b.x, b.sc.status, b.rz_last, b.sc.rz0, b.u, b.ranges, b.relres);
 }
 
 // ---------------------------------------------------------------------------

@@ -256,6 +256,17 @@ class BatchResult:
     stats: Optional[dict] = None
 
 
+@dataclass
+class LoadCaseResult:
+    """Outputs of ``Batch.solve_load_cases``: per load case, what ``BatchResult`` holds for the batch's sample."""
+    u: np.ndarray          # (K, n_vertices, 2)
+    ranges: np.ndarray     # (K, 4): min ux, max ux, min uy, max uy
+    iters: np.ndarray      # (K,) outer iterations
+    relres: np.ndarray     # (K,)
+    status: np.ndarray     # (K,)
+    stats: dict            # fea_solve_stats of the call (iterations = the largest outer count)
+
+
 class PinnedArena:
     """A reusable block of page-locked host memory handed out as numpy arrays: staging buffers of a
     pipeline step are carved from it (``empty``) and recycled with ``reset`` -- no page faults, no
@@ -708,6 +719,27 @@ class Batch:
         indices, data = np.empty(nnz, np.int32), np.empty(nnz)
         self.ctx._check(self.ctx.lib.fea_batch_get_level_transfer(self.h, int(level), None, ptr(indices), ptr(data)))
         return sp.csr_matrix((data, indices, indptr), shape=(n, m))
+
+    def solve_load_cases(self, loads: np.ndarray, rtol: float = 1e-10, max_iter: int = 20000) -> LoadCaseResult:
+        """Solve K = len(loads) load cases (1..8) of the batch's one sample together with its multigrid hierarchy.
+        ``loads`` (K, n_vertices, 2) float64: full-DOF loads like ``Sample.rhs`` (values at fixed DOFs are not
+        read).  Case k's outputs equal, bit for bit, those of ``solve`` on a batch whose rhs is loads[k]; the
+        batch's own results (``download``) do not change."""
+        nv = self.packed.n_vertices
+        if not isinstance(loads, np.ndarray) or loads.dtype != np.float64:
+            raise TypeError("loads must be a float64 numpy array")
+        if loads.ndim != 3 or loads.shape[1:] != (nv, 2):
+            raise ValueError("loads must have shape (K, %d, 2), not %s" % (nv, loads.shape))
+        loads = np.ascontiguousarray(loads)
+        k = loads.shape[0]
+        r = LoadCaseResult(u=np.empty((k, nv, 2)), ranges=np.empty((k, 4)), iters=np.empty(k, np.int32),
+                           relres=np.empty(k), status=np.empty(k, np.int32), stats={})
+        st = SolveStats()
+        self.ctx._check(self.ctx.lib.fea_batch_solve_load_cases(
+            self.h, int(k), ptr(loads), float(rtol), int(max_iter), ptr(r.u), ptr(r.ranges), ptr(r.iters),
+            ptr(r.relres), ptr(r.status), C.byref(st)))
+        r.stats = st.as_dict()
+        return r
 
     def mg_apply(self, r: np.ndarray) -> np.ndarray:
         """z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as ``spmv``)."""

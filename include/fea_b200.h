@@ -354,7 +354,8 @@ int  fea_batch_spmv(fea_batch* b, int32_t sample, const double* x, double* y);
 typedef struct {
   int64_t n_vertices, n_cells, n_active_dofs, nnz;   /* nnz of the reduced scalar CSR */
   double lambda_max;   /* estimate of the largest eigenvalue of the block-Jacobi-scaled operator */
-  double vcycle_ms;    /* V-cycle time spent on the level in the last solve (level 0: the coarse solves) */
+  double vcycle_ms;    /* V-cycle time spent on the level in the last solve, by fea_batch_solve or
+                        * fea_batch_solve_load_cases (level 0: the coarse solves) */
 } fea_mg_level;
 /* The batch's only sample is its own mesh refined `levels` (1..8) times, in the vertex and cell numbering
  * of uniform red refinement: vertices of level l-1 keep their indices, the midpoint of each level-(l-1)
@@ -373,6 +374,21 @@ int  fea_batch_get_mg_levels(fea_batch* b, int32_t cap, fea_mg_level* out, int32
 int  fea_batch_get_level_csr(fea_batch* b, int32_t level, int32_t* indptr, int32_t* indices, double* data);
 /* z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as fea_batch_spmv) */
 int  fea_batch_mg_apply(fea_batch* b, const double* r, double* z);
+/* K = n_cases load cases of the batch's one sample, solved together by the multigrid solve of
+ * fea_batch_set_refinement / fea_batch_set_coarse_meshes.  rhs [n_cases][n_vertices*2]: full-DOF loads in
+ * the layout of fea_batch_desc.rhs (values at fixed DOFs are not read).  Outputs (any may be NULL), with the
+ * meaning they have in fea_batch_download: u [n_cases][n_vertices*2], ranges [n_cases][4], iters, relres,
+ * status [n_cases]; stats as fea_batch_get_solve_stats (iterations = the largest outer count).
+ * Case k's outputs are bit for bit those fea_batch_solve gives a batch whose rhs is rhs[k], whatever other
+ * cases share the call.  The batch's own results (fea_batch_download, images, strain/stress) are not touched.
+ * The K cases share the hierarchy, every matrix read of the V-cycles and outer iterations (vectors of the
+ * cases are interleaved per row), and their coarse systems are solved side by side in one batch of K copies
+ * of level 0, built on the first call with that K and kept with the hierarchy.
+ * FEA_BAD_STATE: no multigrid hierarchy, or not assembled.  FEA_BAD_ARG: n_cases outside 1..8, null rhs,
+ * rtol < 0 or max_iter < 1. */
+int  fea_batch_solve_load_cases(fea_batch* b, int32_t n_cases, const double* rhs, double rtol, int32_t max_iter,
+                                double* u, double* ranges, int32_t* iters, double* relres, int32_t* status,
+                                fea_solve_stats* stats);
 
 /* ---- multigrid-preconditioned solve of a mesh with coarser meshes of the same domain ------------
  * The batch's only sample (P1 triangles) is the finest level of a hierarchy whose coarser levels are the samples
