@@ -29,6 +29,7 @@ EXPORTS = [
     "fea_batch_get_csr", "fea_batch_spmv", "fea_rasterize_fields", "fea_solve_batch",
     "fea_batch_set_refinement", "fea_batch_get_mg_levels", "fea_batch_get_level_csr", "fea_batch_mg_apply",
     "fea_batch_set_coarse_meshes", "fea_batch_get_level_transfer", "fea_batch_solve_load_cases",
+    "fea_batch_load_case_info", "fea_batch_load_case_images", "fea_batch_load_case_strain_stress", "fea_batch_load_case_cell_components",
 ]
 
 STATUS_NAMES = {0: "OK", 1: "BAD_ARG", 2: "CUDA_ERROR", 3: "OUT_OF_MEMORY", 4: "BAD_STATE", 5: "MESH_ERROR"}
@@ -169,6 +170,10 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "fea_batch_set_coarse_meshes": (C.c_int, [P, C.POINTER(BatchDesc)]),
         "fea_batch_get_level_transfer": (C.c_int, [P, I32, P, P, P]),
         "fea_batch_solve_load_cases": (C.c_int, [P, I32, P, F64, I32, P, P, P, P, P, C.POINTER(SolveStats)]),
+        "fea_batch_load_case_info": (C.c_int, [P, P, P, P]),
+        "fea_batch_load_case_images": (C.c_int, [P, I32, P, F64, P]),
+        "fea_batch_load_case_strain_stress": (C.c_int, [P, I32, P, P]),
+        "fea_batch_load_case_cell_components": (C.c_int, [P, I32, I32, P, F64, P, P]),
         "fea_solve_batch": (C.c_int, [P, C.POINTER(BatchDesc), F64, I32, I32, P, F64, P, P, P, P, P, P,
                                       C.POINTER(SolveStats)]),
     }

@@ -927,6 +927,120 @@ int fea_batch_solve_load_cases(fea_batch* hb, int32_t n_cases, const double* rhs
   return mg_solve_load_cases(ctx, b, n_cases, rhs, rtol, max_iter, u, ranges, iters, relres, status, stats);
 }
 
+int fea_batch_load_case_info(fea_batch* hb, int32_t* n_cases, int32_t* status, int32_t* image_size) {
+  if (!hb || !n_cases) return FEA_BAD_ARG;
+  *n_cases = 0;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg || !b.mg->n_kept) return api_fail(ctx, FEA_BAD_STATE, "no fea_batch_solve_load_cases call has succeeded on the batch");
+  const Mg& mg = *b.mg;
+  *n_cases = mg.n_kept;
+  if (image_size) *image_size = mg.case_size;
+  if (status) {
+    CK(ctx, cudaSetDevice(ctx->c.device));
+    CK(ctx, cudaMemcpyAsync(status, mg.case_status, sizeof(int32_t) * mg.n_kept, cudaMemcpyDeviceToHost, ctx->c.stream));
+    CK(ctx, cudaStreamSynchronize(ctx->c.stream));
+  }
+  return FEA_OK;
+}
+
+int fea_batch_load_case_images(fea_batch* hb, int32_t size, const double* affine, double value_scale, uint8_t* images) {
+  if (!hb || !affine || !images) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg || !b.mg->n_kept) return api_fail(ctx, FEA_BAD_STATE, "no fea_batch_solve_load_cases call has succeeded on the batch");
+  if (size < 1 || size > 8192) return api_fail(ctx, FEA_BAD_ARG, "image size out of range");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
+  Mg& mg = *b.mg;
+  const int K = mg.n_kept;
+  const int64_t per = (int64_t)size * size;
+  Scratch scratch(st);
+  double* d_affine = nullptr;
+  uint8_t* d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_affine, 4));
+  CK(ctx, scratch.alloc(&d_images, 2 * K * per));
+  // the owner map stays with the batch for fea_batch_load_case_cell_components (valid again once it is rebuilt)
+  const int32_t old_size = mg.case_size;
+  mg.case_size = 0;
+  if (old_size != size) {
+    if (mg.case_owner) CK(ctx, cudaFreeAsync(mg.case_owner, st));
+    mg.case_owner = nullptr;
+    CK(ctx, cudaMallocAsync((void**)&mg.case_owner, sizeof(int32_t) * per, st));
+  }
+  CK(ctx, cudaMemcpyAsync(d_affine, affine, sizeof(double) * 4, cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_case_owner(b, size, d_affine, mg.case_owner));
+  CK(ctx, launch_case_raster(b, K, size, d_affine, mg.case_owner, mg.case_u, mg.case_ranges, value_scale, d_images));
+  ctx->c.launches += 3;
+  mg.case_size = size;
+  CK(ctx, cudaMemcpyAsync(images, d_images, (size_t)(2 * K * per), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  return FEA_OK;
+}
+
+int fea_batch_load_case_strain_stress(fea_batch* hb, int32_t stress_region, double* strain, double* stress) {
+  if (!hb || (!strain && !stress)) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg || !b.mg->n_kept) return api_fail(ctx, FEA_BAD_STATE, "no fea_batch_solve_load_cases call has succeeded on the batch");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
+  const int K = b.mg->n_kept;
+  Scratch scratch(st);
+  double *d_strain = nullptr, *d_stress = nullptr;
+  CK(ctx, scratch.alloc(&d_strain, K * b.NC * 3));
+  CK(ctx, scratch.alloc(&d_stress, K * b.NC * 3));
+  CK(ctx, launch_case_strain_stress(b, K, b.mg->case_u, stress_region, d_strain, d_stress));
+  ctx->c.launches += 1;
+  if (strain) CK(ctx, cudaMemcpyAsync(strain, d_strain, sizeof(double) * 3 * b.NC * K, cudaMemcpyDeviceToHost, st));
+  if (stress) CK(ctx, cudaMemcpyAsync(stress, d_stress, sizeof(double) * 3 * b.NC * K, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  return FEA_OK;
+}
+
+int fea_batch_load_case_cell_components(fea_batch* hb, int32_t stress_region, int32_t n_fields, const int32_t* field_ids,
+                                        double value_scale, uint8_t* images, double* ranges) {
+  if (!hb || !field_ids || n_fields < 1 || n_fields > 4 || (!images && !ranges)) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg || !b.mg->n_kept) return api_fail(ctx, FEA_BAD_STATE, "no fea_batch_solve_load_cases call has succeeded on the batch");
+  Mg& mg = *b.mg;
+  if (!mg.case_size)
+    return api_fail(ctx, FEA_BAD_STATE, "fea_batch_load_case_cell_components before fea_batch_load_case_images");
+  for (int f = 0; f < n_fields; ++f)
+    if (field_ids[f] < 0 || field_ids[f] > 3) return api_fail(ctx, FEA_BAD_ARG, "field id must be 0..3");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
+  const int K = mg.n_kept;
+  const size_t per = (size_t)mg.case_size * mg.case_size;
+  const int64_t n_img = (int64_t)n_fields * K;
+  Scratch scratch(st);
+  double *d_strain = nullptr, *d_stress = nullptr, *d_ranges = nullptr;
+  int32_t* d_ids = nullptr;
+  int64_t* d_case_off = nullptr;
+  uint8_t* d_images = nullptr;
+  CK(ctx, scratch.alloc(&d_strain, K * b.NC * 3));
+  CK(ctx, scratch.alloc(&d_stress, K * b.NC * 3));
+  CK(ctx, scratch.alloc(&d_ids, 4));
+  CK(ctx, scratch.alloc(&d_case_off, kMaxCases + 1));
+  CK(ctx, scratch.alloc(&d_ranges, 2 * n_img));
+  CK(ctx, scratch.alloc(&d_images, n_img * (int64_t)per));
+  int32_t ids[4] = {0, 0, 0, 0};
+  for (int f = 0; f < n_fields; ++f) ids[f] = field_ids[f];
+  int64_t case_off[kMaxCases + 1];   // case k's cells in the case-major strain / stress arrays
+  for (int k = 0; k <= K; ++k) case_off[k] = k * b.NC;
+  CK(ctx, cudaMemcpyAsync(d_ids, ids, sizeof(ids), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaMemcpyAsync(d_case_off, case_off, sizeof(int64_t) * (K + 1), cudaMemcpyHostToDevice, st));
+  CK(ctx, launch_case_strain_stress(b, K, mg.case_u, stress_region, d_strain, d_stress));
+  CK(ctx, launch_case_cell_fields(b, K, mg.case_size, mg.case_owner, n_fields, d_ids, d_case_off, d_strain, d_stress,
+                                  value_scale, d_ranges, d_images));
+  ctx->c.launches += 3;
+  if (images) CK(ctx, cudaMemcpyAsync(images, d_images, (size_t)n_img * per, cudaMemcpyDeviceToHost, st));
+  if (ranges) CK(ctx, cudaMemcpyAsync(ranges, d_ranges, sizeof(double) * 2 * n_img, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));   // ids and case_off (host arrays) must outlive the copies
+  return FEA_OK;
+}
+
 int fea_batch_mg_apply(fea_batch* hb, const double* r, double* z) {
   if (!hb || !r || !z) return FEA_BAD_ARG;
   fea_ctx* ctx = hb->owner;

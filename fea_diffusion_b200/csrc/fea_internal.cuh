@@ -204,6 +204,14 @@ struct Mg {
   // coarsest batches of load-case solves: coarse[K] has K samples, each a copy of level 0 (built on first use)
   fea_batch* coarse[kMaxCases + 1] = {};
   int64_t case_rows = 0;         // block rows of one sample of those batches
+  // the last successful fea_batch_solve_load_cases, read by the fea_batch_load_case_* outputs (DESIGN.md 3.11)
+  int n_kept = 0;                // its K (0: no such call yet)
+  int kept_cap = 0;              // cases case_u has room for
+  double* case_u = nullptr;      // [kept_cap][NV*2] finalized u of each case
+  double* case_ranges = nullptr; // [kMaxCases][4]
+  int32_t* case_status = nullptr;   // [kMaxCases] what each kept field is (fea_batch_load_case_info)
+  int32_t* case_owner = nullptr; // [case_size^2] owner map of the last fea_batch_load_case_images (mesh and camera)
+  int32_t case_size = 0;
 };
 
 }  // namespace fea
@@ -299,6 +307,9 @@ cudaError_t launch_topology_counts(Batch& b);                 // incidence + adj
 cudaError_t launch_topology_fill(Batch& b);                   // adjacency fill
 cudaError_t launch_element_stiffness(Batch& b);
 cudaError_t launch_cell_strain_stress(Batch& b, int stress_region, double* d_strain, double* d_stress);
+// the same for the n_cases displacements u [n_cases][NV*2] of a one-sample triangle batch; outputs [n_cases][NC*3]
+cudaError_t launch_case_strain_stress(Batch& b, int n_cases, const double* u, int stress_region, double* d_strain,
+                                      double* d_stress);
 cudaError_t launch_sell_lengths(Batch& b);                    // slice_len + slice_ptr
 cudaError_t launch_sell_fill(Batch& b);                       // dscale, val, col
 cudaError_t launch_csr_export(Batch& b, int32_t s, int32_t* d_indptr, int32_t* d_indices,
@@ -321,6 +332,17 @@ cudaError_t launch_raster_flags(Batch& b, int64_t n_img, const int64_t* d_field_
                                 const uint8_t* d_flags, uint8_t* d_images);
 cudaError_t launch_raster_cell_fields(Batch& b, int n_fields, const int32_t* d_ids, const double* d_strain,
                                       const double* d_stress, double scale, double* d_ranges, uint8_t* d_images);
+// Load cases of a one-sample triangle batch (fea_batch_load_case_*), from one owner map [size*size] of the mesh:
+// owner fills it (cover pass with `affine` [4]); the shade launchers read it for every case.
+cudaError_t launch_case_owner(Batch& b, int size, const double* d_affine, int32_t* owner);
+// images [n_cases][2][size][size] of u [n_cases][NV*2] with ranges [n_cases][4]
+cudaError_t launch_case_raster(Batch& b, int n_cases, int size, const double* d_affine, const int32_t* owner,
+                               const double* u, const double* ranges, double value_scale, uint8_t* d_images);
+// strain / stress [n_cases][NC*3]; d_case_off = device {0, NC, ..., n_cases*NC}; ranges [n_fields][n_cases][2],
+// images [n_fields][n_cases][size][size]
+cudaError_t launch_case_cell_fields(Batch& b, int n_cases, int size, const int32_t* owner, int n_fields,
+                                    const int32_t* d_ids, const int64_t* d_case_off, const double* d_strain,
+                                    const double* d_stress, double scale, double* d_ranges, uint8_t* d_images);
 // n_fields vertex-scalar images of one mesh; cell_off2 = device {0, n_cell}
 cudaError_t launch_raster_fields(cudaStream_t st, int npc, int64_t n_v, int64_t n_cell, const int32_t* conn,
                                  const double* xy, const double* affine, const int64_t* cell_off2, int size,

@@ -1464,12 +1464,27 @@ int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int K, const double* rhs, double
     case 8: rc = solve<8>(ctx, b, w, rtol, max_iter, o, s); break;
   }
   if (rc != FEA_OK) return rc;
+  // keep u, ranges and status of the cases for the fea_batch_load_case_* outputs, replacing the last call's
+  mg.n_kept = 0;
+  if (mg.kept_cap < K) {
+    if (mg.case_u) CK(ctx, cudaFreeAsync(mg.case_u, st));
+    mg.case_u = nullptr;
+    mg.kept_cap = 0;
+    CK(ctx, cudaMallocAsync((void**)&mg.case_u, sizeof(double) * 2 * b.NV * K, st));
+    mg.kept_cap = K;
+  }
+  if (!mg.case_ranges) CK(ctx, cudaMallocAsync((void**)&mg.case_ranges, sizeof(double) * 4 * kMaxCases, st));
+  if (!mg.case_status) CK(ctx, cudaMallocAsync((void**)&mg.case_status, sizeof(int32_t) * kMaxCases, st));
+  CK(ctx, cudaMemcpyAsync(mg.case_u, o.u, sizeof(double) * 2 * b.NV * K, cudaMemcpyDeviceToDevice, st));
+  CK(ctx, cudaMemcpyAsync(mg.case_ranges, o.ranges, sizeof(double) * 4 * K, cudaMemcpyDeviceToDevice, st));
+  CK(ctx, cudaMemcpyAsync(mg.case_status, o.status, sizeof(int32_t) * K, cudaMemcpyDeviceToDevice, st));
   if (u) CK(ctx, cudaMemcpyAsync(u, o.u, sizeof(double) * 2 * b.NV * K, cudaMemcpyDeviceToHost, st));
   if (ranges) CK(ctx, cudaMemcpyAsync(ranges, o.ranges, sizeof(double) * 4 * K, cudaMemcpyDeviceToHost, st));
   if (iters) CK(ctx, cudaMemcpyAsync(iters, o.iters, sizeof(int32_t) * K, cudaMemcpyDeviceToHost, st));
   if (relres) CK(ctx, cudaMemcpyAsync(relres, o.relres, sizeof(double) * K, cudaMemcpyDeviceToHost, st));
   if (status) CK(ctx, cudaMemcpyAsync(status, o.status, sizeof(int32_t) * K, cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
+  mg.n_kept = K;
   if (stats) *stats = s;
   return FEA_OK;
 }
@@ -1481,6 +1496,8 @@ void mg_release(Batch& b) {
     if (L.hb) api_free_batch(L.hb);
   for (fea_batch* cb : mg->coarse)
     if (cb) api_free_batch(cb);
+  for (void* p : {(void*)mg->case_u, (void*)mg->case_ranges, (void*)mg->case_status, (void*)mg->case_owner})
+    if (p) cudaFreeAsync(p, b.ctx->stream);
   for (auto& ev : mg->ev) cudaEventDestroy(ev);
   if (mg->h_sc) cudaFreeHost(mg->h_sc);
   delete mg;

@@ -80,6 +80,25 @@ __global__ void k_raster_cover(int64_t NT, const int64_t* __restrict__ cell_off,
   }
 }
 
+// Gray level of component c of a displacement u at a pixel of triangle vid (weights w / a2): value_scale * u
+// interpolated, normalised by value_scale * (rng[2c], rng[2c+1]).  Every displacement image is shaded by this.
+__device__ __forceinline__ uint8_t shade_displacement(const double w[3], double a2, const int32_t vid[3],
+                                                      const double* __restrict__ u, int c, const double* __restrict__ rng4,
+                                                      double value_scale) {
+  const double s0 = __dmul_rn(value_scale, u[2 * (int64_t)vid[0] + c]);
+  const double s1 = __dmul_rn(value_scale, u[2 * (int64_t)vid[1] + c]);
+  const double s2 = __dmul_rn(value_scale, u[2 * (int64_t)vid[2] + c]);
+  const double val = __ddiv_rn(__dadd_rn(__dadd_rn(__dmul_rn(w[0], s0), __dmul_rn(w[1], s1)), __dmul_rn(w[2], s2)), a2);
+  const double vmin = __dmul_rn(value_scale, rng4[2 * c]);
+  const double vmax = __dmul_rn(value_scale, rng4[2 * c + 1]);
+  const double rng = __dsub_rn(vmax, vmin);
+  double tt = 0.0;
+  if (rng > 0.0) tt = __ddiv_rn(__dsub_rn(val, vmin), rng);
+  tt = fmin(fmax(tt, 0.0), 1.0);
+  const double q = fmin(floor(__dmul_rn(256.0, tt)), 255.0);
+  return (uint8_t)(255.0 - q);
+}
+
 template <int NPC>
 __global__ void k_raster_shade(int ns, int size, const int64_t* __restrict__ cell_off,
                                const int32_t* __restrict__ conn, const double* __restrict__ xy,
@@ -104,20 +123,7 @@ __global__ void k_raster_shade(int ns, int size, const int64_t* __restrict__ cel
     bary(t, (double)i + 0.5, (double)j + 0.5, w, &a2);
     uint8_t g[2];
 #pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const double s0 = __dmul_rn(value_scale, u[2 * (int64_t)vid[0] + c]);
-      const double s1 = __dmul_rn(value_scale, u[2 * (int64_t)vid[1] + c]);
-      const double s2 = __dmul_rn(value_scale, u[2 * (int64_t)vid[2] + c]);
-      const double val = __ddiv_rn(__dadd_rn(__dadd_rn(__dmul_rn(w[0], s0), __dmul_rn(w[1], s1)), __dmul_rn(w[2], s2)), a2);
-      const double vmin = __dmul_rn(value_scale, ranges[4 * s + 2 * c]);
-      const double vmax = __dmul_rn(value_scale, ranges[4 * s + 2 * c + 1]);
-      const double rng = __dsub_rn(vmax, vmin);
-      double tt = 0.0;
-      if (rng > 0.0) tt = __ddiv_rn(__dsub_rn(val, vmin), rng);
-      tt = fmin(fmax(tt, 0.0), 1.0);
-      const double q = fmin(floor(__dmul_rn(256.0, tt)), 255.0);
-      g[c] = (uint8_t)(255.0 - q);
-    }
+    for (int c = 0; c < 2; ++c) g[c] = shade_displacement(w, a2, vid, u, c, ranges + 4 * s, value_scale);
     g0 = g[0];
     g1 = g[1];
   }
@@ -278,6 +284,17 @@ __global__ void k_cell_field_ranges(int ns, const int32_t* __restrict__ ids, con
     ranges[2 * blockIdx.x + 1] = mx;
   }
 }
+// Gray level of the cell value v: scale * v normalised by scale * (rng[0], rng[1]).  Every cell-component image
+// is shaded by this.
+__device__ __forceinline__ uint8_t shade_cell(double scale, double v, const double* __restrict__ rng2) {
+  const double val = __dmul_rn(scale, v);
+  const double vmin = __dmul_rn(scale, rng2[0]), vmax = __dmul_rn(scale, rng2[1]);
+  const double rng = __dsub_rn(vmax, vmin);
+  double tt = 0.0;
+  if (rng > 0.0) tt = __ddiv_rn(__dsub_rn(val, vmin), rng);
+  tt = fmin(fmax(tt, 0.0), 1.0);
+  return (uint8_t)(255.0 - fmin(floor(__dmul_rn(256.0, tt)), 255.0));
+}
 template <int NPC>
 __global__ void k_raster_cell_fields(int ns, int size, int n_fields, const int32_t* __restrict__ ids,
                                      const int64_t* __restrict__ cell_off, const int32_t* __restrict__ owner,
@@ -295,13 +312,7 @@ __global__ void k_raster_cell_fields(int ns, int size, int n_fields, const int32
   uint8_t g = 255;
   if (o != 0x7fffffff) {
     const int64_t cell = cell_off[s] + o / SUB;
-    const double val = __dmul_rn(scale, cell_component(ids[f], strain, stress)[3 * cell]);
-    const double vmin = __dmul_rn(scale, ranges[2 * (f * ns + s)]), vmax = __dmul_rn(scale, ranges[2 * (f * ns + s) + 1]);
-    const double rng = __dsub_rn(vmax, vmin);
-    double tt = 0.0;
-    if (rng > 0.0) tt = __ddiv_rn(__dsub_rn(val, vmin), rng);
-    tt = fmin(fmax(tt, 0.0), 1.0);
-    g = (uint8_t)(255.0 - fmin(floor(__dmul_rn(256.0, tt)), 255.0));
+    g = shade_cell(scale, cell_component(ids[f], strain, stress)[3 * cell], ranges + 2 * (f * ns + s));
   }
   images[gid] = g;
 }
@@ -318,6 +329,85 @@ cudaError_t launch_raster_cell_fields(Batch& b, int n_fields, const int32_t* d_i
     k_raster_cell_fields<3><<<g, T, 0, st>>>(b.ns, b.img_size, n_fields, d_ids, b.d_cell_off, b.owner, d_strain, d_stress, d_ranges, scale, d_images);
   else
     k_raster_cell_fields<4><<<g, T, 0, st>>>(b.ns, b.img_size, n_fields, d_ids, b.d_cell_off, b.owner, d_strain, d_stress, d_ranges, scale, d_images);
+  return cudaGetLastError();
+}
+
+// ---- the load cases of one triangle mesh (fea_batch_load_case_images / _cell_components, DESIGN.md 3.11) ----
+// The cases share the mesh, so one cover pass finds each pixel's owner triangle for all of them, and one thread
+// per pixel computes that triangle's weights once and shades every case (and field) from them with the helpers
+// of the single-batch kernels above: case k's pixels are, bit for bit, those of a batch solved with load k.
+__global__ void k_raster_shade_cases(int n_cases, int size, const int32_t* __restrict__ conn, const double* __restrict__ xy,
+                                     const double* __restrict__ affine, const int32_t* __restrict__ owner,
+                                     const double* __restrict__ u, int64_t u_stride, const double* __restrict__ ranges,
+                                     double value_scale, uint8_t* __restrict__ images) {
+  const int64_t lp = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t per = (int64_t)size * size;
+  if (lp >= per) return;
+  const int32_t o = owner[lp];
+  if (o == 0x7fffffff) {
+    for (int m = 0; m < 2 * n_cases; ++m) images[(int64_t)m * per + lp] = 255;
+    return;
+  }
+  const int j = (int)(lp / size), i = (int)(lp - (int64_t)j * size);
+  Tri t;
+  int32_t vid[3];
+  load_tri<3>(o, 0, conn, xy, affine, t, vid);
+  double w[3], a2;
+  bary(t, (double)i + 0.5, (double)j + 0.5, w, &a2);
+  for (int k = 0; k < n_cases; ++k) {
+#pragma unroll
+    for (int c = 0; c < 2; ++c)
+      images[(2 * (int64_t)k + c) * per + lp] = shade_displacement(w, a2, vid, u + k * u_stride, c, ranges + 4 * k, value_scale);
+  }
+}
+
+__global__ void k_raster_cell_fields_cases(int n_cases, int size, int n_fields, const int32_t* __restrict__ ids, int64_t nc,
+                                           const int32_t* __restrict__ owner, const double* __restrict__ strain,
+                                           const double* __restrict__ stress, const double* __restrict__ ranges,
+                                           double scale, uint8_t* __restrict__ images) {
+  const int64_t lp = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t per = (int64_t)size * size;
+  if (lp >= per) return;
+  const int32_t o = owner[lp];
+  for (int f = 0; f < n_fields; ++f) {
+    const double* src = cell_component(ids[f], strain, stress);
+    for (int k = 0; k < n_cases; ++k) {
+      uint8_t g = 255;
+      if (o != 0x7fffffff) g = shade_cell(scale, src[3 * (k * nc + o)], ranges + 2 * (f * n_cases + k));
+      images[((int64_t)f * n_cases + k) * per + lp] = g;
+    }
+  }
+}
+
+cudaError_t launch_case_owner(Batch& b, int size, const double* d_affine, int32_t* owner) {
+  cudaStream_t st = b.ctx->stream;
+  const int T = 256;
+  const int64_t per = (int64_t)size * size;
+  k_owner_init<<<(unsigned)((per + T - 1) / T), T, 0, st>>>(per, owner);
+  if (b.NC) k_raster_cover<3><<<(unsigned)((b.NC + T - 1) / T), T, 0, st>>>(b.NC, b.d_cell_off, 1, b.conn, b.xy, d_affine, size, owner);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_case_raster(Batch& b, int n_cases, int size, const double* d_affine, const int32_t* owner,
+                               const double* u, const double* ranges, double value_scale, uint8_t* d_images) {
+  const int T = 256;
+  const int64_t per = (int64_t)size * size;
+  k_raster_shade_cases<<<(unsigned)((per + T - 1) / T), T, 0, b.ctx->stream>>>(n_cases, size, b.conn, b.xy, d_affine, owner, u,
+                                                                                 2 * b.NV, ranges, value_scale, d_images);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_case_cell_fields(Batch& b, int n_cases, int size, const int32_t* owner, int n_fields,
+                                    const int32_t* d_ids, const int64_t* d_case_off, const double* d_strain,
+                                    const double* d_stress, double scale, double* d_ranges, uint8_t* d_images) {
+  cudaStream_t st = b.ctx->stream;
+  const int T = 256;
+  const int64_t per = (int64_t)size * size;
+  // case k is "sample" k of the case-major strain / stress arrays: each (field, case) range is reduced by the
+  // single-batch kernel in the single batch's order
+  k_cell_field_ranges<<<n_fields * n_cases, 256, 0, st>>>(n_cases, d_ids, d_case_off, d_strain, d_stress, d_ranges);
+  k_raster_cell_fields_cases<<<(unsigned)((per + T - 1) / T), T, 0, st>>>(n_cases, size, n_fields, d_ids, b.NC, owner, d_strain,
+                                                                          d_stress, d_ranges, scale, d_images);
   return cudaGetLastError();
 }
 

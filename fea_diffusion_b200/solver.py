@@ -741,6 +741,55 @@ class Batch:
         r.stats = st.as_dict()
         return r
 
+    # ---- outputs of every case of the last solve_load_cases, from the displacements kept on the device ----------
+    def load_case_info(self):
+        """(K, status (K,) int32, image size) of the fields the last successful ``solve_load_cases`` kept; the image
+        size is that of the camera the last ``load_case_images`` kept, 0 before one.  FeaError (BAD_STATE) before
+        any such call (fea_batch_load_case_info)."""
+        k, size, status = C.c_int32(), C.c_int32(), np.empty(8, np.int32)   # K <= 8
+        self.ctx._check(self.ctx.lib.fea_batch_load_case_info(self.h, C.byref(k), ptr(status), C.byref(size)))
+        return k.value, status[:k.value].copy(), size.value
+
+    def load_case_images(self, size: int, affine: np.ndarray, value_scale: float = 1.0) -> np.ndarray:
+        """Displacement images of every case of the last ``solve_load_cases``: (K, 2, size, size) uint8, case k bit
+        for bit those ``rasterize`` + ``download(images=True)`` give a batch solved with loads[k].  ``affine`` holds
+        the 4 camera values of the batch's one sample.  The camera is kept for ``load_case_cell_components``."""
+        if isinstance(size, bool) or not isinstance(size, (int, np.integer)) or not 1 <= size <= 8192:
+            raise ValueError("size must be an integer in 1..8192, not %r" % (size,))
+        affine = np.ascontiguousarray(affine, dtype=np.float64)
+        if affine.size != 4:
+            raise ValueError("affine must hold the 4 camera values of the batch's one sample, not %d" % affine.size)
+        k = self.load_case_info()[0]
+        img = np.empty((k, 2, int(size), int(size)), np.uint8)
+        self.ctx._check(self.ctx.lib.fea_batch_load_case_images(self.h, int(size), ptr(affine.reshape(4)),
+                                                                float(value_scale), ptr(img)))
+        return img
+
+    def load_case_strain_stress(self, stress_region: int = -1):
+        """(strain, stress), each (K, n_cells, 3): ``cell_strain_stress(stress_region)`` of every case of the last
+        ``solve_load_cases``, bit for bit."""
+        k = self.load_case_info()[0]
+        nc = self.packed.n_cells
+        strain, stress = np.empty((k, nc, 3)), np.empty((k, nc, 3))
+        self.ctx._check(self.ctx.lib.fea_batch_load_case_strain_stress(self.h, int(stress_region), ptr(strain), ptr(stress)))
+        return strain, stress
+
+    def load_case_cell_components(self, stress_region: int, names: Sequence[str], value_scale: float = 1.0):
+        """``rasterize_cell_components`` of every case of the last ``solve_load_cases``, bit for bit, with the camera of
+        the last ``load_case_images``: ({name: (K, size, size) uint8}, {name: (K, 2) f64})."""
+        names = list(names)
+        if not 1 <= len(names) <= 4 or any(nm not in self.CELL_FIELDS for nm in names):
+            raise ValueError("names must be 1..4 of %s, not %r" % (sorted(self.CELL_FIELDS), names))
+        k, _, size = self.load_case_info()
+        if not size:
+            raise FeaError(4, "load_case_cell_components before load_case_images")
+        ids = np.array([self.CELL_FIELDS[nm] for nm in names], np.int32)
+        img = np.empty((len(ids), k, size, size), np.uint8)
+        rng = np.empty((len(ids), k, 2))
+        self.ctx._check(self.ctx.lib.fea_batch_load_case_cell_components(self.h, int(stress_region), len(ids), ptr(ids),
+                                                                         float(value_scale), ptr(img), ptr(rng)))
+        return {nm: img[i] for i, nm in enumerate(names)}, {nm: rng[i] for i, nm in enumerate(names)}
+
     def mg_apply(self, r: np.ndarray) -> np.ndarray:
         """z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as ``spmv``)."""
         r = np.ascontiguousarray(r, dtype=np.float64)

@@ -385,10 +385,30 @@ int  fea_batch_mg_apply(fea_batch* b, const double* r, double* z);
  * cases are interleaved per row), and their coarse systems are solved side by side in one batch of K copies
  * of level 0, built on the first call with that K and kept with the hierarchy.
  * FEA_BAD_STATE: no multigrid hierarchy, or not assembled.  FEA_BAD_ARG: n_cases outside 1..8, null rhs,
- * rtol < 0 or max_iter < 1. */
+ * rtol < 0 or max_iter < 1.
+ * A successful call keeps its K displacement fields (u as above), ranges and status on the device with the
+ * hierarchy, replacing those of the previous successful call whatever its K; the three calls below read them. */
 int  fea_batch_solve_load_cases(fea_batch* b, int32_t n_cases, const double* rhs, double rtol, int32_t max_iter,
                                 double* u, double* ranges, int32_t* iters, double* relres, int32_t* status,
                                 fea_solve_stats* stats);
+/* Outputs of every case of the last successful fea_batch_solve_load_cases (K = its n_cases), case-major: case k is,
+ * bit for bit, what the single-batch call gives a batch created with rhs[k] and solved by fea_batch_solve (a
+ * BREAKDOWN case included: the outputs of its u).  The K cases share the mesh: one cover pass per image call and
+ * one read of each cell's geometry and D serve them all.  FEA_BAD_STATE before a successful load-case call;
+ * FEA_BAD_ARG for what the single-batch call rejects.
+ * fea_batch_load_case_info: *n_cases = K, status [K] (may be NULL) = each kept case's status, *image_size (may be
+ * NULL) = size of the camera the last fea_batch_load_case_images kept, 0 before one.  FEA_BAD_STATE (and
+ * *n_cases = 0) before a successful load-case call.
+ * images [K][2][size][size]: the displacement images of fea_batch_rasterize + fea_batch_download_images with the
+ * same size, affine [4] and value_scale.  The call keeps its camera's owner map for the cell components below. */
+int  fea_batch_load_case_info(fea_batch* b, int32_t* n_cases, int32_t* status, int32_t* image_size);
+int  fea_batch_load_case_images(fea_batch* b, int32_t size, const double* affine, double value_scale, uint8_t* images);
+/* strain, stress [K][n_cells*3] as fea_batch_cell_strain_stress; either may be NULL. */
+int  fea_batch_load_case_strain_stress(fea_batch* b, int32_t stress_region, double* strain, double* stress);
+/* images [n_fields][K][size][size] and ranges [n_fields][K][2] as fea_batch_rasterize_cell_components, with the
+ * camera (size, affine) of the last fea_batch_load_case_images on the batch: FEA_BAD_STATE before one. */
+int  fea_batch_load_case_cell_components(fea_batch* b, int32_t stress_region, int32_t n_fields, const int32_t* field_ids,
+                                         double value_scale, uint8_t* images, double* ranges);
 
 /* ---- multigrid-preconditioned solve of a mesh with coarser meshes of the same domain ------------
  * The batch's only sample (P1 triangles) is the finest level of a hierarchy whose coarser levels are the samples
