@@ -28,7 +28,7 @@ EXPORTS = [
     "fea_batch_sample_sizes", "fea_batch_get_conn", "fea_batch_get_element_stiffness",
     "fea_batch_get_csr", "fea_batch_spmv", "fea_rasterize_fields", "fea_solve_batch",
     "fea_batch_set_refinement", "fea_batch_get_mg_levels", "fea_batch_get_level_csr", "fea_batch_mg_apply",
-    "fea_batch_set_coarse_meshes", "fea_batch_get_level_transfer", "fea_batch_solve_load_cases",
+    "fea_batch_set_coarse_meshes", "fea_batch_set_grid_hierarchy", "fea_batch_get_level_transfer", "fea_batch_solve_load_cases",
     "fea_batch_load_case_info", "fea_batch_load_case_images", "fea_batch_load_case_strain_stress", "fea_batch_load_case_cell_components",
 ]
 
@@ -168,6 +168,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "fea_batch_get_level_csr": (C.c_int, [P, I32, P, P, P]),
         "fea_batch_mg_apply": (C.c_int, [P, P, P]),
         "fea_batch_set_coarse_meshes": (C.c_int, [P, C.POINTER(BatchDesc)]),
+        "fea_batch_set_grid_hierarchy": (C.c_int, [P, I32]),
         "fea_batch_get_level_transfer": (C.c_int, [P, I32, P, P, P]),
         "fea_batch_solve_load_cases": (C.c_int, [P, I32, P, F64, I32, P, P, P, P, P, C.POINTER(SolveStats)]),
         "fea_batch_load_case_info": (C.c_int, [P, P, P, P]),

@@ -138,6 +138,8 @@ int api_batch_finish(fea_ctx* ctx, Batch& b, const int8_t* creg_local, const int
   return FEA_OK;
 }
 
+int alloc_solver_arrays(fea_ctx* ctx, Batch& b);
+
 int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke) {
   cudaStream_t st = ctx->c.stream;
   const int N = 2 * b.npc;
@@ -166,6 +168,45 @@ int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(B
   b.max_row_blocks = h_err[1];
   CK(ctx, dalloc(b, &b.adj, b.n_adj));
   CK(ctx, launch_topology_fill(b));
+  const int rc = alloc_solver_arrays(ctx, b);
+  if (rc != FEA_OK) return rc;
+  CK(ctx, launch_sell_fill(b));
+  ctx->c.launches += 1 + 10 + 4 + 1 + 2;
+  b.assembled = true;
+  return FEA_OK;
+}
+
+int api_batch_assemble_csr(fea_ctx* ctx, Batch& b, const int32_t* indptr, const int32_t* indices, const double* blocks,
+                           int32_t max_row) {
+  cudaStream_t st = ctx->c.stream;
+  b.from_csr = true;
+  CK(ctx, dalloc(b, &b.adj_ptr, b.NV + 1));
+  CK(ctx, cudaMemcpyAsync(b.adj_ptr, indptr, sizeof(int32_t) * (b.NV + 1), cudaMemcpyDeviceToDevice, st));
+  b.n_slices = (int32_t)(b.NBR / kSlice);
+  CK(ctx, dalloc(b, &b.slice_len, b.n_slices));
+  CK(ctx, dalloc(b, &b.slice_ptr, (int64_t)b.n_slices + 1));
+  CK(ctx, launch_sell_lengths(b));
+  int32_t h_adj = 0;
+  int64_t h_blocks = 0;
+  CK(ctx, cudaMemcpyAsync(&h_adj, b.adj_ptr + b.NV, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(&h_blocks, b.slice_ptr + b.n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  b.n_adj = h_adj;
+  b.n_blocks = b.n_slices ? h_blocks : 0;
+  b.max_row_blocks = max_row;
+  CK(ctx, dalloc(b, &b.adj, b.n_adj));
+  CK(ctx, cudaMemcpyAsync(b.adj, indices, sizeof(int32_t) * b.n_adj, cudaMemcpyDeviceToDevice, st));
+  const int rc = alloc_solver_arrays(ctx, b);
+  if (rc != FEA_OK) return rc;
+  CK(ctx, launch_sell_fill_csr(b, blocks));
+  ctx->c.launches += 4 + 2;
+  b.assembled = true;
+  return FEA_OK;
+}
+
+// block-SELL values, scaling and the solver's vectors and scalars of a batch whose adjacency and slices are known
+int alloc_solver_arrays(fea_ctx* ctx, Batch& b) {
+  cudaStream_t st = ctx->c.stream;
   CK(ctx, dalloc(b, &b.val, b.n_blocks * 4));
   CK(ctx, dalloc(b, &b.col, b.n_blocks));
   CK(ctx, dalloc(b, &b.dscale, b.NBR * 2));
@@ -201,9 +242,6 @@ int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(B
   CK(ctx, cudaMemsetAsync(b.sc.status, 0xFF, sizeof(int32_t) * b.ns, st));
   CK(ctx, cudaMemsetAsync(b.sc.iters, 0, sizeof(int32_t) * b.ns, st));
   CK(ctx, cudaMemsetAsync(b.relres, 0, sizeof(double) * b.ns, st));
-  CK(ctx, launch_sell_fill(b));
-  ctx->c.launches += 1 + 10 + 4 + 1 + 2;
-  b.assembled = true;
   return FEA_OK;
 }
 
@@ -840,8 +878,9 @@ int fea_batch_set_coarse_meshes(fea_batch* hb, const fea_batch_desc* d) {
   Batch& b = hb->b;
   if (b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_set_coarse_meshes after fea_batch_assemble");
   if (b.mg)
-    return api_fail(ctx, FEA_BAD_STATE, b.mg->nonnested ? "the batch already has its coarse meshes"
-                                                        : "the batch already declared its refinement");
+    return api_fail(ctx, FEA_BAD_STATE, b.mg->grid ? "the batch already has its grid hierarchy"
+                                        : b.mg->nonnested ? "the batch already has its coarse meshes"
+                                                          : "the batch already declared its refinement");
   if (b.ns != 1 || b.npc != 3) return api_fail(ctx, FEA_BAD_ARG, "a multigrid hierarchy needs one sample of triangles");
   if (!d) return api_fail(ctx, FEA_BAD_ARG, "null coarse mesh description");
   if (d->n_samples < 1 || d->n_samples > 8) return api_fail(ctx, FEA_BAD_ARG, "1..8 coarse meshes");
@@ -864,6 +903,21 @@ int fea_batch_set_coarse_meshes(fea_batch* hb, const fea_batch_desc* d) {
   }
   CK(ctx, cudaSetDevice(ctx->c.device));
   return mg_set_coarse_meshes(ctx, b, d);
+}
+
+int fea_batch_set_grid_hierarchy(fea_batch* hb, int32_t levels) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_set_grid_hierarchy after fea_batch_assemble");
+  if (b.mg)
+    return api_fail(ctx, FEA_BAD_STATE, b.mg->grid ? "the batch already has its grid hierarchy"
+                                        : b.mg->nonnested ? "the batch already has its coarse meshes"
+                                                          : "the batch already declared its refinement");
+  if (b.ns != 1 || b.npc != 3) return api_fail(ctx, FEA_BAD_ARG, "a multigrid hierarchy needs one sample of triangles");
+  if (levels < 1 || levels > 8) return api_fail(ctx, FEA_BAD_ARG, "levels must be 1..8");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  return mg_set_grid_hierarchy(ctx, b, levels);
 }
 
 int fea_batch_get_level_transfer(fea_batch* hb, int32_t level, int32_t* indptr, int32_t* indices, double* data) {

@@ -114,6 +114,7 @@ struct Batch {
   int32_t* err_flag = nullptr;   // device error flag (valence overflow etc.)
   // element matrices
   double* ke = nullptr;          // [NC*(2*npc)^2]
+  bool from_csr = false;         // matrix given as a block-CSR (api_batch_assemble_csr): no ke, no incidence lists
   // scaled block-SELL matrix
   int32_t n_slices = 0;
   int32_t* slice_len = nullptr;  // [n_slices]
@@ -185,6 +186,12 @@ struct MgLevel {
   int32_t* par3 = nullptr;       // [nv*3]
   double* w3 = nullptr;          // [nv*3] their interpolation weights
   double* child_w = nullptr;     // weights of the child entries
+  // grid hierarchies only (coarse levels): the level's unscaled Galerkin operator as a block-CSR over its vertices
+  // (rows of fixed vertices empty, columns ascending); kept for level 0 only once assemble is done
+  int32_t* g_ptr = nullptr;      // [nv+1]
+  int32_t* g_col = nullptr;      // [nnz]
+  double* g_val = nullptr;       // [nnz*4] 2x2 blocks (k00, k01, k10, k11)
+  int32_t g_max_row = 0;         // most blocks in a row (the diagonal included)
   double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};   // levels >= 1
   double lmax = 0.0;             // power-iteration estimate of the largest eigenvalue of Khat
   double inv_theta = 0.0, c1[2] = {0.0, 0.0}, c2[2] = {0.0, 0.0};   // Chebyshev coefficients
@@ -193,7 +200,8 @@ struct MgLevel {
 constexpr int kMaxCases = 8;     // load cases of one fea_batch_solve_load_cases call
 struct Mg {
   int levels = 0;
-  bool nonnested = false;        // coarse levels are the caller's meshes (fea_batch_set_coarse_meshes)
+  bool nonnested = false;        // transfers by up to 3 weighted parents: the caller's coarse meshes or grids
+  bool grid = false;             // coarse levels are nested background grids (fea_batch_set_grid_hierarchy)
   bool failed = false;           // building the hierarchy failed in fea_batch_assemble: the batch cannot be solved
   std::vector<MgLevel> lev;      // [levels + 1]
   double2 *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, finest row space (x = Batch::x)
@@ -250,6 +258,11 @@ int api_batch_finish(fea_ctx* ctx, Batch& b, const int8_t* d_creg_local, const i
 // element stiffness (fill_ke: launch_element_stiffness, or the Galerkin product of a multigrid level),
 // topology, block-SELL matrix and solver vectors of a created batch
 int api_batch_assemble(fea_ctx* ctx, Batch& b, const std::function<cudaError_t(Batch&)>& fill_ke);
+// the same from an unscaled block-CSR over the batch's vertices instead of element matrices: indptr [NV+1],
+// indices (sorted, the diagonal included, active vertices only; rows of fixed vertices empty), blocks [nnz*4];
+// max_row = most entries in a row.  Adjacency, 2x2 scaling and block-SELL values are read off it.
+int api_batch_assemble_csr(fea_ctx* ctx, Batch& b, const int32_t* indptr, const int32_t* indices, const double* blocks,
+                           int32_t max_row);
 
 // multigrid path (k_mg.cu): return FEA_OK or a status with the message set on ctx
 int mg_set_refinement(fea_ctx* ctx, Batch& b, int levels);   // derive and validate the hierarchy
@@ -262,8 +275,18 @@ int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int n_cases, const double* rhs, 
 void mg_release(Batch& b);
 // non-nested hierarchy (k_mg_nonnested.cu): coarse level batches from `coarse`, point location, transfers
 int mg_set_coarse_meshes(fea_ctx* ctx, Batch& b, const fea_batch_desc* coarse);
-// P_level as CSR over active DOFs (either kind of hierarchy, assembled batch); any array may be NULL
+// P_level as CSR over active DOFs (any kind of hierarchy, assembled batch); any array may be NULL
 int mg_level_transfer(fea_ctx* ctx, Batch& b, int level, int32_t* indptr, int32_t* indices, double* data);
+// point location of F's nvf vertices xyf in the triangles of a coarser level inside `box` (x0, x1, y0, y1):
+// F.par3 / F.w3, parents counted in cnt[nvc + 1]; then the restriction lists of F from those counts
+int mg_locate_points(fea_ctx* ctx, Batch& top, int l, MgLevel& F, int64_t nvf, const double* xyf, int64_t nvc, int64_t ncc,
+                     const int32_t* connc, const double* xyc, const double box[4], int32_t* cnt);
+int mg_child_lists(fea_ctx* ctx, Batch& top, MgLevel& F, int64_t nvc, int32_t* cnt);
+// grid hierarchy (k_mg_grid.cu): declare `levels` grid levels; build them at assemble (Galerkin operators, level batches)
+int mg_set_grid_hierarchy(fea_ctx* ctx, Batch& b, int levels);
+int mg_grid_assemble(fea_ctx* ctx, Batch& b);
+// the batch kb of n_cases copies of a grid level 0 (set up by api_batch_finish): matrices from level 0's block-CSR
+int mg_grid_assemble_cases(fea_ctx* ctx, const MgLevel& L0, Batch& kb, int n_cases);
 
 template <class T>
 inline cudaError_t dalloc(Batch& b, T** p, int64_t n) {
@@ -314,6 +337,10 @@ cudaError_t launch_sell_lengths(Batch& b);                    // slice_len + sli
 cudaError_t launch_sell_fill(Batch& b);                       // dscale, val, col
 cudaError_t launch_csr_export(Batch& b, int32_t s, int32_t* d_indptr, int32_t* d_indices,
                               double* d_data);
+// the batch's matrices as a block-CSR over its adjacency (blocks [n_adj*4], unscaled, rows of active vertices)
+cudaError_t launch_block_csr(Batch& b, double* d_blocks);
+// dscale, val, col of a batch assembled from a block-CSR (api_batch_assemble_csr)
+cudaError_t launch_sell_fill_csr(Batch& b, const double* d_blocks);
 // whole lock-step PCG loop (init, chunks of kChunk iterations, polling); fills b.stats / timings
 cudaError_t run_pcg(Batch& b, double rtol, int max_iter);
 void pcg_release(Ctx& c);                                     // destroys the cached graphs

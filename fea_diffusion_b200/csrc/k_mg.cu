@@ -19,6 +19,8 @@
 // Dot products: one partial per CTA, summed by one block in a fixed order (bitwise reproducible).
 // A non-nested hierarchy (fea_batch_set_coarse_meshes, k_mg_nonnested.cu; DESIGN.md section 3.10) runs the same
 // V-cycle and outer CG with rediscretised coarse operators and the k_mgn_* transfers (up to 3 weighted parents).
+// A grid hierarchy (fea_batch_set_grid_hierarchy, k_mg_grid.cu; DESIGN.md section 3.12) uses the same transfers
+// with nested background grids as coarse levels and Galerkin operators read from block-CSRs.
 // Both solve K = 1..8 load cases at once (fea_batch_solve_load_cases; DESIGN.md section 3.11): the V-cycle and
 // outer-CG kernels are templates on the number of columns they carry (a group of at most 4 cases), and
 // fea_batch_solve is the case K = 1.
@@ -1178,7 +1180,7 @@ __global__ void k_mg_replicate_cells(int64_t nc, int n_cases, const int32_t* __r
 }
 
 // The coarsest batch of a solve of K > 1 cases: K samples, each a copy of level 0 -- mesh, fixed mask, D and
-// its matrices ke (copied, not recomputed; Galerkin or rediscretised alike) -- so that each of its systems is
+// its matrices ke or block-CSR (copied, not recomputed; Galerkin or rediscretised alike) -- so that each of its systems is
 // bit for bit level 0's.  Built once per K and kept in mg.coarse[K].
 int coarse_for_cases(fea_ctx* ctx, Batch& b, int K) {
   Mg& mg = *b.mg;
@@ -1223,14 +1225,17 @@ int coarse_for_cases(fea_ctx* ctx, Batch& b, int K) {
   // level 0's cells are oriented already: take them exactly as they are, whatever the orientation test made of them
   k_mg_replicate_cells<<<gcell, 256, 0, st>>>(nc, K, c0.conn, c0.cell_dreg, nv, kb.conn, nullptr);
   CK(ctx, cudaGetLastError());
-  rc = api_batch_assemble(ctx, kb, [&c0, K](Batch& x) -> cudaError_t {
-    for (int k = 0; k < K; ++k) {
-      const cudaError_t e = cudaMemcpyAsync(x.ke + 36 * c0.NC * k, c0.ke, sizeof(double) * 36 * c0.NC, cudaMemcpyDeviceToDevice,
-                                            x.ctx->stream);
-      if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
-  });
+  if (mg.grid)   // a grid level 0 has no element matrices: its Galerkin block-CSR is copied instead
+    rc = mg_grid_assemble_cases(ctx, mg.lev[0], kb, K);
+  else
+    rc = api_batch_assemble(ctx, kb, [&c0, K](Batch& x) -> cudaError_t {
+      for (int k = 0; k < K; ++k) {
+        const cudaError_t e = cudaMemcpyAsync(x.ke + 36 * c0.NC * k, c0.ke, sizeof(double) * 36 * c0.NC, cudaMemcpyDeviceToDevice,
+                                              x.ctx->stream);
+        if (e != cudaSuccess) return e;
+      }
+      return cudaSuccess;
+    });
   if (rc != FEA_OK) return rc;
   int64_t rows = 0;   // block rows of one sample (every sample has level 0's)
   CK(ctx, cudaMemcpyAsync(&rows, kb.row_base + 1, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
@@ -1313,8 +1318,12 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
   cudaStream_t st = ctx->c.stream;
   // coarse level batches, finest-but-one first: each one's matrices are the Galerkin product of the next finer.
   // A non-nested hierarchy's coarse batches exist already (mg_set_coarse_meshes) and are rediscretised:
-  // each level's operator is its own mesh's stiffness matrix.
-  for (int l = mg.levels - 1; l >= 0; --l) {
+  // each level's operator is its own mesh's stiffness matrix.  A grid hierarchy builds its levels in k_mg_grid.cu.
+  if (mg.grid) {
+    const int rc = mg_grid_assemble(ctx, b);
+    if (rc != FEA_OK) return rc;
+  }
+  for (int l = mg.levels - 1; l >= 0 && !mg.grid; --l) {
     MgLevel& C = mg.lev[l];
     if (mg.nonnested) {
       const int rc = fea_batch_assemble(C.hb);

@@ -161,21 +161,18 @@ __global__ void k_mgn_child_sort(int64_t nvc, const int32_t* __restrict__ ptr, i
 
 unsigned blocks(int64_t n) { return (unsigned)((std::max<int64_t>(n, 1) + kT - 1) / kT); }
 
-// parents of level l's vertices in level l-1 (coarse: C, its host coordinates for the grid)
-int locate_level(fea_ctx* ctx, Batch& top, int l, MgLevel& F, MgLevel& C, const double* xy_host) {
+}  // namespace
+
+// parents and weights (F.par3, F.w3) of the nvf points xyf of level l in the triangles of level l-1 (nvc vertices
+// xyc, ncc triangles connc inside the box [x0, x1] x [y0, y1]); cnt[nvc + 1] (zeroed here) counts each parent's
+// kept entries
+int mg_locate_points(fea_ctx* ctx, Batch& top, int l, MgLevel& F, int64_t nvf, const double* xyf, int64_t nvc, int64_t ncc,
+                     const int32_t* connc, const double* xyc, const double box[4], int32_t* cnt) {
   cudaStream_t st = ctx->c.stream;
-  const Batch& fb = *F.b;
-  const Batch& cb = *C.b;
-  double x0 = xy_host[0], x1 = xy_host[0], y0 = xy_host[1], y1 = xy_host[1];
-  for (int64_t i = 1; i < C.nv; ++i) {
-    x0 = std::min(x0, xy_host[2 * i]);
-    x1 = std::max(x1, xy_host[2 * i]);
-    y0 = std::min(y0, xy_host[2 * i + 1]);
-    y1 = std::max(y1, xy_host[2 * i + 1]);
-  }
+  const double x0 = box[0], x1 = box[1], y0 = box[2], y1 = box[3];
   const double W = x1 - x0, H = y1 - y0, tol = 1e-10 * std::max(W, H);
   // about one grid cell per coarse triangle, square cells
-  const double hg = std::sqrt(std::max(W * H, 1e-300) / (double)std::max<int64_t>(C.nc, 1));
+  const double hg = std::sqrt(std::max(W * H, 1e-300) / (double)std::max<int64_t>(ncc, 1));
   Grid g;
   g.x0 = x0;
   g.y0 = y0;
@@ -187,15 +184,13 @@ int locate_level(fea_ctx* ctx, Batch& top, int l, MgLevel& F, MgLevel& C, const 
   g.inv_hy = H > 0.0 ? g.ny / H : 0.0;
   const int64_t ncell = (int64_t)g.nx * g.ny;
   Scratch scratch(st);
-  int32_t *gcnt = nullptr, *gptr = nullptr, *tmp = nullptr, *bad = nullptr, *cnt = nullptr, *glist = nullptr;
-  const int64_t nmax = std::max<int64_t>(ncell, C.nv);
+  int32_t *gcnt = nullptr, *gptr = nullptr, *tmp = nullptr, *bad = nullptr, *glist = nullptr;
   CK(ctx, scratch.alloc(&gcnt, ncell + 1));
   CK(ctx, scratch.alloc(&gptr, ncell + 1));
-  CK(ctx, scratch.alloc(&tmp, nmax / 4096 + 4));
+  CK(ctx, scratch.alloc(&tmp, ncell / 4096 + 4));
   CK(ctx, scratch.alloc(&bad, 1));
-  CK(ctx, scratch.alloc(&cnt, C.nv + 1));
   CK(ctx, cudaMemsetAsync(gcnt, 0, sizeof(int32_t) * (ncell + 1), st));
-  k_mgn_bin<<<blocks(C.nc), kT, 0, st>>>(C.nc, cb.conn, (const double2*)cb.xy, g, tol, nullptr, gcnt, nullptr);
+  k_mgn_bin<<<blocks(ncc), kT, 0, st>>>(ncc, connc, (const double2*)xyc, g, tol, nullptr, gcnt, nullptr);
   CK(ctx, cudaGetLastError());
   CK(ctx, exclusive_scan_i32(gcnt, gptr, ncell, tmp, st));
   int32_t total = 0;
@@ -203,39 +198,67 @@ int locate_level(fea_ctx* ctx, Batch& top, int l, MgLevel& F, MgLevel& C, const 
   CK(ctx, cudaStreamSynchronize(st));
   CK(ctx, scratch.alloc(&glist, total));
   CK(ctx, cudaMemsetAsync(gcnt, 0, sizeof(int32_t) * (ncell + 1), st));
-  k_mgn_bin<<<blocks(C.nc), kT, 0, st>>>(C.nc, cb.conn, (const double2*)cb.xy, g, tol, gptr, gcnt, glist);
+  k_mgn_bin<<<blocks(ncc), kT, 0, st>>>(ncc, connc, (const double2*)xyc, g, tol, gptr, gcnt, glist);
   CK(ctx, cudaGetLastError());
-  CK(ctx, dalloc(top, &F.par3, 3 * F.nv));
-  CK(ctx, dalloc(top, &F.w3, 3 * F.nv));
-  CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
+  CK(ctx, dalloc(top, &F.par3, 3 * nvf));
+  CK(ctx, dalloc(top, &F.w3, 3 * nvf));
+  CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (nvc + 1), st));
   const int32_t none = INT_MAX;
   CK(ctx, cudaMemcpyAsync(bad, &none, sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  k_mgn_locate<<<blocks(F.nv), kT, 0, st>>>(F.nv, (const double2*)fb.xy, cb.conn, (const double2*)cb.xy, g, tol * tol, gptr,
-                                            glist, F.par3, F.w3, cnt, bad);
+  k_mgn_locate<<<blocks(nvf), kT, 0, st>>>(nvf, (const double2*)xyf, connc, (const double2*)xyc, g, tol * tol, gptr, glist,
+                                           F.par3, F.w3, cnt, bad);
   CK(ctx, cudaGetLastError());
   int32_t h_bad = INT_MAX;
   CK(ctx, cudaMemcpyAsync(&h_bad, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
+  ctx->c.launches += 3;
   if (h_bad != INT_MAX) {
     char msg[200];
     snprintf(msg, sizeof msg, "vertex %d of level %d lies outside every triangle of level %d by more than %.3g", h_bad, l,
              l - 1, tol);
     return api_fail(ctx, FEA_MESH_ERROR, msg);
   }
-  // restriction lists: count (above) / scan / fill / sort
-  CK(ctx, dalloc(top, &F.child_ptr, C.nv + 1));
-  CK(ctx, exclusive_scan_i32(cnt, F.child_ptr, C.nv, tmp, st));
+  return FEA_OK;
+}
+
+// restriction lists of F's parents in a level of nvc vertices: scan of cnt (entries per parent), fill, sort
+int mg_child_lists(fea_ctx* ctx, Batch& top, MgLevel& F, int64_t nvc, int32_t* cnt) {
+  cudaStream_t st = ctx->c.stream;
+  Scratch scratch(st);
+  int32_t* tmp = nullptr;
+  CK(ctx, scratch.alloc(&tmp, nvc / 4096 + 4));
+  CK(ctx, dalloc(top, &F.child_ptr, nvc + 1));
+  CK(ctx, exclusive_scan_i32(cnt, F.child_ptr, nvc, tmp, st));
   int32_t n_child = 0;
-  CK(ctx, cudaMemcpyAsync(&n_child, F.child_ptr + C.nv, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(&n_child, F.child_ptr + nvc, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CK(ctx, cudaStreamSynchronize(st));
   CK(ctx, dalloc(top, &F.child, n_child));
   CK(ctx, dalloc(top, &F.child_w, n_child));
-  CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (C.nv + 1), st));
+  CK(ctx, cudaMemsetAsync(cnt, 0, sizeof(int32_t) * (nvc + 1), st));
   k_mgn_child_fill<<<blocks(F.nv), kT, 0, st>>>(F.nv, F.par3, F.w3, F.child_ptr, cnt, F.child, F.child_w);
-  k_mgn_child_sort<<<blocks(C.nv), kT, 0, st>>>(C.nv, F.child_ptr, F.child, F.child_w);
+  k_mgn_child_sort<<<blocks(nvc), kT, 0, st>>>(nvc, F.child_ptr, F.child, F.child_w);
   CK(ctx, cudaGetLastError());
-  ctx->c.launches += 6;
+  ctx->c.launches += 3;
   return FEA_OK;
+}
+
+namespace {
+
+// parents of level l's vertices in level l-1 (coarse: C, its host coordinates for the bounding box)
+int locate_level(fea_ctx* ctx, Batch& top, int l, MgLevel& F, MgLevel& C, const double* xy_host) {
+  double box[4] = {xy_host[0], xy_host[0], xy_host[1], xy_host[1]};
+  for (int64_t i = 1; i < C.nv; ++i) {
+    box[0] = std::min(box[0], xy_host[2 * i]);
+    box[1] = std::max(box[1], xy_host[2 * i]);
+    box[2] = std::min(box[2], xy_host[2 * i + 1]);
+    box[3] = std::max(box[3], xy_host[2 * i + 1]);
+  }
+  Scratch scratch(ctx->c.stream);
+  int32_t* cnt = nullptr;
+  CK(ctx, scratch.alloc(&cnt, C.nv + 1));
+  int rc = mg_locate_points(ctx, top, l, F, F.nv, F.b->xy, C.nv, C.nc, C.b->conn, C.b->xy, box, cnt);
+  if (rc == FEA_OK) rc = mg_child_lists(ctx, top, F, C.nv, cnt);
+  return rc;
 }
 
 }  // namespace

@@ -708,6 +708,13 @@ class Batch:
         self.ctx._check(self.ctx.lib.fea_batch_set_coarse_meshes(self.h, C.byref(packed.desc)))
         return self
 
+    def set_grid_hierarchy(self, levels: int):
+        """Declare ``levels`` (1..8) coarse levels built from the mesh alone: assemble lays nested background
+        grids over it (finest spacing twice the mean mesh size), prunes them to the mesh's reach and forms
+        Galerkin operators; solve and solve_load_cases then run multigrid-preconditioned CG."""
+        self.ctx._check(self.ctx.lib.fea_batch_set_grid_hierarchy(self.h, int(levels)))
+        return self
+
     def level_transfer(self, level: int):
         """scipy CSR of P_level (level-1 -> level) over active DOFs, in the numbering of ``csr``."""
         import scipy.sparse as sp

@@ -375,8 +375,8 @@ int  fea_batch_get_level_csr(fea_batch* b, int32_t level, int32_t* indptr, int32
 /* z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as fea_batch_spmv) */
 int  fea_batch_mg_apply(fea_batch* b, const double* r, double* z);
 /* K = n_cases load cases of the batch's one sample, solved together by the multigrid solve of
- * fea_batch_set_refinement / fea_batch_set_coarse_meshes.  rhs [n_cases][n_vertices*2]: full-DOF loads in
- * the layout of fea_batch_desc.rhs (values at fixed DOFs are not read).  Outputs (any may be NULL), with the
+ * fea_batch_set_refinement / fea_batch_set_coarse_meshes / fea_batch_set_grid_hierarchy.  rhs
+ * [n_cases][n_vertices*2]: full-DOF loads in the layout of fea_batch_desc.rhs (values at fixed DOFs are not read).  Outputs (any may be NULL), with the
  * meaning they have in fea_batch_download: u [n_cases][n_vertices*2], ranges [n_cases][4], iters, relres,
  * status [n_cases]; stats as fea_batch_get_solve_stats (iterations = the largest outer count).
  * Case k's outputs are bit for bit those fea_batch_solve gives a batch whose rhs is rhs[k], whatever other
@@ -428,6 +428,20 @@ int  fea_batch_load_case_cell_components(fea_batch* b, int32_t stress_region, in
  * connectivity index out of range.  If fea_batch_assemble then fails to build the coarse levels, the batch
  * stays unassembled: a second fea_batch_assemble returns FEA_BAD_STATE. */
 int  fea_batch_set_coarse_meshes(fea_batch* b, const fea_batch_desc* coarse);
+/* Declare `levels` (1..8) coarse levels that fea_batch_assemble builds itself, for a single triangle mesh whose
+ * coarser meshes the caller does not have: nested background grids over the mesh's bounding box (DESIGN.md
+ * section 3.12).  With h = sqrt(2 * area / n_cells), coarse level levels-1 is a grid of spacing 2h and each
+ * coarser level doubles it; the mesh's vertices are located in the finest grid's triangles by the rules of
+ * fea_batch_set_coarse_meshes, and grid to grid P is the red refinement's (weights 1 and 1/2).  Grid vertices
+ * that no active vertex of the next finer level reaches have no row.  Coarse operators are Galerkin,
+ * K_(l-1) = P^T K_l P, so the grids need no material or constraint data.  Solves, load cases and every output
+ * are those of fea_batch_set_coarse_meshes, and fea_batch_get_mg_levels / get_level_csr / get_level_transfer
+ * read the grid levels.  FEA_BAD_ARG: more than one sample, quads, levels outside 1..8.  FEA_BAD_STATE: after
+ * fea_batch_assemble or when the batch already has a hierarchy of any kind.  Accepted on batches from
+ * fea_batch_create and from fea_batch_create_from_conditions.  If fea_batch_assemble fails to build the levels
+ * (FEA_MESH_ERROR when a Galerkin row of a level would exceed 63 neighbours; the message names the level), the
+ * batch stays unassembled: a second fea_batch_assemble returns FEA_BAD_STATE. */
+int  fea_batch_set_grid_hierarchy(fea_batch* b, int32_t levels);
 /* P_l (level l-1 -> level l) as CSR over active DOFs, unscaled: rows = active DOFs of level l, columns = active DOFs
  * of level l-1, same numbering rule as fea_batch_get_csr; level 1..levels; for either kind of hierarchy.  After
  * fea_batch_assemble; any pointer may be NULL (indptr [rows+1] alone gives nnz = indptr[rows]). */
