@@ -30,6 +30,7 @@ EXPORTS = [
     "fea_batch_set_refinement", "fea_batch_get_mg_levels", "fea_batch_get_level_csr", "fea_batch_mg_apply",
     "fea_batch_set_coarse_meshes", "fea_batch_set_grid_hierarchy", "fea_batch_get_level_transfer", "fea_batch_solve_load_cases",
     "fea_batch_load_case_info", "fea_batch_load_case_images", "fea_batch_load_case_strain_stress", "fea_batch_load_case_cell_components",
+    "fea_batch_set_coarse_solver", "fea_batch_get_coarse_info", "fea_batch_coarse_solve",
 ]
 
 STATUS_NAMES = {0: "OK", 1: "BAD_ARG", 2: "CUDA_ERROR", 3: "OUT_OF_MEMORY", 4: "BAD_STATE", 5: "MESH_ERROR"}
@@ -98,6 +99,16 @@ class MgLevel(C.Structure):
     _fields_ = [
         ("n_vertices", C.c_int64), ("n_cells", C.c_int64), ("n_active_dofs", C.c_int64), ("nnz", C.c_int64),
         ("lambda_max", C.c_double), ("vcycle_ms", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class CoarseInfo(C.Structure):
+    """fea_coarse_info (include/fea_b200.h)."""
+    _fields_ = [
+        ("solver", C.c_int32), ("n", C.c_int32), ("factor_ms", C.c_double), ("min_pivot", C.c_double), ("bytes", C.c_int64),
     ]
 
     def as_dict(self):
@@ -175,6 +186,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "fea_batch_load_case_images": (C.c_int, [P, I32, P, F64, P]),
         "fea_batch_load_case_strain_stress": (C.c_int, [P, I32, P, P]),
         "fea_batch_load_case_cell_components": (C.c_int, [P, I32, I32, P, F64, P, P]),
+        "fea_batch_set_coarse_solver": (C.c_int, [P, I32]),
+        "fea_batch_get_coarse_info": (C.c_int, [P, C.POINTER(CoarseInfo)]),
+        "fea_batch_coarse_solve": (C.c_int, [P, P, P]),
         "fea_solve_batch": (C.c_int, [P, C.POINTER(BatchDesc), F64, I32, I32, P, F64, P, P, P, P, P, P,
                                       C.POINTER(SolveStats)]),
     }

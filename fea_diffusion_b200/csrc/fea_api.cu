@@ -1119,4 +1119,58 @@ int fea_batch_mg_apply(fea_batch* hb, const double* r, double* z) {
   return FEA_OK;
 }
 
+int fea_batch_set_coarse_solver(fea_batch* hb, int32_t solver) {
+  if (!hb) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch has no multigrid hierarchy");
+  if (b.assembled || b.mg->failed) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_set_coarse_solver after fea_batch_assemble");
+  if (solver != FEA_COARSE_CG && solver != FEA_COARSE_DIRECT)
+    return api_fail(ctx, FEA_BAD_ARG, "solver must be FEA_COARSE_CG or FEA_COARSE_DIRECT");
+  b.mg->coarse_solver = solver;
+  return FEA_OK;
+}
+
+int fea_batch_get_coarse_info(fea_batch* hb, fea_coarse_info* out) {
+  if (!hb || !out) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch has no multigrid hierarchy");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_get_coarse_info before fea_batch_assemble");
+  const Mg& mg = *b.mg;
+  *out = fea_coarse_info{};
+  out->solver = mg.coarse_solver;
+  if (mg.coarse_solver == FEA_COARSE_DIRECT) {
+    out->n = (int32_t)mg.coarse_n;
+    out->factor_ms = mg.factor_ms;
+    out->min_pivot = mg.min_pivot;
+    out->bytes = (int64_t)sizeof(double) * mg.coarse_ld * mg.coarse_ld;
+  }
+  return FEA_OK;
+}
+
+int fea_batch_coarse_solve(fea_batch* hb, const double* r, double* x) {
+  if (!hb || !r || !x) return FEA_BAD_ARG;
+  fea_ctx* ctx = hb->owner;
+  Batch& b = hb->b;
+  if (!b.mg) return api_fail(ctx, FEA_BAD_STATE, "the batch has no multigrid hierarchy");
+  if (!b.assembled) return api_fail(ctx, FEA_BAD_STATE, "fea_batch_coarse_solve before fea_batch_assemble");
+  CK(ctx, cudaSetDevice(ctx->c.device));
+  cudaStream_t st = ctx->c.stream;
+  int32_t na = 0;
+  CK(ctx, cudaMemcpyAsync(&na, b.mg->lev[0].b->n_active, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  const int64_t n = 2 * (int64_t)na;
+  Scratch scratch(st);
+  double *d_r = nullptr, *d_x = nullptr;
+  CK(ctx, scratch.alloc(&d_r, n));
+  CK(ctx, scratch.alloc(&d_x, n));
+  CK(ctx, cudaMemcpyAsync(d_r, r, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  const int rc = mg_coarse_solve(ctx, b, d_r, d_x);
+  if (rc != FEA_OK) return rc;
+  CK(ctx, cudaMemcpyAsync(x, d_x, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaStreamSynchronize(st));
+  return FEA_OK;
+}
+
 }  // extern "C"

@@ -220,7 +220,19 @@ struct Mg {
   int32_t* case_status = nullptr;   // [kMaxCases] what each kept field is (fea_batch_load_case_info)
   int32_t* case_owner = nullptr; // [case_size^2] owner map of the last fea_batch_load_case_images (mesh and camera)
   int32_t case_size = 0;
+  // coarsest-level solver (fea_batch_set_coarse_solver; DESIGN.md section 3.13)
+  int coarse_solver = FEA_COARSE_CG;
+  double* coarse_inv = nullptr;  // FEA_COARSE_DIRECT: Khat_0^-1 [coarse_ld][coarse_ld], full symmetric storage
+  double* coarse_y = nullptr;    // [kMaxCases][coarse_ld] S^T rhs of each case (k_mg_direct.cu)
+  int64_t coarse_n = 0;          // level 0's active DOFs (0 for the CG solver)
+  int64_t coarse_ld = 0;         // leading dimension: coarse_n padded to the factorisation's tile
+  double factor_ms = 0.0;        // device time of the dense build, Cholesky and inversion
+  double min_pivot = 0.0;        // smallest Cholesky pivot of Khat_0
 };
+// direct coarse solver: largest level 0 (the inverse takes n^2 * 8 bytes, 2 GiB here) and the smallest Cholesky
+// pivot accepted (Khat_0 has identity diagonal blocks, so pivots lie in (0, 1]; DESIGN.md section 3.13)
+constexpr int64_t kMaxDirectDofs = 16384;
+constexpr double kMinDirectPivot = 1e-8;
 
 }  // namespace fea
 
@@ -287,6 +299,18 @@ int mg_set_grid_hierarchy(fea_ctx* ctx, Batch& b, int levels);
 int mg_grid_assemble(fea_ctx* ctx, Batch& b);
 // the batch kb of n_cases copies of a grid level 0 (set up by api_batch_finish): matrices from level 0's block-CSR
 int mg_grid_assemble_cases(fea_ctx* ctx, const MgLevel& L0, Batch& kb, int n_cases);
+// direct coarse solver (k_mg_direct.cu): dense Khat_0, its Cholesky factor and inverse into mg.coarse_inv; FEA_MESH_ERROR
+// above kMaxDirectDofs, for an empty row or a pivot at or below kMinDirectPivot
+int mg_direct_factor(fea_ctx* ctx, Batch& b);
+// x^ = Khat_0^-1 S^T rhs for K cases: case q's unscaled rhs by vertex at rhs + 2 * q * nv_stride (level 0's vertex
+// numbering), its solution in level 0's scaled rows at x[row * row_stride + q * col_stride] (double2 units)
+cudaError_t mg_direct_apply(const Mg& mg, int K, const double* rhs, int64_t nv_stride, double* x, int64_t row_stride,
+                            int64_t col_stride, cudaStream_t st);
+void mg_direct_release(Mg& mg, cudaStream_t st);
+// rhs [nv*2] by vertex from an active-DOF vector numbered by vrank (0 at fixed vertices)
+cudaError_t launch_active_to_vertices(cudaStream_t st, int64_t nv, const int32_t* vrank, const double* in, double* rhs);
+// one coarsest-level solve of level 0 (fea_batch_coarse_solve): r, x unscaled active-DOF vectors on the device
+int mg_coarse_solve(fea_ctx* ctx, Batch& b, const double* d_r, double* d_x);
 
 template <class T>
 inline cudaError_t dalloc(Batch& b, T** p, int64_t n) {

@@ -15,7 +15,9 @@
 //               on Khat (identity diagonal blocks: block-Jacobi Chebyshev) over [lmax/30, 1.1 lmax], lmax
 //               from 20 Lanczos steps per level at assemble time.
 //   coarsest  : run_pcg on the level-0 batch to rtol 1e-4; the inexact coarse solve makes the outer
-//               iteration flexible CG, beta = z+.(r+ - r) / (r.z) = -alpha z+.q / (r.z).
+//               iteration flexible CG, beta = z+.(r+ - r) / (r.z) = -alpha z+.q / (r.z).  A batch that asks for
+//               it (fea_batch_set_coarse_solver) applies a dense inverse of level 0 instead (k_mg_direct.cu;
+//               DESIGN.md section 3.13), and its V-cycle is a fixed symmetric operator.
 // Dot products: one partial per CTA, summed by one block in a fixed order (bitwise reproducible).
 // A non-nested hierarchy (fea_batch_set_coarse_meshes, k_mg_nonnested.cu; DESIGN.md section 3.10) runs the same
 // V-cycle and outer CG with rediscretised coarse operators and the k_mgn_* transfers (up to 3 weighted parents).
@@ -926,9 +928,15 @@ cudaError_t vcycle(fea_ctx* ctx, Batch& fine, Work& w, int l) {
   MgLevel& L = mg.lev[l];
   cudaEvent_t* ev = mg.ev.data() + 4 * l;
   cudaError_t e;
-  if (l == 0) {   // coarsest: block-Jacobi CG of the coarsest batch on the restricted residuals
+  if (l == 0) {   // coarsest: block-Jacobi CG of the coarsest batch on the restricted residuals, or the dense inverse
     if ((e = cudaEventRecord(ev[0], st)) != cudaSuccess) return e;
-    if ((e = run_pcg(*w.coarse, kCoarseRtol, kCoarseMaxIter)) != cudaSuccess) return e;
+    if (mg.coarse_solver == FEA_COARSE_DIRECT) {   // all K cases in one read of the inverse, into coarse->x
+      e = mg_direct_apply(mg, K, w.coarse->rhs, w.coarse_nv, w.coarse->x, w.coarse_map.row_stride, w.coarse_map.col_stride, st);
+      c.launches += 2;
+    } else {
+      e = run_pcg(*w.coarse, kCoarseRtol, kCoarseMaxIter);
+    }
+    if (e != cudaSuccess) return e;
     return cudaEventRecord(ev[1], st);
   }
   const Batch& b = *L.b;
@@ -1380,6 +1388,7 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
     for (auto& ev : mg.ev) CK(ctx, cudaEventCreate(&ev));
   }
   for (int l = 0; l <= mg.levels; ++l) CK(ctx, estimate_lmax(b, mg.lev[l]));
+  if (mg.coarse_solver == FEA_COARSE_DIRECT) return mg_direct_factor(ctx, b);
   return FEA_OK;
 }
 
@@ -1397,6 +1406,23 @@ int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z) {
   CK(ctx, cudaGetLastError());
   CK(ctx, cudaStreamSynchronize(st));
   accumulate_level_ms(mg);
+  return FEA_OK;
+}
+
+int mg_coarse_solve(fea_ctx* ctx, Batch& b, const double* d_r, double* d_x) {
+  Mg& mg = *b.mg;
+  Batch& l0 = *mg.lev[0].b;
+  cudaStream_t st = ctx->c.stream;
+  CK(ctx, launch_active_to_vertices(st, l0.NV, l0.vrank, d_r, l0.rhs));
+  if (mg.coarse_solver == FEA_COARSE_DIRECT)
+    CK(ctx, mg_direct_apply(mg, 1, l0.rhs, l0.NV, l0.x, 1, 0, st));
+  else
+    CK(ctx, run_pcg(l0, kCoarseRtol, kCoarseMaxIter));
+  const unsigned g = grid_rows(l0);
+  if (g) k_mg_store<<<g, kT, 0, st>>>(side_of(l0), l0.vrank, (const double2*)l0.x, d_x);
+  ctx->c.launches += 3;
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaStreamSynchronize(st));
   return FEA_OK;
 }
 
@@ -1507,6 +1533,7 @@ void mg_release(Batch& b) {
     if (cb) api_free_batch(cb);
   for (void* p : {(void*)mg->case_u, (void*)mg->case_ranges, (void*)mg->case_status, (void*)mg->case_owner})
     if (p) cudaFreeAsync(p, b.ctx->stream);
+  mg_direct_release(*mg, b.ctx->stream);
   for (auto& ev : mg->ev) cudaEventDestroy(ev);
   if (mg->h_sc) cudaFreeHost(mg->h_sc);
   delete mg;

@@ -14,7 +14,7 @@ from typing import List, Optional, Sequence
 import numpy as np
 
 from . import _capi
-from ._capi import BatchDesc, BatchInfo, ConditionsDesc, FeaError, MgLevel, SolveStats, ptr
+from ._capi import BatchDesc, BatchInfo, CoarseInfo, ConditionsDesc, FeaError, MgLevel, SolveStats, ptr
 
 
 @dataclass
@@ -796,6 +796,37 @@ class Batch:
         self.ctx._check(self.ctx.lib.fea_batch_load_case_cell_components(self.h, int(stress_region), len(ids), ptr(ids),
                                                                          float(value_scale), ptr(img), ptr(rng)))
         return {nm: img[i] for i, nm in enumerate(names)}, {nm: rng[i] for i, nm in enumerate(names)}
+
+    COARSE_SOLVERS = {"cg": 0, "direct": 1}
+
+    def set_coarse_solver(self, name: str):
+        """Choose the coarsest-level solver of the declared hierarchy before ``assemble``: "cg" (block-Jacobi CG to rtol
+        1e-4, the default) or "direct" (a dense inverse of level 0, factorised on the device at assemble time)."""
+        if not isinstance(name, str) or name not in self.COARSE_SOLVERS:
+            raise ValueError("coarse solver must be one of %s, not %r" % (sorted(self.COARSE_SOLVERS), name))
+        self.ctx._check(self.ctx.lib.fea_batch_set_coarse_solver(self.h, self.COARSE_SOLVERS[name]))
+        return self
+
+    def coarse_info(self) -> dict:
+        """solver (0 cg, 1 direct), n, factor_ms, min_pivot and bytes of the assembled coarsest-level solver."""
+        i = CoarseInfo()
+        self.ctx._check(self.ctx.lib.fea_batch_get_coarse_info(self.h, C.byref(i)))
+        return i.as_dict()
+
+    def coarse_solve(self, r: np.ndarray) -> np.ndarray:
+        """x = level 0's solver applied to r, a float64 vector over level 0's active DOFs (unscaled, numbered as
+        ``level_csr(0)``)."""
+        if not isinstance(r, np.ndarray) or r.dtype != np.float64:
+            raise TypeError("r must be a float64 numpy array")
+        if r.ndim != 1:
+            raise ValueError("r must be one vector over level 0's active DOFs, not of shape %s" % (r.shape,))
+        n = int(self.mg_levels()[0]["n_active_dofs"])
+        if r.shape[0] != n:
+            raise ValueError("r must have level 0's %d active DOFs, not %d" % (n, r.shape[0]))
+        r = np.ascontiguousarray(r)
+        x = np.empty_like(r)
+        self.ctx._check(self.ctx.lib.fea_batch_coarse_solve(self.h, ptr(r), ptr(x)))
+        return x
 
     def mg_apply(self, r: np.ndarray) -> np.ndarray:
         """z = M r: one V-cycle on an active-DOF vector of the finest level (unscaled, as ``spmv``)."""

@@ -349,7 +349,7 @@ int  fea_batch_spmv(fea_batch* b, int32_t sample, const double* x, double* y);
  * (before fea_batch_assemble).  fea_batch_assemble then also builds the coarse levels -- Galerkin
  * operators P^T K P assembled cell by cell, block-Jacobi Chebyshev smoothers -- and fea_batch_solve
  * runs flexible CG preconditioned by one V-cycle per iteration, whose coarsest level is solved by the
- * block-Jacobi CG of fea_batch_solve to rtol 1e-4.  Outputs keep their meaning: iterations are outer
+ * block-Jacobi CG of fea_batch_solve to rtol 1e-4 (or exactly: fea_batch_set_coarse_solver).  Outputs keep their meaning: iterations are outer
  * iterations, relres is the TRUE residual in the block-Jacobi-scaled norm. */
 typedef struct {
   int64_t n_vertices, n_cells, n_active_dofs, nnz;   /* nnz of the reduced scalar CSR */
@@ -442,6 +442,35 @@ int  fea_batch_set_coarse_meshes(fea_batch* b, const fea_batch_desc* coarse);
  * (FEA_MESH_ERROR when a Galerkin row of a level would exceed 63 neighbours; the message names the level), the
  * batch stays unassembled: a second fea_batch_assemble returns FEA_BAD_STATE. */
 int  fea_batch_set_grid_hierarchy(fea_batch* b, int32_t levels);
+/* ---- coarsest-level solver of a multigrid batch ----------------------------------------------
+ * FEA_COARSE_CG (the default): each V-cycle solves level 0 by the block-Jacobi CG of fea_batch_solve to rtol 1e-4.
+ * FEA_COARSE_DIRECT: fea_batch_assemble also forms level 0's block-Jacobi-scaled operator Khat_0 = S^T K_0 S as a
+ * dense matrix (its active block rows in the level's solver order), factorises it by Cholesky on the device and
+ * replaces it with its full symmetric inverse; each V-cycle then applies that inverse to the restricted residuals of
+ * all its load cases in one read (DESIGN.md section 3.13).  The coarse solve is exact, so the V-cycle is a fixed
+ * symmetric operator.  The inverse takes n^2 * 8 bytes for n level-0 DOFs (188 MB at n = 4 844).
+ * fea_batch_set_coarse_solver: after fea_batch_set_refinement, set_coarse_meshes or set_grid_hierarchy and before
+ * fea_batch_assemble; the last call counts.  FEA_BAD_STATE without a hierarchy or after assemble; FEA_BAD_ARG for
+ * another solver value.  With FEA_COARSE_DIRECT, fea_batch_assemble fails with FEA_MESH_ERROR (the message names the
+ * number) when level 0 has more than 16 384 active DOFs, an empty row, or a Cholesky pivot at or below 1e-8 (a
+ * floating or nearly floating level 0); the batch then stays unassembled: a second assemble returns FEA_BAD_STATE. */
+enum { FEA_COARSE_CG = 0, FEA_COARSE_DIRECT = 1 };
+typedef struct {
+  int32_t solver;      /* FEA_COARSE_CG or FEA_COARSE_DIRECT */
+  int32_t n;           /* DOFs of the dense inverse (level 0's active DOFs); 0 for CG */
+  double factor_ms;    /* device time of the dense build, the factorisation and the inversion; 0 for CG */
+  double min_pivot;    /* smallest Cholesky pivot of Khat_0, in (0, 1]; 0 for CG */
+  int64_t bytes;       /* device memory the inverse keeps; 0 for CG */
+} fea_coarse_info;
+int  fea_batch_set_coarse_solver(fea_batch* b, int32_t solver);
+/* FEA_BAD_STATE without a hierarchy or before fea_batch_assemble */
+int  fea_batch_get_coarse_info(fea_batch* b, fea_coarse_info* out);
+/* x = level 0's solver applied to r, one vector over level 0's active DOFs in the numbering of
+ * fea_batch_get_level_csr(b, 0), both unscaled: the dense inverse, or the block-Jacobi CG to rtol 1e-4 that the
+ * V-cycle runs.  An inspection call, like fea_batch_mg_apply.  FEA_BAD_ARG for null pointers; FEA_BAD_STATE without
+ * a hierarchy or before fea_batch_assemble. */
+int  fea_batch_coarse_solve(fea_batch* b, const double* r, double* x);
+
 /* P_l (level l-1 -> level l) as CSR over active DOFs, unscaled: rows = active DOFs of level l, columns = active DOFs
  * of level l-1, same numbering rule as fea_batch_get_csr; level 1..levels; for either kind of hierarchy.  After
  * fea_batch_assemble; any pointer may be NULL (indptr [rows+1] alone gives nnz = indptr[rows]). */
