@@ -169,8 +169,9 @@ struct Batch {
 
 // One level of the multigrid hierarchy of a single-sample batch: a uniform refinement (DESIGN.md section
 // 3.9) or a mesh with coarser meshes of the same domain (section 3.10).
-// Level 0 is the coarsest mesh, level `levels` the batch itself.  Vectors are in the level's scaled
-// row space (Khat = S^T K S, rows in the level batch's solver order).
+// Level 0 is the coarsest mesh, level `levels` the batch itself.  It holds what assemble builds; the
+// vectors of a solve belong to the call (k_mg.cu) and are in the level's scaled row space (Khat = S^T K S,
+// rows in the level batch's solver order).
 struct MgLevel {
   fea_batch* hb = nullptr;       // internal batch of a coarse level (nullptr for the finest: the batch itself)
   Batch* b = nullptr;            // the level's batch
@@ -192,22 +193,20 @@ struct MgLevel {
   int32_t* g_col = nullptr;      // [nnz]
   double* g_val = nullptr;       // [nnz*4] 2x2 blocks (k00, k01, k10, k11)
   int32_t g_max_row = 0;         // most blocks in a row (the diagonal included)
-  double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};   // levels >= 1
   double lmax = 0.0;             // power-iteration estimate of the largest eigenvalue of Khat
   double inv_theta = 0.0, c1[2] = {0.0, 0.0}, c2[2] = {0.0, 0.0};   // Chebyshev coefficients
   double ms = 0.0;               // V-cycle time spent on the level in the last solve (of either kind)
 };
 constexpr int kMaxCases = 8;     // load cases of one fea_batch_solve_load_cases call
+// The hierarchy of a batch: what assemble builds and what the calls keep between them.  A solve's vectors are
+// its own (k_mg.cu).
 struct Mg {
   int levels = 0;
   bool nonnested = false;        // transfers by up to 3 weighted parents: the caller's coarse meshes or grids
   bool grid = false;             // coarse levels are nested background grids (fea_batch_set_grid_hierarchy)
   bool failed = false;           // building the hierarchy failed in fea_batch_assemble: the batch cannot be solved
   std::vector<MgLevel> lev;      // [levels + 1]
-  double2 *r = nullptr, *p = nullptr, *q = nullptr;   // outer flexible CG, finest row space (x = Batch::x)
-  double *partA = nullptr, *partB = nullptr;          // per-CTA partial sums
-  double* sc = nullptr;          // device scalars (kSc* slots, k_mg.cu)
-  double* h_sc = nullptr;        // pinned copy, room for kMaxCases cases
+  double* h_sc = nullptr;        // pinned host copy of a solve's device scalars (kSc* slots, k_mg.cu), kMaxCases cases
   std::vector<cudaEvent_t> ev;   // 4 per level + 2 around the solve
   // coarsest batches of load-case solves: coarse[K] has K samples, each a copy of level 0 (built on first use)
   fea_batch* coarse[kMaxCases + 1] = {};

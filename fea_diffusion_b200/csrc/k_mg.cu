@@ -26,6 +26,8 @@
 // Both solve K = 1..8 load cases at once (fea_batch_solve_load_cases; DESIGN.md section 3.11): the V-cycle and
 // outer-CG kernels are templates on the number of columns they carry (a group of at most 4 cases), and
 // fea_batch_solve is the case K = 1.
+// The hierarchy (Mg) keeps what assemble builds: level batches, transfers, smoother coefficients, the coarse
+// solver.  The vectors of a solve, a V-cycle or a Lanczos estimate belong to the call (a Scratch).
 #include <cmath>
 #include <cstdio>
 #include <memory>
@@ -814,25 +816,24 @@ double tridiag_max(const std::vector<double>& a, const std::vector<double>& b) {
   return hi;
 }
 
-// largest eigenvalue of level L's Khat: the top Ritz value of kLanczos Lanczos steps (vectors borrowed from
-// the outer CG).  15 power iterations, the cheaper alternative, stay at 2.03-2.07 on the C3 meshes where
-// Lanczos finds 2.34-2.39 (true 2.36-2.42): the smoother would then amplify the top of the spectrum.
-cudaError_t estimate_lmax(Batch& fine, MgLevel& L) {
-  Mg& mg = *fine.mg;
+// largest eigenvalue of level L's Khat: the top Ritz value of kLanczos Lanczos steps.  v, vp, w [NBR] and
+// part [NBR/kT] are sized to the finest level, sc holds kScCount + 2 kLanczos scalars.  15 power iterations,
+// the cheaper alternative, stay at 2.03-2.07 on the C3 meshes where Lanczos finds 2.34-2.39 (true 2.36-2.42):
+// the smoother would then amplify the top of the spectrum.
+cudaError_t estimate_lmax(Batch& fine, MgLevel& L, double2* v, double2* vp, double2* w, double* part, double* sc) {
   cudaStream_t st = fine.ctx->stream;
   const Batch& b = *L.b;
   const unsigned g = grid_rows(b);
   if (!g) return cudaSuccess;
-  double2 *v = mg.p, *vp = mg.q, *w = mg.r;
-  double* lz = mg.sc + kScCount;   // [2 kLanczos]: alpha_k, beta_k^2
-  k_mg_lz_init<<<g, kT, 0, st>>>(b.vertex_of_row, w, mg.partA);
-  cudaError_t e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, kScNrm);
-  if (e == cudaSuccess) k_mg_lz_next<<<g, kT, 0, st>>>(v, vp, w, mg.sc + kScNrm);
+  double* lz = sc + kScCount;   // [2 kLanczos]: alpha_k, beta_k^2
+  k_mg_lz_init<<<g, kT, 0, st>>>(b.vertex_of_row, w, part);
+  cudaError_t e = reduce(fine, sc, 1, part, nullptr, (int)g, kRedStore, kScNrm);
+  if (e == cudaSuccess) k_mg_lz_next<<<g, kT, 0, st>>>(v, vp, w, sc + kScNrm);
   for (int k = 0; k < kLanczos && e == cudaSuccess; ++k) {
-    k_mg_lz_apply<<<g, kT, 0, st>>>(op_of(b), v, w, mg.partA);
-    e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k);
-    k_mg_lz_orth<<<g, kT, 0, st>>>(v, vp, w, lz + 2 * k, k ? lz + 2 * k - 1 : nullptr, mg.partA);
-    if (e == cudaSuccess) e = reduce(fine, mg.sc, 1, mg.partA, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k + 1);
+    k_mg_lz_apply<<<g, kT, 0, st>>>(op_of(b), v, w, part);
+    e = reduce(fine, sc, 1, part, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k);
+    k_mg_lz_orth<<<g, kT, 0, st>>>(v, vp, w, lz + 2 * k, k ? lz + 2 * k - 1 : nullptr, part);
+    if (e == cudaSuccess) e = reduce(fine, sc, 1, part, nullptr, (int)g, kRedStore, 0, 0, 1, lz + 2 * k + 1);
     k_mg_lz_next<<<g, kT, 0, st>>>(v, vp, w, lz + 2 * k + 1);
   }
   std::vector<double> h(2 * kLanczos, 0.0);
@@ -876,9 +877,8 @@ void each_group(F&& f) {
 template <class T>
 T* at(T* v, int64_t n, int c0) { return v ? v + c0 * n : v; }
 
-// The vectors of one solve of K cases.  fea_batch_solve and fea_batch_mg_apply (K = 1) use the hierarchy's own
-// (mg.r/p/q/sc, MgLevel x/bv/r/d, the batch's x) and level 0's batch as the coarsest; a load-case call takes
-// them from a Scratch and, for K > 1, solves the coarsest systems in a batch of K copies of level 0.
+// The vectors of one call on K cases (make_work): a solve, a V-cycle of fea_batch_mg_apply (K = 1).  The
+// coarsest systems are those of a batch: level 0's own for K = 1, K copies of level 0 for K > 1.
 struct Vecs {
   double2 *x = nullptr, *bv = nullptr, *r = nullptr, *d[2] = {nullptr, nullptr};
 };
@@ -894,29 +894,12 @@ struct Work {
   int64_t coarse_nv = 0;                  // vertices per sample of the coarsest batch
 };
 
-Work own_work(Batch& b) {
-  Mg& mg = *b.mg;
-  Work w;
-  w.v.resize(mg.levels + 1);
-  for (int l = 1; l <= mg.levels; ++l) {
-    const MgLevel& L = mg.lev[l];
-    w.v[l].x = L.x;
-    w.v[l].bv = L.bv;
-    w.v[l].r = L.r;
-    w.v[l].d[0] = L.d[0];
-    w.v[l].d[1] = L.d[1];
-  }
-  w.x = (double2*)b.x;
-  w.r = mg.r;
-  w.p = mg.p;
-  w.q = mg.q;
-  w.partA = mg.partA;
-  w.partB = mg.partB;
-  w.sc = mg.sc;
-  w.rhs = b.rhs;
-  w.coarse = mg.lev[0].b;
-  w.coarse_nv = mg.lev[0].b->NV;
-  return w;
+// level 0's solver on the K systems of `coarse`, whose rhs holds case k's load by vertex at vertex k * nv_stride:
+// the dense inverse, all K cases in one read of it, into coarse.x at cm; or block-Jacobi CG of the whole batch
+cudaError_t coarse_solve(const Mg& mg, Batch& coarse, int K, int64_t nv_stride, ColMap cm, cudaStream_t st) {
+  if (mg.coarse_solver == FEA_COARSE_DIRECT)
+    return mg_direct_apply(mg, K, coarse.rhs, nv_stride, coarse.x, cm.row_stride, cm.col_stride, st);
+  return run_pcg(coarse, kCoarseRtol, kCoarseMaxIter);
 }
 
 // one V-cycle from level l down; level l's b, r, d[0], x are set up by the caller (restriction / top init)
@@ -928,14 +911,10 @@ cudaError_t vcycle(fea_ctx* ctx, Batch& fine, Work& w, int l) {
   MgLevel& L = mg.lev[l];
   cudaEvent_t* ev = mg.ev.data() + 4 * l;
   cudaError_t e;
-  if (l == 0) {   // coarsest: block-Jacobi CG of the coarsest batch on the restricted residuals, or the dense inverse
+  if (l == 0) {   // coarsest: the restricted residuals are in the coarsest batch's rhs
     if ((e = cudaEventRecord(ev[0], st)) != cudaSuccess) return e;
-    if (mg.coarse_solver == FEA_COARSE_DIRECT) {   // all K cases in one read of the inverse, into coarse->x
-      e = mg_direct_apply(mg, K, w.coarse->rhs, w.coarse_nv, w.coarse->x, w.coarse_map.row_stride, w.coarse_map.col_stride, st);
-      c.launches += 2;
-    } else {
-      e = run_pcg(*w.coarse, kCoarseRtol, kCoarseMaxIter);
-    }
+    e = coarse_solve(mg, *w.coarse, K, w.coarse_nv, w.coarse_map, st);
+    if (mg.coarse_solver == FEA_COARSE_DIRECT) c.launches += 2;
     if (e != cudaSuccess) return e;
     return cudaEventRecord(ev[1], st);
   }
@@ -1254,6 +1233,63 @@ int coarse_for_cases(fea_ctx* ctx, Batch& b, int K) {
   return FEA_OK;
 }
 
+// The Work of K (1..kMaxCases) cases, its vectors from `scratch` (one allocation each: DESIGN.md section 3.11).
+// Only the scalars are cleared: the driver and the V-cycle write every row of a vector before they read it.
+int make_work(fea_ctx* ctx, Batch& b, int K, Scratch& scratch, Work& w) {
+  Mg& mg = *b.mg;
+  if (K == 1) {
+    w.coarse = mg.lev[0].b;
+  } else {
+    const int rc = coarse_for_cases(ctx, b, K);
+    if (rc != FEA_OK) return rc;
+    w.coarse = &mg.coarse[K]->b;
+    w.coarse_map = ColMap{1, mg.case_rows};
+  }
+  w.coarse_nv = mg.lev[0].b->NV;
+  w.v.resize(mg.levels + 1);
+  for (int l = 1; l <= mg.levels; ++l) {
+    const int64_t n = mg.lev[l].b->NBR * K;
+    Vecs& V = w.v[l];
+    CK(ctx, scratch.alloc(&V.x, n));
+    CK(ctx, scratch.alloc(&V.r, n));
+    CK(ctx, scratch.alloc(&V.d[0], n));
+    CK(ctx, scratch.alloc(&V.d[1], n));
+    if (l < mg.levels) CK(ctx, scratch.alloc(&V.bv, n));   // the finest level's b is the outer CG's r
+  }
+  const int64_t nbr = b.NBR, np = nbr / kT;
+  CK(ctx, scratch.alloc(&w.x, nbr * K));
+  CK(ctx, scratch.alloc(&w.r, nbr * K));
+  CK(ctx, scratch.alloc(&w.p, nbr * K));
+  CK(ctx, scratch.alloc(&w.q, nbr * K));
+  CK(ctx, scratch.alloc(&w.partA, np * K));
+  CK(ctx, scratch.alloc(&w.partB, np * K));
+  CK(ctx, scratch.alloc(&w.sc, (int64_t)kScCount * K));
+  CK(ctx, cudaMemsetAsync(w.sc, 0, sizeof(double) * kScCount * K, ctx->c.stream));
+  return FEA_OK;
+}
+
+// solve<K> of K (1..kMaxCases) cases on a Work of the call: loads on the device, case k at rhs + k * rhs_stride
+int solve_cases(fea_ctx* ctx, Batch& b, int K, const double* rhs, int64_t rhs_stride, double rtol, int max_iter, const Out& o,
+                fea_solve_stats& stats) {
+  Scratch scratch(ctx->c.stream);
+  Work w;
+  const int rc = make_work(ctx, b, K, scratch, w);
+  if (rc != FEA_OK) return rc;
+  w.rhs = rhs;
+  w.rhs_stride = rhs_stride;
+  switch (K) {
+    case 1: return solve<1>(ctx, b, w, rtol, max_iter, o, stats);
+    case 2: return solve<2>(ctx, b, w, rtol, max_iter, o, stats);
+    case 3: return solve<3>(ctx, b, w, rtol, max_iter, o, stats);
+    case 4: return solve<4>(ctx, b, w, rtol, max_iter, o, stats);
+    case 5: return solve<5>(ctx, b, w, rtol, max_iter, o, stats);
+    case 6: return solve<6>(ctx, b, w, rtol, max_iter, o, stats);
+    case 7: return solve<7>(ctx, b, w, rtol, max_iter, o, stats);
+    case 8: return solve<8>(ctx, b, w, rtol, max_iter, o, stats);
+  }
+  return FEA_BAD_ARG;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1363,31 +1399,23 @@ int mg_assemble(fea_ctx* ctx, Batch& b) {
     if (rc != FEA_OK) return rc;
     ctx->c.launches += 1;
   }
-  // vectors: outer CG on the finest level, V-cycle state on every smoothed level
-  const int64_t nbr = b.NBR;
-  CK(ctx, dalloc(b, &mg.r, nbr));
-  CK(ctx, dalloc(b, &mg.p, nbr));
-  CK(ctx, dalloc(b, &mg.q, nbr));
-  CK(ctx, dalloc(b, &mg.partA, nbr / kT));
-  CK(ctx, dalloc(b, &mg.partB, nbr / kT));
-  CK(ctx, dalloc(b, &mg.sc, kScCount + 2 * kLanczos));
-  CK(ctx, cudaMemsetAsync(mg.sc, 0, sizeof(double) * (kScCount + 2 * kLanczos), st));
-  for (int l = 1; l <= mg.levels; ++l) {
-    MgLevel& L = mg.lev[l];
-    const int64_t n = L.b->NBR;
-    double2** v[5] = {&L.x, &L.r, &L.d[0], &L.d[1], &L.bv};   // the finest level's b is the outer CG's r
-    for (double2** p : v) {
-      if (p == &L.bv && l == mg.levels) continue;
-      CK(ctx, dalloc(b, p, n));
-      CK(ctx, cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st));
-    }
-  }
   if (!mg.h_sc) CK(ctx, cudaHostAlloc((void**)&mg.h_sc, sizeof(double) * kScCount * kMaxCases, cudaHostAllocDefault));
   if (mg.ev.empty()) {
     mg.ev.resize(4 * (mg.levels + 1) + 2);
     for (auto& ev : mg.ev) CK(ctx, cudaEventCreate(&ev));
   }
-  for (int l = 0; l <= mg.levels; ++l) CK(ctx, estimate_lmax(b, mg.lev[l]));
+  {   // Lanczos vectors of every level, sized to the finest
+    Scratch scratch(st);
+    const int64_t nbr = b.NBR;
+    double2 *v = nullptr, *vp = nullptr, *w = nullptr;
+    double *part = nullptr, *sc = nullptr;
+    CK(ctx, scratch.alloc(&v, nbr));
+    CK(ctx, scratch.alloc(&vp, nbr));
+    CK(ctx, scratch.alloc(&w, nbr));
+    CK(ctx, scratch.alloc(&part, nbr / kT));
+    CK(ctx, scratch.alloc(&sc, kScCount + 2 * kLanczos));
+    for (int l = 0; l <= mg.levels; ++l) CK(ctx, estimate_lmax(b, mg.lev[l], v, vp, w, part, sc));
+  }
   if (mg.coarse_solver == FEA_COARSE_DIRECT) return mg_direct_factor(ctx, b);
   return FEA_OK;
 }
@@ -1398,9 +1426,12 @@ int mg_apply(fea_ctx* ctx, Batch& b, const double* d_r, double* d_z) {
   const unsigned g = grid_rows(b);
   if (!g) return FEA_OK;
   for (auto& L : mg.lev) L.ms = 0.0;
-  Work w = own_work(b);
-  k_mg_load<<<g, kT, 0, st>>>(side_of(b), b.vrank, d_r, mg.r);
-  CK(ctx, vcycle_top<1>(ctx, b, w, mg.r, 1u));
+  Scratch scratch(st);
+  Work w;
+  const int rc = make_work(ctx, b, 1, scratch, w);
+  if (rc != FEA_OK) return rc;
+  k_mg_load<<<g, kT, 0, st>>>(side_of(b), b.vrank, d_r, w.r);
+  CK(ctx, vcycle_top<1>(ctx, b, w, w.r, 1u));
   k_mg_store<<<g, kT, 0, st>>>(side_of(b), b.vrank, w.v[mg.levels].x, d_z);
   ctx->c.launches += 2;
   CK(ctx, cudaGetLastError());
@@ -1414,10 +1445,7 @@ int mg_coarse_solve(fea_ctx* ctx, Batch& b, const double* d_r, double* d_x) {
   Batch& l0 = *mg.lev[0].b;
   cudaStream_t st = ctx->c.stream;
   CK(ctx, launch_active_to_vertices(st, l0.NV, l0.vrank, d_r, l0.rhs));
-  if (mg.coarse_solver == FEA_COARSE_DIRECT)
-    CK(ctx, mg_direct_apply(mg, 1, l0.rhs, l0.NV, l0.x, 1, 0, st));
-  else
-    CK(ctx, run_pcg(l0, kCoarseRtol, kCoarseMaxIter));
+  CK(ctx, coarse_solve(mg, l0, 1, l0.NV, ColMap{1, 0}, st));
   const unsigned g = grid_rows(l0);
   if (g) k_mg_store<<<g, kT, 0, st>>>(side_of(l0), l0.vrank, (const double2*)l0.x, d_x);
   ctx->c.launches += 3;
@@ -1427,56 +1455,20 @@ int mg_coarse_solve(fea_ctx* ctx, Batch& b, const double* d_r, double* d_x) {
 }
 
 int mg_solve(fea_ctx* ctx, Batch& b, double rtol, int max_iter) {
-  Work w = own_work(b);
   b.t_spmv.clear();
   b.t_update.clear();
   const Out o{b.sc.status, b.sc.iters, b.sc.rz0, b.rz_last, b.u, b.ranges, b.relres, nullptr};
-  return solve<1>(ctx, b, w, rtol, max_iter, o, b.stats);
+  return solve_cases(ctx, b, 1, b.rhs, 0, rtol, max_iter, o, b.stats);
 }
 
 int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int K, const double* rhs, double rtol, int max_iter, double* u, double* ranges,
                         int32_t* iters, double* relres, int32_t* status, fea_solve_stats* stats) {
   Mg& mg = *b.mg;
   cudaStream_t st = ctx->c.stream;
-  Work w;
-  if (K == 1) {
-    w.coarse = mg.lev[0].b;
-  } else {
-    const int rc = coarse_for_cases(ctx, b, K);
-    if (rc != FEA_OK) return rc;
-    w.coarse = &mg.coarse[K]->b;
-    w.coarse_map = ColMap{1, mg.case_rows};
-  }
-  w.coarse_nv = mg.lev[0].b->NV;
   Scratch scratch(st);
-  auto zeroed = [&](double2** p, int64_t n) -> cudaError_t {
-    cudaError_t e = scratch.alloc(p, n);
-    return e == cudaSuccess ? cudaMemsetAsync(*p, 0, sizeof(double2) * std::max<int64_t>(1, n), st) : e;
-  };
-  w.v.resize(mg.levels + 1);
-  for (int l = 1; l <= mg.levels; ++l) {
-    const int64_t n = mg.lev[l].b->NBR * K;
-    Vecs& V = w.v[l];
-    CK(ctx, zeroed(&V.x, n));
-    CK(ctx, zeroed(&V.r, n));
-    CK(ctx, zeroed(&V.d[0], n));
-    CK(ctx, zeroed(&V.d[1], n));
-    if (l < mg.levels) CK(ctx, zeroed(&V.bv, n));   // the finest level's b is the outer CG's r
-  }
-  const int64_t nbr = b.NBR, np = nbr / kT;
-  CK(ctx, zeroed(&w.x, nbr * K));
-  CK(ctx, zeroed(&w.r, nbr * K));
-  CK(ctx, zeroed(&w.p, nbr * K));
-  CK(ctx, zeroed(&w.q, nbr * K));
-  CK(ctx, scratch.alloc(&w.partA, np * K));
-  CK(ctx, scratch.alloc(&w.partB, np * K));
-  CK(ctx, scratch.alloc(&w.sc, (int64_t)kScCount * K));
-  CK(ctx, cudaMemsetAsync(w.sc, 0, sizeof(double) * kScCount * K, st));
   double* d_rhs = nullptr;
   CK(ctx, scratch.alloc(&d_rhs, 2 * b.NV * K));
   CK(ctx, cudaMemcpyAsync(d_rhs, rhs, sizeof(double) * 2 * b.NV * K, cudaMemcpyHostToDevice, st));
-  w.rhs = d_rhs;
-  w.rhs_stride = 2 * b.NV;
   Out o{};
   CK(ctx, scratch.alloc(&o.status, K));
   CK(ctx, scratch.alloc(&o.iters, K));
@@ -1485,19 +1477,9 @@ int mg_solve_load_cases(fea_ctx* ctx, Batch& b, int K, const double* rhs, double
   CK(ctx, scratch.alloc(&o.u, 2 * b.NV * K));
   CK(ctx, scratch.alloc(&o.ranges, 4 * K));
   CK(ctx, scratch.alloc(&o.relres, K));
-  if (K > 1) CK(ctx, scratch.alloc(&o.col, nbr));
+  if (K > 1) CK(ctx, scratch.alloc(&o.col, b.NBR));
   fea_solve_stats s{};
-  int rc = FEA_BAD_ARG;
-  switch (K) {
-    case 1: rc = solve<1>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 2: rc = solve<2>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 3: rc = solve<3>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 4: rc = solve<4>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 5: rc = solve<5>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 6: rc = solve<6>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 7: rc = solve<7>(ctx, b, w, rtol, max_iter, o, s); break;
-    case 8: rc = solve<8>(ctx, b, w, rtol, max_iter, o, s); break;
-  }
+  const int rc = solve_cases(ctx, b, K, d_rhs, 2 * b.NV, rtol, max_iter, o, s);
   if (rc != FEA_OK) return rc;
   // keep u, ranges and status of the cases for the fea_batch_load_case_* outputs, replacing the last call's
   mg.n_kept = 0;
